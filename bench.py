@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--generations n]
                     [--workload tree|arterial] [--scaling weak|strong] [--strong-generations m]
+                    [--dump-outputs DIR]
 
 A "step" is one numeric assembly (matrix + rhs) followed by one solve.  Workloads:
 
@@ -18,6 +19,11 @@ network is cut over the GPUs (weak: n + log2 N generations, strong: the same n).
 ``parity`` (size-independent checks of the returned solution, recomputed on the host in NumPy outside
 the timed region), ``setup_ms`` and a ``strong`` block (the same fixed tree at every N).  Prints ONE JSON
 line on rank 0.
+
+``--dump-outputs DIR`` (single GPU) writes the solution of the last timed step as ``Solver.solve()`` hands it
+out, one float64 ``DIR/<name>.npy`` per block (``flux_color_i``, ``pressure``, ``global_flux``).  The inputs
+depend on the arguments only, so two builds run with the same arguments can be compared block by block.
+Above 64 MB in all, every block is cut to the same share of its entries at indices drawn by a fixed seed.
 """
 
 from __future__ import annotations
@@ -390,6 +396,39 @@ def closed_form_check(pb, q0_local, lam_local, dist, torch):
             "multipliers": float(np.linalg.norm(lg - lam_ref) / den_l) if den_l > 0 else 0.0}
 
 
+def solution_blocks(solver):
+    """Copies of the blocks of ``solver.x`` under the names of the Functions ``Solver.solve()`` returns."""
+    asm = solver.assembler
+    spaces = [*asm.flux_spaces, asm.pressure_space, asm.lm_space]
+    names = [f"flux_color_{i}" for i in range(len(spaces) - 2)] + ["pressure", "global_flux"]
+    solver.x.mark_device_modified()
+    x = solver.x.array_r  # one D2H of the whole vector
+    out, off = {}, 0
+    for V, name in zip(spaces, names):
+        out[name] = x[off:off + V.num_dofs].copy()
+        off += V.num_dofs
+    return out
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, max_bytes=DUMP_MAX_BYTES, seed=0):
+    """``{name: array}`` -> ``out_dir/<name>.npy`` in float64, at most ``max_bytes`` in all (file headers
+    included).  Beyond that every array keeps the same share of its entries, at sorted indices drawn by a
+    generator seeded with ``seed``: arrays of the same sizes are always sampled at the same places."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(a, dtype=np.float64).ravel() for k, a in arrays.items()}
+    data_bytes = sum(a.nbytes for a in arrays.values())
+    budget = max_bytes - 128 * len(arrays)  # an .npy header is 128 bytes for a 1-D array
+    share = min(1.0, budget / data_bytes) if data_bytes else 1.0
+    for name, a in arrays.items():
+        if share < 1.0:
+            idx = np.random.default_rng(seed).choice(a.size, int(a.size * share), replace=False)
+            a = a[np.sort(idx)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def time_kernel(dev, fn, reps):
     fn()
     dev.sync()
@@ -424,6 +463,8 @@ def run_gpu(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise RuntimeError("bench.py needs a CUDA device: the product has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise RuntimeError("--dump-outputs writes the solution of a single-GPU run; run it without torchrun")
     torch.cuda.set_device(local_rank)
     dist = None
     if world > 1:
@@ -462,6 +503,8 @@ def run_gpu(args):
     sampler = ClockSampler(local_rank)
     sampler.start()  # sampled from warm-up to the end of the e2e loop (GPU under load throughout)
     ms_per_step, launches = pb.timed_steps(args.steps, args.warmup, barrier, dist, torch)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, solution_blocks(solver))
     value = n_dofs_total / (ms_per_step * 1e-3)
     opts, info, _lib = pb.opts, pb.info, pb._lib
     # true residual of the final iterate (one extra SpMV, outside the timed region)
@@ -750,7 +793,13 @@ def main():
                     help="P2/P1 and P3/P2 side measurement on make_tree(m), N=4 (single GPU); 0 = skip")
     ap.add_argument("--strong-generations", type=int, default=23,
                     help="fixed tree of the extra strong-scaling block printed at every N (0 = off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the solution of the last timed step as DIR/<block>.npy (float64, single GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed; it needs --impl b200")
     if args.generations is None:
         args.generations = 20 if args.workload == "tree" else 18
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup

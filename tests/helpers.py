@@ -1,5 +1,7 @@
 """Shared graph builders / comparison helpers for the tests."""
 
+import socket
+
 import networkx as nx
 import numpy as np
 
@@ -88,6 +90,14 @@ def oracle_for(nm, N, G=None, strategy=None):
     assert np.array_equal(colors, nm.edge_colors), "edge colouring differs from the reference's call"
     assert np.array_equal(pos, nm._node_pos)
     return rp.OracleNetwork(pos, edges, colors, N)
+
+
+def free_port() -> int:
+    """A loopback TCP port that is free now, for the rendezvous of multi-process tests (a fixed port
+    collides with another run of the suite on the same host)."""
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
 
 
 def rel_l2(a, b):

@@ -11,6 +11,7 @@ import torch.multiprocessing as mp
 import networks_fenicsx_b200 as nxfx
 from networks_fenicsx_b200 import network_generation as ng
 from networks_fenicsx_b200 import parallel
+from tests import helpers
 
 
 def make_forest():
@@ -46,7 +47,7 @@ def test_forest_partition_world2():
     world = 2
     with mp.Manager() as manager:
         out = manager.dict()
-        mp.spawn(_worker, args=(world, 29611, out), nprocs=world, join=True)
+        mp.spawn(_worker, args=(world, helpers.free_port(), out), nprocs=world, join=True)
         res = dict(out)
     F = make_forest()
     whole = nxfx.HydraulicNetworkAssembler(nxfx.NetworkMesh(F, N=3, color_strategy="smallest_last"))

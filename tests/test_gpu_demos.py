@@ -6,6 +6,8 @@ import sys
 
 import pytest
 
+from tests import helpers
+
 pytestmark = pytest.mark.gpu
 DEMOS = pathlib.Path(__file__).resolve().parent.parent / "demos"
 
@@ -38,7 +40,7 @@ def test_demo_runs_unchanged_under_torchrun(script, args, tmp_path):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
-           "--master-port", "29671", str(DEMOS / script), *args]
+           "--master-port", str(helpers.free_port()), str(DEMOS / script), *args]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=tmp_path,
                          env={**os.environ, "PYTHONPATH": str(DEMOS.parent)})
     assert out.returncode == 0, out.stdout[-2500:] + out.stderr[-2500:]

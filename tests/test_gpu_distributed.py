@@ -8,6 +8,8 @@ import sys
 
 import pytest
 
+from tests import helpers
+
 pytestmark = pytest.mark.gpu
 ROOT = pathlib.Path(__file__).resolve().parent.parent
 
@@ -26,7 +28,7 @@ def test_single_tree_partition_two_gpus(args):
     if torch.cuda.device_count() < 2:
         pytest.skip("needs 2 GPUs")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-           "--master-addr", "127.0.0.1", "--master-port", "29631", str(ROOT / "tests" / "dist_check.py"), *args]
+           "--master-addr", "127.0.0.1", "--master-port", str(helpers.free_port()), str(ROOT / "tests" / "dist_check.py"), *args]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
     assert "-> OK" in out.stdout
@@ -44,7 +46,7 @@ def test_single_tree_partition_ranks_sharing_one_gpu(args, world):
 
     env = dict(os.environ, NXFX_DIST_ONE_GPU="1")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world),
-           "--master-addr", "127.0.0.1", "--master-port", "29641", str(ROOT / "tests" / "dist_check.py"), *args]
+           "--master-addr", "127.0.0.1", "--master-port", str(helpers.free_port()), str(ROOT / "tests" / "dist_check.py"), *args]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, env=env)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
     assert "-> OK" in out.stdout
