@@ -283,7 +283,27 @@ int nxfx_set_condensation(nxfx_ctx* ctx, int32_t continuous_pressure, int32_t fl
  *   nxfx_residual_partial  r = b - A x (local part) and buf = [shared rows of r | partial ||r||^2
  *                        over the non-shared owned rows | owned ||b||^2]  (n_shared + 2 doubles)
  *   nxfx_residual_finish <- all-reduced buf: shared rows written back to r, nrm_out_d = [||r||^2,
- *                        ||b||^2], identical on every rank                                    */
+ *                        ||b||^2], identical on every rank
+ * Higher-order elements (nxfx_set_generic_system + nxfx_set_condensation) take the same calls; the
+ * shared nodes then carry 2 x 2 blocks {P_b, lam_b} and the sections grow (nxfx_exchange_sizes):
+ *   setup  [partial diagonal blocks D | coupling blocks U to the parent | L from the parent]
+ *          12 max(n_shared, 1) doubles, 2 x 2 row-major per shared node (U, L of a link between two
+ *          shared nodes come from rank 0, which holds that edge; the other ranks send zeros)
+ *   apply  [partial nodal right-hand side {P, lam}]  2 max(n_shared, 1) doubles
+ *   residual [lam rows of r | P rows of r | P rows of b | ||r||^2 | ||b||^2]  (continuous pressure;
+ *          DG0: [lam rows of r | ||r||^2 | ||b||^2])
+ * _setup_end / _apply_end compute the shared nodes from the all-reduced buffer alone, in an order
+ * that is the same on every rank: the replicated nodal unknowns are bit-identical across ranks.
+ * Shared right-hand-side rows ("stay additive"): with a continuous pressure the row nq + node of a
+ * shared bifurcation is a PARTIAL sum on every rank, in b as assembled (each rank integrates f over
+ * its own cells) as in A x.  The application reads these rows unweighted (the sum over the ranks is
+ * the full row) and the multiplier rows weighted by lam_weight (replicated after _residual_finish;
+ * zero in b).  nxfx_residual_finish therefore writes the multiplier rows back replicated and the
+ * nodal pressure rows on the owner only (lam_weight 1, the others 0), and ||b||^2 takes the shared
+ * P rows of b from the all-reduced buffer, so every shared row counts once in both norms.  With
+ * those degrees nxfx_pack_shared / nxfx_unpack_shared move [lam rows | P rows] (2 n_shared).
+ * The peer exchange (nxfx_comm_create) is flux degree 1 / pressure degree 0 only and returns
+ * NXFX_ERR_UNSUPPORTED on such a ctx.                                                          */
 int nxfx_set_shared(nxfx_ctx* ctx, int32_t n_shared, const int32_t* shared_lm_h,
                     const double* lam_weight_h);
 /* Peer exchange over NVLink: with a communicator the library does the small SUM all-reduces itself.
@@ -304,6 +324,11 @@ int nxfx_comm_create(nxfx_ctx* ctx, int32_t rank, int32_t nranks, void* handle_o
 int nxfx_comm_connect(nxfx_ctx* ctx, const void* handles_all_h);
 int nxfx_comm_destroy(nxfx_ctx* ctx);
 int nxfx_top_size(nxfx_ctx* ctx, int32_t* n_shared); /* size of one exchanged section */
+/* doubles of the exchanged sections of the host-driven path, for either element family:
+ * setup (nxfx_pc_setup_begin), apply (nxfx_pc_apply_begin; _setup_apply_* take setup + apply, the
+ * application's part at offset setup) and residual (nxfx_residual_partial).  P1/DG0: 2 nt, nt and
+ * n_shared + 2 with nt = max(n_shared, 1).                                                          */
+int nxfx_exchange_sizes(nxfx_ctx* ctx, int32_t* setup, int32_t* apply, int32_t* residual);
 int nxfx_pc_setup_begin(nxfx_ctx* ctx, double* buf_d);
 int nxfx_pc_setup_end(nxfx_ctx* ctx, double* buf_d);
 int nxfx_pc_apply_begin(nxfx_ctx* ctx, const double* r_d, double* buf_d);

@@ -130,6 +130,7 @@ SIGNATURES = {
     "nxfx_comm_connect": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_comm_destroy": (C.c_int, [C.c_void_p]),
     "nxfx_top_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
+    "nxfx_exchange_sizes": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "nxfx_pc_setup_begin": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_pc_setup_end": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_pc_apply_begin": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),

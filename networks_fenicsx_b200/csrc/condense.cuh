@@ -345,10 +345,11 @@ cond_edge_rhs_kernel(Net g, CondDev c, const double* __restrict__ r) {
 
 // Nodal blocks, one thread per bifurcation.  FACTOR: diagonal block = sum of the incident S_e blocks (in
 // incidence order: deterministic), coupling blocks to the parent from the link edge.  Else: right-hand side
-// r_z - sum D_e y0.
+// r_z - sum D_e y0.  lam_w (partitioned network, else nullptr): weight of this rank's copy of a multiplier row
+// of r (replicated rows count on their owner only); the nodal pressure rows are read unweighted (additive).
 template <bool FACTOR>
 __global__ void __launch_bounds__(kThreads)
-cond_node_kernel(Net g, TreeDev t, CondDev c, const double* __restrict__ r) {
+cond_node_kernel(Net g, TreeDev t, CondDev c, const double* __restrict__ r, const double* __restrict__ lam_w = nullptr) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= g.n_bif) return;
   const size_t E = (size_t)g.E;
@@ -385,7 +386,7 @@ cond_node_kernel(Net g, TreeDev t, CondDev c, const double* __restrict__ r) {
       c.bL[4 * (size_t)n + k] = L[k];
     }
   } else {
-    double r0 = c.cont ? r[g.nq + c.bif_node[b]] : 0.0, r1 = r[g.loff + b];
+    double r0 = c.cont ? r[g.nq + c.bif_node[b]] : 0.0, r1 = lam_w ? lam_w[b] * r[g.loff + b] : r[g.loff + b];
     for (int k = g.bif_ptr[b]; k < g.bif_ptr[b + 1]; ++k) {
       const int inc = g.bif_inc[k];
       const int e = inc >> 1, o = (inc & 1) ? 2 : 0;
@@ -468,6 +469,167 @@ btree_sweep_kernel(TreeDev t, CondDev c, int chunk0) {
       }
       __syncthreads();
     }
+  }
+}
+
+// Top chunk of a partitioned network, split around the caller's all-reduce (block version of tree_top_kernel's
+// kPartial / kFinish, precond.cuh).  sh_idx[i]: position k of top-chunk node b0 + i in the exchanged order of the
+// shared nodes (identical on every rank), -1 for a node private to this rank (sh_idx == nullptr: no shared node).
+// Payload, nt = max(n_shared, 1):
+//   FACTOR: partial diagonal block D_k at buf[4k], coupling blocks U_k (to the parent) at buf[4nt + 4k] and
+//           L_k (from the parent) at buf[8nt + 4k], 2 x 2 row-major -- 12 nt doubles;
+//   SOLVE:  partial nodal right-hand side at buf[2k] -- 2 nt doubles.
+// A shared node's coupling blocks come from the edge to its shared parent, which lives on rank 0 (partition_tree):
+// the other ranks contribute zeros and the sum broadcasts them.
+// kPartial eliminates the private nodes (a private node has private children or bottom-chunk roots only), folds
+// them and this rank's bottom-chunk roots into their shared parents and packs the shared nodes.
+// kFinish reads nothing but the all-reduced payload and what it computes from it: the shared children of a shared
+// node are folded in their exchanged order, so every rank performs the same operations in the same order and
+// writes bit-identical factors and nodal unknowns.  The DG0 identity placeholder on the P slot (cond_node_kernel)
+// arrives summed over the ranks and is set again here.  SOLVE kFinish then runs the backward sweep of the top chunk.
+template <bool FACTOR, int PHASE>
+__global__ void __launch_bounds__(1024)
+btree_top_split_kernel(TreeDev t, CondDev c, int chunk, const int32_t* __restrict__ sh_idx, int nt, double* __restrict__ buf) {
+  const int L0 = t.chunk_lptr[chunk], L1 = t.chunk_lptr[chunk + 1];
+  const int b0 = t.lvl_ptr[L0];
+  auto kof = [&](int n) { return (sh_idx && n >= b0) ? sh_idx[n - b0] : -1; };  // n < b0: a bottom-chunk root
+  for (int L = L1 - 1; L >= L0; --L) {
+    const int lb = t.lvl_ptr[L], le = t.lvl_ptr[L + 1];
+    for (int n = lb + threadIdx.x; n < le; n += blockDim.x) {
+      const int k = kof(n);
+      if (PHASE == kFinish && k < 0) continue;  // private: complete after kPartial
+      const int c0 = t.t_cptr[n], c1 = t.t_cptr[n + 1];
+      if (FACTOR) {
+        M2 D = PHASE == kFinish ? ld2(buf, k) : ld2(c.bd0, n);
+        auto fold = [&](int ch) {
+          const M2 p = mul2(ld2(c.bH, ch), ld2(c.bU, ch));
+          D.a -= p.a; D.b -= p.b; D.c -= p.c; D.d -= p.d;
+        };
+        if (PHASE == kPartial) {
+          for (int q = c0; q < c1; ++q)
+            if (kof(t.t_cidx[q]) < 0) fold(t.t_cidx[q]);
+          if (k >= 0) {
+            st2(buf, k, D);
+            st2(buf + 4 * (size_t)nt, k, ld2(c.bU, n));
+            st2(buf + 8 * (size_t)nt, k, ld2(c.bL, n));
+            continue;
+          }
+        } else {
+          for (int last = -1;;) {  // shared children in exchanged order
+            int best = 0x7fffffff, bc = -1;
+            for (int q = c0; q < c1; ++q) {
+              const int kc = kof(t.t_cidx[q]);
+              if (kc > last && kc < best) { best = kc; bc = t.t_cidx[q]; }
+            }
+            if (bc < 0) break;
+            fold(bc);
+            last = best;
+          }
+          if (!c.cont) { D.a = 1.0; D.b = 0.0; D.c = 0.0; }
+          st2(c.bU, n, ld2(buf + 4 * (size_t)nt, k));
+          st2(c.bL, n, ld2(buf + 8 * (size_t)nt, k));
+        }
+        const double idet = 1.0 / (D.a * D.d - D.b * D.c);
+        const M2 Di{D.d * idet, -D.b * idet, -D.c * idet, D.a * idet};
+        st2(c.bDinv, n, Di);
+        st2(c.bG, n, mul2(Di, ld2(c.bU, n)));
+        st2(c.bH, n, mul2(ld2(c.bL, n), Di));
+      } else {
+        double r0, r1;
+        if (PHASE == kFinish) { r0 = buf[2 * (size_t)k]; r1 = buf[2 * (size_t)k + 1]; }
+        else { r0 = c.br[2 * (size_t)n]; r1 = c.br[2 * (size_t)n + 1]; }
+        auto fold = [&](int ch) {
+          const M2 H = ld2(c.bH, ch);
+          const double s0 = c.br[2 * (size_t)ch], s1 = c.br[2 * (size_t)ch + 1];
+          r0 -= H.a * s0 + H.b * s1;
+          r1 -= H.c * s0 + H.d * s1;
+        };
+        if (PHASE == kPartial) {
+          for (int q = c0; q < c1; ++q)
+            if (kof(t.t_cidx[q]) < 0) fold(t.t_cidx[q]);
+          if (k >= 0) { buf[2 * (size_t)k] = r0; buf[2 * (size_t)k + 1] = r1; continue; }
+        } else {
+          for (int last = -1;;) {
+            int best = 0x7fffffff, bc = -1;
+            for (int q = c0; q < c1; ++q) {
+              const int kc = kof(t.t_cidx[q]);
+              if (kc > last && kc < best) { best = kc; bc = t.t_cidx[q]; }
+            }
+            if (bc < 0) break;
+            fold(bc);
+            last = best;
+          }
+        }
+        c.br[2 * (size_t)n] = r0;
+        c.br[2 * (size_t)n + 1] = r1;
+      }
+    }
+    __syncthreads();
+  }
+  if (FACTOR || PHASE != kFinish) return;
+  for (int L = L0; L < L1; ++L) {  // backward sweep of the whole top chunk (as btree_sweep_kernel MODE 2)
+    const int lb = t.lvl_ptr[L], le = t.lvl_ptr[L + 1];
+    for (int n = lb + threadIdx.x; n < le; n += blockDim.x) {
+      const int p = t.t_parent[n];
+      const M2 Di = ld2(c.bDinv, n);
+      const double r0 = c.br[2 * (size_t)n], r1 = c.br[2 * (size_t)n + 1];
+      double z0 = Di.a * r0 + Di.b * r1, z1 = Di.c * r0 + Di.d * r1;
+      if (p >= 0) {
+        const M2 G = ld2(c.bG, n);
+        const double p0 = c.bz[2 * (size_t)p], p1 = c.bz[2 * (size_t)p + 1];
+        z0 -= G.a * p0 + G.b * p1;
+        z1 -= G.c * p0 + G.d * p1;
+      }
+      c.bz[2 * (size_t)n] = z0;
+      c.bz[2 * (size_t)n + 1] = z1;
+    }
+    __syncthreads();
+  }
+}
+
+// Partitioned network, continuous pressure: the nodal pressure rows nq + node of the shared bifurcations
+// (packed after the multiplier rows, in the exchanged order)
+__global__ void __launch_bounds__(kThreads)
+pack_nodal_kernel(int n_shared, int nq, const int32_t* __restrict__ shared_lm, const int32_t* __restrict__ bif_node,
+                  const double* __restrict__ v, double* __restrict__ buf) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n_shared) buf[i] = v[nq + bif_node[shared_lm[i]]];
+}
+__global__ void __launch_bounds__(kThreads)
+unpack_nodal_kernel(int n_shared, int nq, const int32_t* __restrict__ shared_lm, const int32_t* __restrict__ bif_node,
+                    const double* __restrict__ buf, double* __restrict__ v) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n_shared) v[nq + bif_node[shared_lm[i]]] = buf[i];
+}
+
+// After the all-reduce of [lam rows of r | (cont) P rows of r | (cont) P rows of b | ||r||^2 | ||b||^2] (the norm
+// partials without any shared row): multiplier rows back into r replicated, nodal pressure rows back into r on the
+// owner only (lam_weight) -- the nodal right-hand side reads them unweighted, so they must sum to the full row --
+// and the norms with every shared row counted once (identical on every rank).  One block.
+__global__ void __launch_bounds__(kThreads)
+cond_residual_finish_kernel(int n_shared, int loff, int nq, int cont, const int32_t* __restrict__ shared_lm,
+                            const int32_t* __restrict__ bif_node, const double* __restrict__ lam_weight,
+                            const double* __restrict__ buf, double* __restrict__ r, double* __restrict__ nrm_out) {
+  __shared__ double red[kThreads / 32];
+  double ar = 0.0, ab = 0.0;
+  for (int i = threadIdx.x; i < n_shared; i += blockDim.x) {
+    const int lm = shared_lm[i];
+    const double v = buf[i];
+    r[loff + lm] = v;
+    ar += v * v;
+    if (cont) {
+      const double p = buf[n_shared + i], pb = buf[2 * n_shared + i];
+      r[nq + bif_node[lm]] = lam_weight[lm] * p;
+      ar += p * p;
+      ab += pb * pb;
+    }
+  }
+  const int nr = cont ? 3 * n_shared : n_shared;
+  ar = block_sum<kThreads>(ar, red);
+  ab = block_sum<kThreads>(ab, red);
+  if (threadIdx.x == 0) {
+    nrm_out[0] = buf[nr] + ar;
+    nrm_out[1] = buf[nr + 1] + ab;
   }
 }
 

@@ -76,6 +76,7 @@ struct Condensation {
   DevBuf<int32_t> type_n, loc_ptr, loc_kind, loc_off, k_ptr, k_row, k_col, k_cell, c_ptr, c_row, c_slot, d_ptr, d_slot,
       d_col, bif_node, ipiv;
   DevBuf<double> k_coef, c_coef, d_coef, band, Y, S, y0, h, bd0, bU, bL, bDinv, bG, bH, br, bz;
+  std::vector<int32_t> bif_node_h;  // host copy (nodal pressure rows of the shared bifurcations)
 };
 
 // Peer exchange of the partitioned solve (peer.cuh): this rank's exchange buffer and the mapped
@@ -142,7 +143,9 @@ struct nxfx_ctx {
   nxfx::DevBuf<int32_t> shared_lm;
   std::vector<int32_t> shared_lm_h;
   nxfx::DevBuf<int32_t> top_sh_pos;  // [n_shared] position of every shared multiplier inside the top chunk
+  nxfx::DevBuf<int32_t> top_sh_idx;  // [n_top] inverse of top_sh_pos: exchanged index of a top-chunk node, -1 = private
   nxfx::DevBuf<double> lam_weight, lam_nonshared;
+  nxfx::DevBuf<double> p_nonshared;  // [n_nodes] continuous pressure: 0 on the shared bifurcations (partial rows)
   nxfx::PeerComm comm;
   // solution mirror: pinned host copy of x that nxfx_solve fills while the residual check still runs
   double* mirror_h = nullptr;

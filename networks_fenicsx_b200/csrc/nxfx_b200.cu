@@ -119,6 +119,7 @@ int upload(nxfx_ctx* ctx, DevBuf<T>& buf, const T* src, size_t n) {
 // positions of the shared multipliers inside the top chunk (needs both the schedule and the shared list)
 int update_top_shared(nxfx_ctx* ctx) {
   ctx->top_sh_pos.release();
+  ctx->top_sh_idx.release();
   ctx->tree.sh_lmax = -1;
   ctx->tree.pr_lmin = 0;
   if (!ctx->tree.set || ctx->n_shared == 0 || ctx->tree.t_of_bif_h.empty()) return NXFX_OK;
@@ -131,6 +132,10 @@ int update_top_shared(nxfx_ctx* ctx) {
   }
   NXFX_CUDA(ctx, ctx->top_sh_pos.alloc(pos.size()));
   NXFX_CUDA(ctx, cudaMemcpy(ctx->top_sh_pos.p, pos.data(), pos.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  std::vector<int32_t> idx((size_t)ctx->tree.n_top, -1);
+  for (int32_t i = 0; i < ctx->n_shared; ++i) idx[pos[i]] = i;
+  NXFX_CUDA(ctx, ctx->top_sh_idx.alloc(idx.size()));
+  NXFX_CUDA(ctx, cudaMemcpy(ctx->top_sh_idx.p, idx.data(), idx.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
   // level ranges: shared nodes live in levels [0, sh_lmax], private ones in [pr_lmin, nl)
   const std::vector<int32_t>& lv = ctx->tree.top_lvl_h;
   const int nl = (int)lv.size() - 1;
@@ -143,6 +148,18 @@ int update_top_shared(nxfx_ctx* ctx) {
       if (is_sh[n - ctx->tree.top_b0]) ctx->tree.sh_lmax = L;
       else ctx->tree.pr_lmin = std::min(ctx->tree.pr_lmin, L);
     }
+  return NXFX_OK;
+}
+
+// continuous pressure on a partitioned network: weights of the nodal pressure rows in the local norms (needs the
+// shared list and the condensation tables, whichever comes last builds it)
+int update_pressure_weight(nxfx_ctx* ctx) {
+  ctx->p_nonshared.release();
+  if (!ctx->generic || !ctx->cond.set || !ctx->cond.cont || !ctx->lam_weight.p || ctx->n_shared == 0) return NXFX_OK;
+  std::vector<double> w((size_t)ctx->n_nodes, 1.0);
+  for (int32_t lm : ctx->shared_lm_h) w[ctx->cond.bif_node_h[lm]] = 0.0;
+  NXFX_CUDA(ctx, ctx->p_nonshared.alloc(w.size()));
+  NXFX_CUDA(ctx, cudaMemcpy(ctx->p_nonshared.p, w.data(), w.size() * sizeof(double), cudaMemcpyHostToDevice));
   return NXFX_OK;
 }
 
@@ -433,7 +450,8 @@ int cond_rhs_threads(const nxfx_ctx* ctx) {
   return (int)t;
 }
 
-int do_cond_setup(nxfx_ctx* ctx) {
+// everything of the factorisation below the top chunk: edge factors, nodal blocks, bottom chunks
+int cond_factor_local(nxfx_ctx* ctx) {
   NXFX_REQUIRE(ctx, ctx->cond.set, "nxfx_set_condensation has not been called");
   NXFX_REQUIRE(ctx, ctx->tree.set, "nxfx_set_tree_schedule has not been called");
   Net g = make_net(ctx);
@@ -451,18 +469,23 @@ int do_cond_setup(nxfx_ctx* ctx) {
     NXFX_LAUNCH(ctx, cond_node_kernel<true>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, c, nullptr);
     const int nb = ctx->tree.n_chunks - 1;
     if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<0>, nb, 1024, 0, t, c, 0);
-    NXFX_LAUNCH(ctx, btree_sweep_kernel<0>, 1, 1024, 0, t, c, nb);
   }
+  return NXFX_OK;
+}
+
+int do_cond_setup(nxfx_ctx* ctx) {
+  int rc = cond_factor_local(ctx);
+  if (rc) return rc;
+  if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<0>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
   ctx->pc_ready = true;
   ctx->pc_mat = ctx->cur->id;
   return NXFX_OK;
 }
 
-int do_cond_apply(nxfx_ctx* ctx, const double* r, double* z, bool add) {
-  NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
+// y0, h per edge, nodal right-hand sides, forward sweep of the bottom chunks (lam_w: see cond_node_kernel)
+int cond_forward_local(nxfx_ctx* ctx, const double* r, const double* lam_w) {
   Net g = make_net(ctx);
   CondDev c = make_cond(ctx);
-  TreeDev t = make_tree(ctx);
   const int tr = cond_rhs_threads(ctx);
   if (tr > 0) {
     NXFX_LAUNCH(ctx, cond_edge_rhs_kernel<true>, (int)cdiv(ctx->E, tr), tr, (size_t)c.n_max * sizeof(double) * tr, g, c, r);
@@ -470,16 +493,33 @@ int do_cond_apply(nxfx_ctx* ctx, const double* r, double* z, bool add) {
     NXFX_LAUNCH(ctx, cond_edge_rhs_kernel<false>, (int)cdiv(ctx->E, kCondThreads), kCondThreads, 0, g, c, r);
   }
   if (ctx->n_bif > 0) {
-    NXFX_LAUNCH(ctx, cond_node_kernel<false>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, c, r);
+    TreeDev t = make_tree(ctx);
+    NXFX_LAUNCH(ctx, cond_node_kernel<false>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, c, r, lam_w);
     const int nb = ctx->tree.n_chunks - 1;
     if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<1>, nb, 1024, 0, t, c, 0);
-    NXFX_LAUNCH(ctx, btree_sweep_kernel<3>, 1, 1024, 0, t, c, nb);
-    if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<2>, nb, 1024, 0, t, c, 0);
   }
+  return NXFX_OK;
+}
+
+// backward sweep of the bottom chunks, back-substitution on the edges
+int cond_backward_local(nxfx_ctx* ctx, double* z, bool add) {
+  Net g = make_net(ctx);
+  CondDev c = make_cond(ctx);
+  TreeDev t = make_tree(ctx);
+  const int nb = ctx->tree.n_chunks - 1;
+  if (ctx->n_bif > 0 && nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<2>, nb, 1024, 0, t, c, 0);
   const int grid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kCondThreads);
   if (add) NXFX_LAUNCH(ctx, cond_backsub_kernel<true>, grid, kCondThreads, 0, g, t, c, z);
   else NXFX_LAUNCH(ctx, cond_backsub_kernel<false>, grid, kCondThreads, 0, g, t, c, z);
   return NXFX_OK;
+}
+
+int do_cond_apply(nxfx_ctx* ctx, const double* r, double* z, bool add) {
+  NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
+  int rc = cond_forward_local(ctx, r, nullptr);
+  if (rc) return rc;
+  if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<3>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
+  return cond_backward_local(ctx, z, add);
 }
 
 int do_pc_setup(nxfx_ctx* ctx) {
@@ -1027,9 +1067,11 @@ int nxfx_set_network(nxfx_ctx* ctx, int32_t n_nodes, int32_t n_edges, int32_t gd
   ctx->shared_lm.release();
   ctx->shared_lm_h.clear();
   ctx->top_sh_pos.release();
+  ctx->top_sh_idx.release();
   ctx->tree.t_of_bif_h.clear();
   ctx->lam_weight.release();
   ctx->lam_nonshared.release();
+  ctx->p_nonshared.release();
   ctx->tree.set = false;
   ctx->n_nodes = n_nodes; ctx->E = n_edges; ctx->gdim = gdim; ctx->N = N; ctx->n_bif = n_bif;
   ctx->n_inc = n_inc; ctx->nv = nv; ctx->nc = nc; ctx->nq = nq; ctx->poff = nq; ctx->loff = nq + nc;
@@ -1616,6 +1658,7 @@ int nxfx_set_condensation(nxfx_ctx* ctx, int32_t continuous_pressure, int32_t fl
   NXFX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   k.n_max = n_max; k.kl = kl; k.per_edge = flux_dofs_per_edge; k.pcell_base = pcell_base; k.pcell_stride = pcell_stride;
   k.cont = continuous_pressure ? 1 : 0;
+  k.bif_node_h.assign(bif_node, bif_node + ctx->n_bif);
   NXFX_CUDA(ctx, cudaFuncSetAttribute(cond_edge_rhs_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCondSmemMax));
   NXFX_CUDA(ctx, cudaFuncSetAttribute(cond_factor_group_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCondSmemMax));
   NXFX_CUDA(ctx, cudaFuncSetAttribute(cond_factor_group_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCondSmemMax));
@@ -1631,7 +1674,7 @@ int nxfx_set_condensation(nxfx_ctx* ctx, int32_t continuous_pressure, int32_t fl
   NXFX_CUDA(ctx, k.br.alloc(2 * nb));
   NXFX_CUDA(ctx, k.bz.alloc(2 * nb));
   k.set = true;
-  return NXFX_OK;
+  return update_pressure_weight(ctx);
 }
 
 // ---- (6) multi-GPU: partitioned network ----------------------------------------------------------
@@ -1651,15 +1694,49 @@ int nxfx_set_shared(nxfx_ctx* ctx, int32_t n_shared, const int32_t* shared_lm, c
   NXFX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   ctx->n_shared = n_shared;
   ctx->shared_lm_h.assign(shared_lm, shared_lm + n_shared);
+  if ((rc = update_pressure_weight(ctx))) return rc;
   return update_top_shared(ctx);
 }
 
 static int dist_ready(nxfx_ctx* ctx, const double* buf) {
-  NXFX_REQUIRE(ctx, ctx->tree.set && ctx->tree.fast_ok && ctx->tree.n_chunks >= 1 && buf,
+  // (the block sweeps of the table-driven path run out of global memory: any schedule fits them)
+  NXFX_REQUIRE(ctx, ctx->tree.set && (ctx->tree.fast_ok || ctx->generic) && ctx->tree.n_chunks >= 1 && buf,
                "needs a tree schedule that fits the shared-memory sweeps and a buffer");
+  NXFX_REQUIRE(ctx, !ctx->generic || ctx->cond.set, "nxfx_set_condensation has not been called");
   NXFX_REQUIRE(ctx, ctx->cur && ctx->cur->acc_count <= 1,
                "the partitioned solve does not take a matrix accumulated over several assemblies");
   NXFX_REQUIRE(ctx, ctx->n_shared == 0 || ctx->top_sh_pos.p, "nxfx_set_shared / nxfx_set_tree_schedule have not both been called");
+  return NXFX_OK;
+}
+
+// doubles of the three exchanged sections (see nxfx_exchange_sizes)
+static void exchange_sizes(const nxfx_ctx* ctx, int32_t* setup, int32_t* apply, int32_t* residual) {
+  const int32_t nt = std::max(ctx->n_shared, 1);
+  const bool cont = ctx->generic && ctx->cond.cont;
+  *setup = (ctx->generic ? 12 : 2) * nt;
+  *apply = (ctx->generic ? 2 : 1) * nt;
+  *residual = (cont ? 3 : 1) * ctx->n_shared + 2;
+}
+
+int nxfx_exchange_sizes(nxfx_ctx* ctx, int32_t* setup, int32_t* apply, int32_t* residual) {
+  if (!ctx || !setup || !apply || !residual) return NXFX_ERR_INVALID;
+  NXFX_REQUIRE(ctx, ctx->tree.set && ctx->tree.n_chunks >= 1, "no tree schedule");
+  NXFX_REQUIRE(ctx, !ctx->generic || ctx->cond.set, "nxfx_set_condensation has not been called");
+  exchange_sizes(ctx, setup, apply, residual);
+  return NXFX_OK;
+}
+
+// table-driven path: the top chunk's half of a split phase (condense.cuh btree_top_split_kernel)
+static int cond_top_split(nxfx_ctx* ctx, bool factor, bool finish, double* buf) {
+  if (ctx->n_bif == 0) return NXFX_OK;
+  TreeDev t = make_tree(ctx);
+  CondDev c = make_cond(ctx);
+  const int top = ctx->tree.n_chunks - 1, nt = std::max(ctx->n_shared, 1);
+  const int32_t* idx = ctx->n_shared > 0 ? ctx->top_sh_idx.p : nullptr;
+  if (factor && !finish) NXFX_LAUNCH(ctx, (btree_top_split_kernel<true, kPartial>), 1, 1024, 0, t, c, top, idx, nt, buf);
+  else if (factor) NXFX_LAUNCH(ctx, (btree_top_split_kernel<true, kFinish>), 1, 1024, 0, t, c, top, idx, nt, buf);
+  else if (!finish) NXFX_LAUNCH(ctx, (btree_top_split_kernel<false, kPartial>), 1, 1024, 0, t, c, top, idx, nt, buf);
+  else NXFX_LAUNCH(ctx, (btree_top_split_kernel<false, kFinish>), 1, 1024, 0, t, c, top, idx, nt, buf);
   return NXFX_OK;
 }
 
@@ -1675,6 +1752,11 @@ int nxfx_pc_setup_begin(nxfx_ctx* ctx, double* buf) {
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
   NXFX_REQUIRE(ctx, is_assembled(ctx), "assemble the matrix before pc_setup");
+  if (ctx->generic) {
+    if ((rc = cond_factor_local(ctx)) || (rc = cond_top_split(ctx, true, false, buf))) return rc;
+    ctx->bottom_factored = true;
+    return NXFX_OK;
+  }
   auto& s = ctx->tree;
   TreeDev t = make_tree(ctx);
   const int nb = s.n_chunks - 1;
@@ -1695,6 +1777,13 @@ int nxfx_pc_setup_end(nxfx_ctx* ctx, double* buf) {
   if (!ctx) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
+  if (ctx->generic) {
+    NXFX_REQUIRE(ctx, ctx->bottom_factored, "nxfx_pc_setup_begin has not been run");
+    if ((rc = cond_top_split(ctx, true, true, buf))) return rc;
+    ctx->pc_ready = true;
+    ctx->pc_mat = ctx->cur->id;
+    return NXFX_OK;
+  }
   NXFX_LAUNCH(ctx, (tree_top_kernel<true, kFinish>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), ctx->tree.n_chunks - 1, buf);
   ctx->pc_ready = true;
   ctx->pc_mat = ctx->cur->id;
@@ -1709,6 +1798,10 @@ int nxfx_pc_apply_begin(nxfx_ctx* ctx, const double* r, double* buf) {
   // nxfx_pc_setup_end, so that setup and first application share one all-reduce
   NXFX_REQUIRE(ctx, ctx->pc_ready || ctx->bottom_factored, "nxfx_pc_setup_begin has not been run");
   NXFX_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(r) & 15) == 0, "vectors must be 16-byte aligned");
+  if (ctx->generic) {
+    if ((rc = cond_forward_local(ctx, r, ctx->lam_weight.p))) return rc;
+    return cond_top_split(ctx, false, false, buf);
+  }
   Net g = make_net(ctx);
   TreeDev t = make_tree(ctx);
   const int nb = ctx->tree.n_chunks - 1;
@@ -1728,6 +1821,11 @@ int nxfx_pc_apply_end(nxfx_ctx* ctx, const double* r, double* z, double* buf, in
   if (!ctx || !r || !z) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
+  if (ctx->generic) {
+    NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
+    if ((rc = cond_top_split(ctx, false, true, buf))) return rc;
+    return cond_backward_local(ctx, z, add != 0);
+  }
   Net g = make_net(ctx);
   TreeDev t = make_tree(ctx);
   const int nb = ctx->tree.n_chunks - 1;
@@ -1754,10 +1852,11 @@ int nxfx_pc_setup_apply_begin(nxfx_ctx* ctx, const double* r, double* buf) {
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
   NXFX_REQUIRE(ctx, is_assembled(ctx), "assemble the matrix before pc_setup");
-  const int nt = std::max(ctx->n_shared, 1);
-  if (ctx->N != 1) {
+  int32_t ns, na, nr;
+  exchange_sizes(ctx, &ns, &na, &nr);
+  if (ctx->N != 1 || ctx->generic) {
     if ((rc = nxfx_pc_setup_begin(ctx, buf))) return rc;
-    return nxfx_pc_apply_begin(ctx, r, buf + 2 * (size_t)nt);
+    return nxfx_pc_apply_begin(ctx, r, buf + ns);
   }
   NXFX_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(r) & 15) == 0, "vectors must be 16-byte aligned");
   auto& s = ctx->tree;
@@ -1775,10 +1874,11 @@ int nxfx_pc_setup_apply_end(nxfx_ctx* ctx, const double* r, double* z, double* b
   if (!ctx || !r || !z) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
-  const int nt = std::max(ctx->n_shared, 1);
-  if (ctx->N != 1) {
+  int32_t ns, na, nr;
+  exchange_sizes(ctx, &ns, &na, &nr);
+  if (ctx->N != 1 || ctx->generic) {
     if ((rc = nxfx_pc_setup_end(ctx, buf))) return rc;
-    return nxfx_pc_apply_end(ctx, r, z, buf + 2 * (size_t)nt, 0);
+    return nxfx_pc_apply_end(ctx, r, z, buf + ns, 0);
   }
   NXFX_REQUIRE(ctx, ctx->bottom_factored, "nxfx_pc_setup_apply_begin has not been run");
   auto& s = ctx->tree;
@@ -1817,6 +1917,9 @@ int nxfx_comm_destroy(nxfx_ctx* ctx) {
 
 int nxfx_comm_create(nxfx_ctx* ctx, int32_t rank, int32_t nranks, void* handle_out, int32_t* slot_doubles) {
   if (!ctx || !handle_out) return NXFX_ERR_INVALID;
+  if (ctx->generic)
+    return fail(ctx, NXFX_ERR_UNSUPPORTED, "the in-kernel exchange is implemented for flux degree 1 / pressure degree 0 "
+                "only; use the split phases (nxfx_pc_*_begin/_end) instead");
   NXFX_REQUIRE(ctx, nranks >= 2 && nranks <= kMaxPeers && rank >= 0 && rank < nranks, "bad rank / nranks");
   NXFX_REQUIRE(ctx, ctx->tree.set && ctx->lam_nonshared.p, "call nxfx_set_tree_schedule and nxfx_set_shared first");
   // the exchange lives in the fused cooperative tree kernel: one cell per edge, all chunks of this rank co-resident
@@ -1869,6 +1972,9 @@ int nxfx_pack_shared(nxfx_ctx* ctx, const double* v, double* buf) {
   if (ctx->n_shared > 0)
     NXFX_LAUNCH(ctx, pack_shared_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->loff,
                 ctx->shared_lm.p, v, buf);
+  if (ctx->n_shared > 0 && ctx->generic && ctx->cond.set && ctx->cond.cont)
+    NXFX_LAUNCH(ctx, pack_nodal_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->nq,
+                ctx->shared_lm.p, ctx->cond.bif_node.p, v, buf + ctx->n_shared);
   return NXFX_OK;
 }
 
@@ -1877,6 +1983,9 @@ int nxfx_unpack_shared(nxfx_ctx* ctx, const double* buf, double* v) {
   if (ctx->n_shared > 0)
     NXFX_LAUNCH(ctx, unpack_shared_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->loff,
                 ctx->shared_lm.p, buf, v);
+  if (ctx->n_shared > 0 && ctx->generic && ctx->cond.set && ctx->cond.cont)
+    NXFX_LAUNCH(ctx, unpack_nodal_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->nq,
+                ctx->shared_lm.p, ctx->cond.bif_node.p, buf + ctx->n_shared, v);
   return NXFX_OK;
 }
 
@@ -1885,6 +1994,22 @@ int nxfx_residual_partial(nxfx_ctx* ctx, const double* b, const double* x, doubl
   NXFX_REQUIRE(ctx, ctx->has_pattern && ctx->lam_nonshared.p, "nxfx_set_shared has not been called");
   NXFX_REQUIRE(ctx, is_assembled(ctx), "matrix has not been assembled");
   int rc;
+  if (ctx->generic) {
+    // [lam rows of r | P rows of r | P rows of b | norm partials without any shared row]: a plain residual, then
+    // the packs and a weighted-norm kernel that also skips the nodal pressure rows of the shared bifurcations
+    NXFX_REQUIRE(ctx, ctx->cond.set, "nxfx_set_condensation has not been called");
+    const bool cont = ctx->cond.cont && ctx->n_shared > 0;
+    if ((rc = do_residual(ctx, b, x, r, slot(ctx, 0)))) return rc;
+    if ((rc = nxfx_pack_shared(ctx, r, buf))) return rc;
+    if (cont)
+      NXFX_LAUNCH(ctx, pack_nodal_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->nq,
+                  ctx->shared_lm.p, ctx->cond.bif_node.p, b, buf + 2 * (size_t)ctx->n_shared);
+    const int n = (int)ctx->ndofs, nr = (cont ? 3 : 1) * ctx->n_shared;
+    NXFX_LAUNCH(ctx, weighted_norm2_pair_kernel, vec_grid(ctx, n), kThreads, 0, n, (int)ctx->loff, r, ctx->lam_nonshared.p,
+                b, ctx->lam_weight.p, ctx->scal.p, ctx->ticket.p, buf + nr, (int)ctx->nq, cont ? ctx->n_nodes : 0,
+                cont ? ctx->p_nonshared.p : nullptr);
+    return NXFX_OK;
+  }
   if (ctx->pipe_ok) {  // the weighted partial norms come out of the residual kernel itself
     const int ntiles = (int)cdiv(ctx->ndofs, kTileRows);
     const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
@@ -1904,6 +2029,13 @@ int nxfx_residual_partial(nxfx_ctx* ctx, const double* b, const double* x, doubl
 int nxfx_residual_finish(nxfx_ctx* ctx, const double* buf, double* r, double* nrm_out) {
   if (!ctx || !buf || !r || !nrm_out) return NXFX_ERR_INVALID;
   NXFX_REQUIRE(ctx, ctx->lam_nonshared.p, "nxfx_set_shared has not been called");
+  if (ctx->generic) {
+    NXFX_REQUIRE(ctx, ctx->cond.set, "nxfx_set_condensation has not been called");
+    NXFX_LAUNCH(ctx, cond_residual_finish_kernel, 1, kThreads, 0, ctx->n_shared, (int)ctx->loff, (int)ctx->nq,
+                ctx->cond.cont && ctx->n_shared > 0 ? 1 : 0, ctx->shared_lm.p, ctx->cond.bif_node.p, ctx->lam_weight.p,
+                buf, r, nrm_out);
+    return NXFX_OK;
+  }
   NXFX_LAUNCH(ctx, residual_finish_kernel, 1, kThreads, 0, ctx->n_shared, (int)ctx->loff, ctx->shared_lm.p, buf, r, nrm_out);
   return NXFX_OK;
 }

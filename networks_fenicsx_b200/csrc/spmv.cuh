@@ -384,18 +384,21 @@ weighted_norm2_kernel(int n, int loff, const double* __restrict__ v, const doubl
 
 // out[0] = sum w1_i r_i^2, out[1] = sum w2_i b_i^2 in one pass (weights as above; multi-GPU residual:
 // w1 excludes every replicated multiplier row -- their partial sums are O(1) and only cancel in the
-// all-reduce, so they must never enter a local norm -- w2 counts owned rows)
+// all-reduce, so they must never enter a local norm -- w2 counts owned rows).  pw (nullptr: none): extra weight of the rows p0 .. p0 + np - 1 in both sums -- 0 on
+// the nodal pressure rows of the shared bifurcations (continuous pressure), partial sums like the multiplier rows
 __global__ void __launch_bounds__(kThreads)
 weighted_norm2_pair_kernel(int n, int loff, const double* __restrict__ r, const double* __restrict__ w1,
                            const double* __restrict__ b, const double* __restrict__ w2, double* partial,
-                           unsigned int* ticket, double* out) {
+                           unsigned int* ticket, double* out, int p0 = 0, int np = 0,
+                           const double* __restrict__ pw = nullptr) {
   __shared__ double red[kThreads / 32];
   double a1 = 0.0, a2 = 0.0;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const double ri = r[i], bi = b[i];
     const bool lam = i >= loff;
-    a1 += (lam ? w1[i - loff] : 1.0) * ri * ri;
-    a2 += (lam ? w2[i - loff] : 1.0) * bi * bi;
+    const double wp = (pw && i >= p0 && i < p0 + np) ? pw[i - p0] : 1.0;
+    a1 += (lam ? w1[i - loff] : wp) * ri * ri;
+    a2 += (lam ? w2[i - loff] : wp) * bi * bi;
   }
   double mine[2] = {block_sum<kThreads>(a1, red), block_sum<kThreads>(a2, red)};
   finish_partials<kThreads, 2>(mine, partial, gridDim.x, ticket, out, red);

@@ -12,6 +12,11 @@ ranks.  Everything that couples ranks is additive and small (n_top doubles):
   chunk redundantly and back-substitutes its own chunks;
 * norms: owned entries only, one all-reduce of the scalars.
 
+Higher-order elements go the same way: the shared nodes carry 2 x 2 blocks {P_b, lam_b} (their
+diagonal blocks, coupling blocks and nodal right-hand sides are exchanged), and with a continuous
+pressure the nodal pressure rows of the shared bifurcations are partial sums like their multiplier
+rows.  The section sizes come from the library (``nxfx_exchange_sizes``).
+
 Host code (NumPy) in this file; collectives through ``torch.distributed`` (NCCL on GPUs, gloo in
 the CPU tests).
 """
@@ -144,11 +149,13 @@ class DistributedSolver:
             per GPU); ``"nccl"``: split phases around ``torch.distributed`` all-reduces;
             ``"auto"``: peer when available.
         device: CUDA ordinal of this rank.
+        flux_degree, pressure_degree: element degrees as in :class:`HydraulicNetworkAssembler` (the peer
+            exchange is implemented for 1 / 0 only: other degrees use the all-reduces).
     """
 
     def __init__(self, graph: ArrayGraph, N: int, p_bc_ex, f=None, R=None, device: int = 0,
                  color_strategy="smallest_last", chunk_nodes: int = CHUNK_NODES, group=None,
-                 exchange: str = "auto"):
+                 exchange: str = "auto", flux_degree: int = 1, pressure_degree: int = 0):
         import torch.distributed as dist
 
         from .assembly import HydraulicNetworkAssembler
@@ -160,7 +167,7 @@ class DistributedSolver:
         # the sub-network is handed over explicitly (comm = serial): no second partitioning inside
         mesh = NetworkMesh(part.graph, N=N, color_strategy=color_strategy, device=device,
                            node_degree=part.node_degree, comm=SerialComm())
-        assembler = HydraulicNetworkAssembler(mesh)
+        assembler = HydraulicNetworkAssembler(mesh, flux_degree=flux_degree, pressure_degree=pressure_degree)
         assembler.compute_forms(p_bc_ex=p_bc_ex, f=self._restrict(f, N, graph), R=self._restrict(R, N, graph))
         solver = Solver(assembler, schedule=part.schedule)
         self._attach(part, mesh, assembler, solver, group, exchange)
@@ -194,8 +201,11 @@ class DistributedSolver:
         weight = np.ascontiguousarray(part.lam_weight, dtype=np.float64)
         self.dev.call("nxfx_set_shared", shared.size, _lib.as_i32p(shared), _lib.as_f64p(weight))
         cuda = torch.device("cuda", device)
-        self._top = torch.zeros(3 * max(part.n_top, 1), dtype=torch.float64, device=cuda)  # [setup 2n | apply n]
-        self._sh = torch.zeros(shared.size + 2, dtype=torch.float64, device=cuda)  # halo rows + 2 norm partials
+        n_setup, n_apply, n_res = C.c_int32(0), C.c_int32(0), C.c_int32(0)
+        self.dev.call("nxfx_exchange_sizes", C.byref(n_setup), C.byref(n_apply), C.byref(n_res))
+        self._n_apply = n_apply.value
+        self._top = torch.zeros(n_setup.value + n_apply.value, dtype=torch.float64, device=cuda)  # [setup | apply]
+        self._sh = torch.zeros(n_res.value, dtype=torch.float64, device=cuda)  # halo rows + 2 norm partials
         self._nrm = torch.zeros(2 * 40, dtype=torch.float64, device=cuda)
         self._r = self.dev.empty(self.assembler.num_dofs)
         self.n_dofs_global = int(self._allreduce_scalar(self._owned_dofs()))
@@ -233,8 +243,9 @@ class DistributedSolver:
                 self.dev.call("nxfx_comm_connect", C.c_char_p(blob))
             except RuntimeError as exc:
                 ok, err = 0, str(exc)
-        else:
-            ok, err = 0, "a rank could not create its exchange buffer (or the slot sizes differ)"
+        else:  # keep this rank's own reason when it has one (e.g. a higher-order context)
+            err = err if not ok else "a rank could not create its exchange buffer (or the slot sizes differ)"
+            ok = 0
         if self._allreduce_scalar(float(ok)) == float(self.world):
             self.exchange = "peer"
             dist.barrier(group=self._group)  # every buffer is mapped and zeroed before the first flag is written
@@ -258,7 +269,9 @@ class DistributedSolver:
         return arr
 
     def _owned_dofs(self) -> int:
-        return int(self.assembler.num_dofs - self.part.n_top + (self.part.n_top if self.rank == 0 else 0))
+        # replicated: the multipliers of the shared nodes and, for a continuous pressure, their nodal pressures
+        n_sh = self.part.n_top * (2 if self.assembler.degrees[1] >= 1 else 1)
+        return int(self.assembler.num_dofs - n_sh + (n_sh if self.rank == 0 else 0))
 
     def _allreduce_scalar(self, v: float) -> float:
         t = self._torch.tensor([float(v)], dtype=self._torch.float64, device=self._top.device)
@@ -274,7 +287,7 @@ class DistributedSolver:
     def _apply(self, r_ptr, z_ptr, add: int) -> None:
         top = self._ptr(self._top)
         self.dev.call("nxfx_pc_apply_begin", r_ptr, top)
-        self._dist.all_reduce(self._top[: self.part.n_top], group=self._group)
+        self._dist.all_reduce(self._top[: self._n_apply], group=self._group)
         self.dev.call("nxfx_pc_apply_end", r_ptr, z_ptr, top, add)
 
     def solve(self, refine_steps: int = 1, final_residual: bool = False, refine_rtol: float = 1e-13):
@@ -290,7 +303,7 @@ class DistributedSolver:
             return self._solve_peer(b, x, refine_steps, final_residual, refine_rtol)
         # factorisation and first application share one all-reduce: the forward sweep of the bottom
         # chunks only needs their own factors
-        top = self._ptr(self._top)  # [partial pivots | link conductances | partial rhs], 3 n_top
+        top = self._ptr(self._top)  # [setup: partial pivots / blocks, link couplings | apply: partial rhs]
         dev.call("nxfx_pc_setup_apply_begin", b, top)
         self._dist.all_reduce(self._top, group=self._group)
         dev.call("nxfx_pc_setup_apply_end", b, x, top)
@@ -342,7 +355,7 @@ class DistributedSolver:
 
     def _residual(self, b, x, k: int) -> None:
         """r = b - A x with consistent shared rows and the global [||r||^2, ||b||^2] in slot k:
-        one all-reduce of n_shared + 2 doubles."""
+        one all-reduce of the shared rows + 2 doubles."""
         dev = self.dev
         sh = self._ptr(self._sh)
         dev.call("nxfx_residual_partial", b, x, self._r.c_ptr, sh)
@@ -366,3 +379,44 @@ class DistributedSolver:
         lam = x[nq + E * N:]
         own = self.part.lam_weight > 0
         return self.part.global_edges, q, p, self.part.global_bif[own], lam[own]
+
+    def dof_values(self) -> dict:
+        """The local solution in a form that places into the WHOLE network's numbering for any degree:
+
+        * ``edges`` (global edge ids), ``flux`` ``[E_loc, fd N + 1]`` (the edge's vertex dofs, then the interior
+          dofs cell by cell) and ``pressure`` ``[E_loc, k]``: DG0: the N cell values; continuous: the N - 1
+          interior vertices, then the ``N (pd - 1)`` cell-interior dofs cell by cell;
+        * ``nodes`` / ``node_pressure``: global node id and vertex pressure of the graph nodes this rank owns
+          (continuous pressure; the nodal pressure of a shared bifurcation is owned by rank 0);
+        * ``multipliers`` / ``lam``: global multiplier id and value of the multipliers this rank owns."""
+        x = self.local_solution()
+        N = self.mesh.cells_per_edge
+        fd, pd = self.assembler.degrees
+        ge = self.part.global_edges
+        E = ge.size
+        per_edge = fd * N + 1
+        fb = self.mesh.edge_slot.astype(np.int64) * per_edge
+        flux = x[fb[:, None] + np.arange(per_edge)[None, :]]
+        nq = E * per_edge
+        n_nodes = self.part.global_nodes.size
+        e = np.arange(E)[:, None]
+        if pd == 0:
+            pressure = x[nq + e * N + np.arange(N)[None, :]]
+            nodes = np.zeros(0, dtype=np.int64)
+            node_p = np.zeros(0)
+        else:
+            nv = n_nodes + (N - 1) * E
+            inner = nq + n_nodes + e * (N - 1) + np.arange(N - 1)[None, :]
+            cell = nq + nv + e * (N * (pd - 1)) + np.arange(N * (pd - 1))[None, :]
+            pressure = x[np.concatenate([inner, cell], axis=1)]
+            shared_nodes = self.mesh.bifurcation_values[self.part.shared_lm]
+            own = np.ones(n_nodes, dtype=bool)
+            if self.rank != 0:
+                own[shared_nodes] = False
+            local = np.flatnonzero(own)
+            nodes = self.part.global_nodes[local]
+            node_p = x[nq + local]
+        loff = x.size - self.part.global_bif.size
+        own_lm = self.part.lam_weight > 0
+        return {"edges": ge, "flux": flux, "pressure": pressure, "nodes": nodes, "node_pressure": node_p,
+                "multipliers": self.part.global_bif[own_lm], "lam": x[loff:][own_lm]}

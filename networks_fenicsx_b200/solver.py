@@ -93,8 +93,6 @@ class Solver:
         # partitioned network (NetworkMesh under torchrun): the solve goes through the distributed layer
         self._dist = None
         if getattr(nm, "_partition", None) is not None and not getattr(self, "_no_dist", False):
-            if assembler.is_generic:
-                raise NotImplementedError("a network cut over several GPUs needs flux degree 1 / pressure degree 0")
             from .distributed import DistributedSolver  # noqa: PLC0415
 
             self._dist = DistributedSolver.from_solver(self, nm._partition)
