@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define NXFX_ABI_VERSION 1
+#define NXFX_ABI_VERSION 2
 
 typedef struct nxfx_ctx nxfx_ctx;
 
@@ -266,7 +266,7 @@ int nxfx_set_condensation(nxfx_ctx* ctx, int32_t continuous_pressure, int32_t fl
  *                            the same on every rank (ascending global node id); they must belong to
  *                            the LAST chunk of the schedule
  *   lam_weight_h [n_bif]     1 where this rank counts the multiplier row (norms, -r_lambda), else 0
- *   buf_d                    caller-owned device buffer, n_shared-sized sections (nxfx_top_size)
+ *   buf_d                    caller-owned device buffer, sections sized by nxfx_exchange_sizes
  *   nxfx_pc_setup_begin  -> buf = [partial pivots | link conductances] of the shared nodes (2 n_shared)
  *   nxfx_pc_setup_end    <- all-reduced buf: factorises the top chunk
  *   nxfx_pc_apply_begin  -> buf[0:n_shared] = partial right-hand side of the shared nodes (may be called
@@ -277,9 +277,6 @@ int nxfx_set_condensation(nxfx_ctx* ctx, int32_t continuous_pressure, int32_t fl
  *                        doubles [partial pivots | link conductances | partial right-hand side],
  *                        one all-reduce in between, z = P^{-1} r.  With one cell per edge the
  *                        bottom chunks are factorised WHILE their right-hand sides are eliminated.
- *   nxfx_pack_shared / nxfx_unpack_shared  shared multiplier rows of a vector <-> buf (after
- *                        y = A x these rows are partial sums)
- *   nxfx_norm2_owned     out_d[0] = sum of squares over the entries this rank owns (async)
  *   nxfx_residual_partial  r = b - A x (local part) and buf = [shared rows of r | partial ||r||^2
  *                        over the non-shared owned rows | owned ||b||^2]  (n_shared + 2 doubles)
  *   nxfx_residual_finish <- all-reduced buf: shared rows written back to r, nrm_out_d = [||r||^2,
@@ -300,8 +297,7 @@ int nxfx_set_condensation(nxfx_ctx* ctx, int32_t continuous_pressure, int32_t fl
  * the full row) and the multiplier rows weighted by lam_weight (replicated after _residual_finish;
  * zero in b).  nxfx_residual_finish therefore writes the multiplier rows back replicated and the
  * nodal pressure rows on the owner only (lam_weight 1, the others 0), and ||b||^2 takes the shared
- * P rows of b from the all-reduced buffer, so every shared row counts once in both norms.  With
- * those degrees nxfx_pack_shared / nxfx_unpack_shared move [lam rows | P rows] (2 n_shared).
+ * P rows of b from the all-reduced buffer, so every shared row counts once in both norms.
  * The peer exchange (nxfx_comm_create) is flux degree 1 / pressure degree 0 only and returns
  * NXFX_ERR_UNSUPPORTED on such a ctx.                                                          */
 int nxfx_set_shared(nxfx_ctx* ctx, int32_t n_shared, const int32_t* shared_lm_h,
@@ -323,7 +319,6 @@ int nxfx_comm_create(nxfx_ctx* ctx, int32_t rank, int32_t nranks, void* handle_o
                      int32_t* slot_doubles);
 int nxfx_comm_connect(nxfx_ctx* ctx, const void* handles_all_h);
 int nxfx_comm_destroy(nxfx_ctx* ctx);
-int nxfx_top_size(nxfx_ctx* ctx, int32_t* n_shared); /* size of one exchanged section */
 /* doubles of the exchanged sections of the host-driven path, for either element family:
  * setup (nxfx_pc_setup_begin), apply (nxfx_pc_apply_begin; _setup_apply_* take setup + apply, the
  * application's part at offset setup) and residual (nxfx_residual_partial).  P1/DG0: 2 nt, nt and
@@ -335,9 +330,6 @@ int nxfx_pc_apply_begin(nxfx_ctx* ctx, const double* r_d, double* buf_d);
 int nxfx_pc_apply_end(nxfx_ctx* ctx, const double* r_d, double* z_d, double* buf_d, int add);
 int nxfx_pc_setup_apply_begin(nxfx_ctx* ctx, const double* r_d, double* buf_d);
 int nxfx_pc_setup_apply_end(nxfx_ctx* ctx, const double* r_d, double* z_d, double* buf_d);
-int nxfx_pack_shared(nxfx_ctx* ctx, const double* v_d, double* buf_d);
-int nxfx_unpack_shared(nxfx_ctx* ctx, const double* buf_d, double* v_d);
-int nxfx_norm2_owned(nxfx_ctx* ctx, const double* v_d, double* out_d);
 int nxfx_residual_partial(nxfx_ctx* ctx, const double* b_d, const double* x_d, double* r_d,
                           double* buf_d);
 int nxfx_residual_finish(nxfx_ctx* ctx, const double* buf_d, double* r_d, double* nrm_out_d);

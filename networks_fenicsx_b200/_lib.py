@@ -129,7 +129,6 @@ SIGNATURES = {
     "nxfx_comm_create": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(C.c_int32)]),
     "nxfx_comm_connect": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_comm_destroy": (C.c_int, [C.c_void_p]),
-    "nxfx_top_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
     "nxfx_exchange_sizes": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "nxfx_pc_setup_begin": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_pc_setup_end": (C.c_int, [C.c_void_p, C.c_void_p]),
@@ -137,9 +136,6 @@ SIGNATURES = {
     "nxfx_pc_apply_end": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "nxfx_pc_setup_apply_begin": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "nxfx_pc_setup_apply_end": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "nxfx_pack_shared": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
-    "nxfx_unpack_shared": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
-    "nxfx_norm2_owned": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "nxfx_residual_partial": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "nxfx_residual_finish": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "nxfx_global_flux": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -163,7 +159,7 @@ def load() -> C.CDLL:
         fn = getattr(lib, name)  # AttributeError if the symbol is not exported
         fn.restype = restype
         fn.argtypes = argtypes
-    if lib.nxfx_abi_version() != 1:
+    if lib.nxfx_abi_version() != 2:
         raise RuntimeError("libnxfx_b200.so ABI version mismatch")
     _lib = lib
     return lib

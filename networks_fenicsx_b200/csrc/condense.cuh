@@ -595,12 +595,6 @@ pack_nodal_kernel(int n_shared, int nq, const int32_t* __restrict__ shared_lm, c
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_shared) buf[i] = v[nq + bif_node[shared_lm[i]]];
 }
-__global__ void __launch_bounds__(kThreads)
-unpack_nodal_kernel(int n_shared, int nq, const int32_t* __restrict__ shared_lm, const int32_t* __restrict__ bif_node,
-                    const double* __restrict__ buf, double* __restrict__ v) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n_shared) v[nq + bif_node[shared_lm[i]]] = buf[i];
-}
 
 // After the all-reduce of [lam rows of r | (cont) P rows of r | (cont) P rows of b | ||r||^2 | ||b||^2] (the norm
 // partials without any shared row): multiplier rows back into r replicated, nodal pressure rows back into r on the

@@ -215,6 +215,12 @@ void bind_matrix(nxfx_ctx* ctx, MatState* m) {
   if (ctx->pc_ready && ctx->pc_mat != m->id) ctx->pc_ready = false;
 }
 
+// the factors of the preconditioner now belong to the bound matrix
+void mark_factored(nxfx_ctx* ctx) {
+  ctx->pc_ready = true;
+  ctx->pc_mat = ctx->cur->id;
+}
+
 // callers that never create a matrix (plain C users of the ABI) work on matrix 0
 int ensure_matrix(nxfx_ctx* ctx) {
   if (ctx->cur) return NXFX_OK;
@@ -384,8 +390,8 @@ inline size_t vec_stride(const nxfx_ctx* ctx);
 int ensure_work(nxfx_ctx* ctx, size_t nvec);
 
 // fused: N == 1 -- the kernels evaluate the nodes' diagonal / right-hand side themselves from
-// (r, cell_rh); returns through *did_fuse whether the separate bif_* kernel is still needed.
-int tree_pass(nxfx_ctx* ctx, bool factor, const double* fuse_r = nullptr, bool fuse = false, bool* did_fuse = nullptr) {
+// (r, cell_rh), so the separate bif_*_n1 kernel is not launched.
+int tree_pass(nxfx_ctx* ctx, bool factor, const double* fuse_r = nullptr, bool fuse = false) {
   auto& s = ctx->tree;
   TreeDev t = make_tree(ctx);
   const int nb = s.n_chunks - 1;  // bottom chunks; the last chunk is the top of the forest
@@ -393,12 +399,11 @@ int tree_pass(nxfx_ctx* ctx, bool factor, const double* fuse_r = nullptr, bool f
     const int grid = std::max(nb, 1);
     unsigned int* tk = ctx->ticket.p + 1;
     FusedN1 fin{make_net(ctx), nullptr, nullptr};
-    if (did_fuse) *did_fuse = false;
     if (factor) {
-      if (fuse) { fin.cell_rh = ctx->cur->cell_rh.p; if (did_fuse) *did_fuse = true; }
+      if (fuse) fin.cell_rh = ctx->cur->cell_rh.p;
       NXFX_LAUNCH(ctx, tree_factor_kernel, grid, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, tk, 1, fin);
     } else if (s.coop_ok && nb > 0) {
-      if (fuse) { fin.r = fuse_r; fin.cell_rh = ctx->cur->cell_rh.p; if (did_fuse) *did_fuse = true; }
+      if (fuse) { fin.r = fuse_r; fin.cell_rh = ctx->cur->cell_rh.p; }
       unsigned int* fl = ctx->ticket.p + 2;
       unsigned int ep = ++s.epoch;
       int nbv = nb;
@@ -477,8 +482,7 @@ int do_cond_setup(nxfx_ctx* ctx) {
   int rc = cond_factor_local(ctx);
   if (rc) return rc;
   if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<0>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
-  ctx->pc_ready = true;
-  ctx->pc_mat = ctx->cur->id;
+  mark_factored(ctx);
   return NXFX_OK;
 }
 
@@ -522,24 +526,86 @@ int do_cond_apply(nxfx_ctx* ctx, const double* r, double* z, bool add) {
   return cond_backward_local(ctx, z, add);
 }
 
+// ---- P1/DG0 building blocks: one cell per edge (n1) or several ------------------------------------
+// n1: the node and edge kernels read the cell data themselves and move the two flux dofs of an edge with
+// one 16-byte access.  (The global-memory fallback sweeps of a schedule without fast_ok read edge_g.)
+bool n1_kernels(const nxfx_ctx* ctx) { return ctx->N == 1 && ctx->tree.fast_ok; }
+
+int check_aligned(nxfx_ctx* ctx, const double* r, const double* z = nullptr) {
+  NXFX_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(r) & 15) == 0 && (reinterpret_cast<uintptr_t>(z) & 15) == 0,
+               "vectors must be 16-byte aligned");
+  return NXFX_OK;
+}
+
+// diagonals of the nodes; bif = false: only what the edges contribute (the edge conductances)
+int node_diag(nxfx_ctx* ctx, bool bif) {
+  if (n1_kernels(ctx)) {
+    if (bif) NXFX_LAUNCH(ctx, bif_diag_n1_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx), make_tree(ctx), ctx->cur->cell_rh.p);
+    return NXFX_OK;
+  }
+  NXFX_LAUNCH(ctx, edge_conductance_kernel, (int)cdiv(ctx->E, kThreads), kThreads, 0, ctx->E, ctx->N, ctx->cur->cell_rh.p, ctx->edge_g.p);
+  if (bif) NXFX_LAUNCH(ctx, bif_diag_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx), make_tree(ctx), ctx->edge_g.p);
+  return NXFX_OK;
+}
+
+// right-hand sides of the nodes; bif = false: only the per-edge condensation
+int node_rhs(nxfx_ctx* ctx, const double* r, bool bif) {
+  Net g = make_net(ctx);
+  TreeDev t = make_tree(ctx);
+  if (n1_kernels(ctx)) {
+    if (bif) NXFX_LAUNCH(ctx, bif_rhs_n1_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, r, ctx->cur->cell_rh.p, ctx->lam_weight.p);
+    return NXFX_OK;
+  }
+  NXFX_LAUNCH(ctx, edge_condense_kernel<false>, (int)cdiv(ctx->E, kThreads), kThreads, 0, g, ctx->cur->cell_rh.p, r,
+              ctx->edge_c.p, ctx->edge_fn.p, nullptr);
+  if (bif)
+    NXFX_LAUNCH(ctx, bif_rhs_kernel<false>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, r, ctx->edge_g.p, ctx->edge_c.p,
+                ctx->edge_fn.p, ctx->lam_weight.p);
+  return NXFX_OK;
+}
+
+// z (+)= the edge unknowns from the solved nodal ones.  pdl: the n1 kernel is launched as programmatic dependent of
+// the tree kernel and stages its edge data while that finishes (the general kernel has no such wait: plain launch).
+int edge_backsub(nxfx_ctx* ctx, const double* r, double* z, bool add, bool pdl = false) {
+  Net g = make_net(ctx);
+  TreeDev t = make_tree(ctx);
+  const double* cell_rh = ctx->cur->cell_rh.p;
+  const int grid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kThreads);
+  if (!n1_kernels(ctx)) {
+    if (add) NXFX_LAUNCH(ctx, edge_backsub_kernel<true>, grid, kThreads, 0, g, t, cell_rh, r, ctx->edge_g.p, ctx->edge_c.p, z);
+    else NXFX_LAUNCH(ctx, edge_backsub_kernel<false>, grid, kThreads, 0, g, t, cell_rh, r, ctx->edge_g.p, ctx->edge_c.p, z);
+    return NXFX_OK;
+  }
+  if (!pdl) {
+    if (add) NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<true>, grid, kThreads, 0, g, t, cell_rh, r, z);
+    else NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<false>, grid, kThreads, 0, g, t, cell_rh, r, z);
+    return NXFX_OK;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)grid);
+  cfg.blockDim = dim3(kThreads);
+  cfg.stream = ctx->stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  if (add) NXFX_CUDA(ctx, cudaLaunchKernelEx(&cfg, edge_backsub_n1_kernel<true>, g, t, cell_rh, r, z));
+  else NXFX_CUDA(ctx, cudaLaunchKernelEx(&cfg, edge_backsub_n1_kernel<false>, g, t, cell_rh, r, z));
+  ctx->launches++;
+  return NXFX_OK;
+}
+
 int do_pc_setup(nxfx_ctx* ctx) {
   NXFX_REQUIRE(ctx, is_assembled(ctx), "assemble the matrix before pc_setup");
   if (ctx->generic) return do_cond_setup(ctx);
   NXFX_REQUIRE(ctx, ctx->tree.set, "nxfx_set_tree_schedule has not been called");
-  const bool n1 = ctx->N == 1 && ctx->tree.fast_ok;  // (the global-memory fallback sweeps read edge_g)
-  if (!n1)
-    NXFX_LAUNCH(ctx, edge_conductance_kernel, (int)cdiv(ctx->E, kThreads), kThreads, 0, ctx->E, ctx->N,
-                ctx->cur->cell_rh.p, ctx->edge_g.p);
-  if (ctx->n_bif > 0) {
-    if (!n1) {
-      NXFX_LAUNCH(ctx, bif_diag_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx),
-                  make_tree(ctx), ctx->edge_g.p);
-    }
-    int rc = tree_pass(ctx, true, nullptr, n1);  // N == 1: the factor kernel evaluates the diagonals itself
-    if (rc) return rc;
-  }
-  ctx->pc_ready = true;
-  ctx->pc_mat = ctx->cur->id;
+  const bool n1 = n1_kernels(ctx);
+  int rc;
+  if (!n1 && (rc = node_diag(ctx, ctx->n_bif > 0))) return rc;
+  // n1: the factor kernel evaluates the diagonals itself
+  if (ctx->n_bif > 0 && (rc = tree_pass(ctx, true, nullptr, n1))) return rc;
+  mark_factored(ctx);
   return NXFX_OK;
 }
 
@@ -551,8 +617,11 @@ bool can_fuse_setup(const nxfx_ctx* ctx) {
 
 int do_pc_setup_apply(nxfx_ctx* ctx, const double* r, double* z, bool add = false) {
   NXFX_REQUIRE(ctx, is_assembled(ctx), "assemble the matrix before pc_setup");
-  NXFX_REQUIRE(ctx, ctx->N != 1 || ((reinterpret_cast<uintptr_t>(r) & 15) == 0 && (reinterpret_cast<uintptr_t>(z) & 15) == 0),
-               "vectors must be 16-byte aligned");
+  const bool n1 = n1_kernels(ctx);  // (can_fuse_setup: fast_ok)
+  if (n1) {
+    int rc = check_aligned(ctx, r, z);
+    if (rc) return rc;
+  }
   auto& s = ctx->tree;
   Net g = make_net(ctx);
   TreeDev t = make_tree(ctx);
@@ -562,7 +631,6 @@ int do_pc_setup_apply(nxfx_ctx* ctx, const double* r, double* z, bool add = fals
   unsigned int ep = ++s.epoch;
   int nb = s.n_chunks - 1;
   PeerDev pc = make_peer(ctx, 0);  // multi-GPU: the top block exchanges its partial sums with the peers
-  const bool n1 = ctx->N == 1;
   if (!n1) {
     // several cells per edge: the per-edge condensation and the bifurcation sums are separate streaming
     // kernels; the tree kernel then stages the node arrays (diag0, tg, r) instead of the incidence table
@@ -602,24 +670,8 @@ int do_pc_setup_apply(nxfx_ctx* ctx, const double* r, double* z, bool add = fals
   }
   NXFX_CUDA(ctx, le);
   ctx->launches++;
-  ctx->pc_ready = true;
-  ctx->pc_mat = ctx->cur->id;
-  cudaLaunchConfig_t bc = {};
-  bc.gridDim = dim3((unsigned)cdiv((int64_t)ctx->E + ctx->n_bif, kThreads));
-  bc.blockDim = dim3(kThreads);
-  bc.stream = ctx->stream;
-  bc.attrs = attr + 1;
-  bc.numAttrs = 1;
-  if (!n1) {  // (the general back-substitution has no programmatic-dependency wait: plain launch)
-    const int bgrid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kThreads);
-    if (add) NXFX_LAUNCH(ctx, edge_backsub_kernel<true>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, ctx->edge_g.p, ctx->edge_c.p, z);
-    else NXFX_LAUNCH(ctx, edge_backsub_kernel<false>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, ctx->edge_g.p, ctx->edge_c.p, z);
-    return NXFX_OK;
-  }
-  if (add) NXFX_CUDA(ctx, cudaLaunchKernelEx(&bc, edge_backsub_n1_kernel<true>, g, t, (const double*)ctx->cur->cell_rh.p, r, z));
-  else NXFX_CUDA(ctx, cudaLaunchKernelEx(&bc, edge_backsub_n1_kernel<false>, g, t, (const double*)ctx->cur->cell_rh.p, r, z));
-  ctx->launches++;
-  return NXFX_OK;
+  mark_factored(ctx);
+  return edge_backsub(ctx, r, z, add, true);
 }
 
 int do_pc_apply(nxfx_ctx* ctx, int pc_type, const double* r, double* z, bool add = false) {
@@ -672,38 +724,76 @@ int do_pc_apply(nxfx_ctx* ctx, int pc_type, const double* r, double* z, bool add
   }
   NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
   if (ctx->generic) return do_cond_apply(ctx, r, z, add);
-  Net g = make_net(ctx);
-  TreeDev t = make_tree(ctx);
-  const int bgrid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kThreads);
-  if (ctx->N == 1 && ctx->tree.fast_ok) {
-    // the N == 1 kernels move the two flux dofs of an edge with one 16-byte access
-    NXFX_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(r) & 15) == 0 && (reinterpret_cast<uintptr_t>(z) & 15) == 0,
-                 "vectors must be 16-byte aligned");
-    if (ctx->n_bif > 0) {
-      // single-launch solve: the tree kernel evaluates the bifurcation right-hand sides itself
-      const bool fuse = ctx->tree.coop_ok && ctx->tree.n_chunks > 1 && !ctx->lam_weight.p;
-      if (!fuse)
-        NXFX_LAUNCH(ctx, bif_rhs_n1_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, r, ctx->cur->cell_rh.p,
-                    ctx->lam_weight.p);
-      int rc = tree_pass(ctx, false, r, fuse);
-      if (rc) return rc;
-    }
-    if (add) NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<true>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, z);
-    else NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<false>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, z);
+  const bool n1 = n1_kernels(ctx);
+  int rc;
+  if (n1 && (rc = check_aligned(ctx, r, z))) return rc;
+  // n1, single-launch solve: the tree kernel evaluates the bifurcation right-hand sides itself
+  const bool fuse = n1 && ctx->n_bif > 0 && ctx->tree.coop_ok && ctx->tree.n_chunks > 1 && !ctx->lam_weight.p;
+  if ((rc = node_rhs(ctx, r, ctx->n_bif > 0 && !fuse))) return rc;
+  if (ctx->n_bif > 0 && (rc = tree_pass(ctx, false, r, fuse))) return rc;
+  return edge_backsub(ctx, r, z, add);
+}
+
+// ---- phases of the partitioned preconditioner (nxfx_pc_*_begin/_end), for either element family ----------------
+// factorisation below the top chunk
+int factor_bottom(nxfx_ctx* ctx) {
+  if (ctx->generic) return cond_factor_local(ctx);
+  int rc = node_diag(ctx, true);
+  if (rc) return rc;
+  const int nb = ctx->tree.n_chunks - 1;
+  if (nb > 0) NXFX_LAUNCH(ctx, tree_factor_kernel, nb, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), nb, ctx->ticket.p + 1, 0,
+                          (FusedN1{make_net(ctx), nullptr, nullptr}));
+  return NXFX_OK;
+}
+
+// nodal right-hand sides and forward sweep of the bottom chunks
+int forward_bottom(nxfx_ctx* ctx, const double* r) {
+  if (ctx->generic) return cond_forward_local(ctx, r, ctx->lam_weight.p);
+  int rc = node_rhs(ctx, r, true);
+  if (rc) return rc;
+  const int nb = ctx->tree.n_chunks - 1;
+  if (nb > 0) NXFX_LAUNCH(ctx, tree_solve_kernel<kTreeUp>, nb, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), nb, ctx->ticket.p + 1, 0);
+  return NXFX_OK;
+}
+
+// the top chunk's half of a split phase: kPartial packs this rank's partial sums of the shared nodes into buf,
+// kFinish completes from the all-reduced buf (precond.cuh tree_top_kernel, condense.cuh btree_top_split_kernel)
+template <bool FACTOR, int PHASE>
+int top_split(nxfx_ctx* ctx, double* buf) {
+  const int top = ctx->tree.n_chunks - 1;
+  if (!ctx->generic) {
+    NXFX_LAUNCH(ctx, (tree_top_kernel<FACTOR, PHASE>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), top, buf);
     return NXFX_OK;
   }
-  NXFX_LAUNCH(ctx, edge_condense_kernel<false>, (int)cdiv(ctx->E, kThreads), kThreads, 0, g, ctx->cur->cell_rh.p,
-              r, ctx->edge_c.p, ctx->edge_fn.p, nullptr);
-  if (ctx->n_bif > 0) {
-    NXFX_LAUNCH(ctx, bif_rhs_kernel<false>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, r,
-                ctx->edge_g.p, ctx->edge_c.p, ctx->edge_fn.p, ctx->lam_weight.p);
-    int rc = tree_pass(ctx, false);
-    if (rc) return rc;
-  }
-  if (add)
-    NXFX_LAUNCH(ctx, edge_backsub_kernel<true>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, ctx->edge_g.p, ctx->edge_c.p, z);
-  else
-    NXFX_LAUNCH(ctx, edge_backsub_kernel<false>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, ctx->edge_g.p, ctx->edge_c.p, z);
+  if (ctx->n_bif == 0) return NXFX_OK;
+  const int32_t* idx = ctx->n_shared > 0 ? ctx->top_sh_idx.p : nullptr;
+  NXFX_LAUNCH(ctx, (btree_top_split_kernel<FACTOR, PHASE>), 1, 1024, 0, make_tree(ctx), make_cond(ctx), top, idx,
+              std::max(ctx->n_shared, 1), buf);
+  return NXFX_OK;
+}
+
+// backward sweep of the bottom chunks, back-substitution on the edges
+int backward_bottom(nxfx_ctx* ctx, const double* r, double* z, bool add) {
+  if (ctx->generic) return cond_backward_local(ctx, z, add);
+  const int nb = ctx->tree.n_chunks - 1;
+  if (nb > 0) NXFX_LAUNCH(ctx, tree_solve_kernel<kTreeDown>, nb, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), nb, ctx->ticket.p + 1, 0);
+  return edge_backsub(ctx, r, z, add);
+}
+
+// P1/DG0 with one cell per edge: setup and first application share fused bottom and top kernels
+bool fused_split(const nxfx_ctx* ctx) { return !ctx->generic && n1_kernels(ctx); }
+
+// exchanged rows of a residual, in the order of the shared list: the multiplier rows of r, then (cont: continuous
+// pressure) the nodal pressure rows of r and of b
+int pack_shared(nxfx_ctx* ctx, const double* r, const double* b, double* buf, bool cont) {
+  const int ns = ctx->n_shared;
+  if (ns == 0) return NXFX_OK;
+  NXFX_LAUNCH(ctx, pack_shared_kernel, (int)cdiv(ns, kThreads), kThreads, 0, ns, (int)ctx->loff, ctx->shared_lm.p, r, buf);
+  if (!cont) return NXFX_OK;
+  NXFX_LAUNCH(ctx, pack_nodal_kernel, (int)cdiv(ns, kThreads), kThreads, 0, ns, (int)ctx->nq, ctx->shared_lm.p, ctx->cond.bif_node.p,
+              r, buf + ns);
+  NXFX_LAUNCH(ctx, pack_nodal_kernel, (int)cdiv(ns, kThreads), kThreads, 0, ns, (int)ctx->nq, ctx->shared_lm.p, ctx->cond.bif_node.p,
+              b, buf + 2 * (size_t)ns);
   return NXFX_OK;
 }
 
@@ -1726,49 +1816,12 @@ int nxfx_exchange_sizes(nxfx_ctx* ctx, int32_t* setup, int32_t* apply, int32_t* 
   return NXFX_OK;
 }
 
-// table-driven path: the top chunk's half of a split phase (condense.cuh btree_top_split_kernel)
-static int cond_top_split(nxfx_ctx* ctx, bool factor, bool finish, double* buf) {
-  if (ctx->n_bif == 0) return NXFX_OK;
-  TreeDev t = make_tree(ctx);
-  CondDev c = make_cond(ctx);
-  const int top = ctx->tree.n_chunks - 1, nt = std::max(ctx->n_shared, 1);
-  const int32_t* idx = ctx->n_shared > 0 ? ctx->top_sh_idx.p : nullptr;
-  if (factor && !finish) NXFX_LAUNCH(ctx, (btree_top_split_kernel<true, kPartial>), 1, 1024, 0, t, c, top, idx, nt, buf);
-  else if (factor) NXFX_LAUNCH(ctx, (btree_top_split_kernel<true, kFinish>), 1, 1024, 0, t, c, top, idx, nt, buf);
-  else if (!finish) NXFX_LAUNCH(ctx, (btree_top_split_kernel<false, kPartial>), 1, 1024, 0, t, c, top, idx, nt, buf);
-  else NXFX_LAUNCH(ctx, (btree_top_split_kernel<false, kFinish>), 1, 1024, 0, t, c, top, idx, nt, buf);
-  return NXFX_OK;
-}
-
-int nxfx_top_size(nxfx_ctx* ctx, int32_t* n_top) {
-  if (!ctx || !n_top) return NXFX_ERR_INVALID;
-  NXFX_REQUIRE(ctx, ctx->tree.set && ctx->tree.n_chunks >= 1, "no tree schedule");
-  *n_top = ctx->n_shared;  // the exchanged part of the top chunk
-  return NXFX_OK;
-}
-
 int nxfx_pc_setup_begin(nxfx_ctx* ctx, double* buf) {
   if (!ctx) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
   NXFX_REQUIRE(ctx, is_assembled(ctx), "assemble the matrix before pc_setup");
-  if (ctx->generic) {
-    if ((rc = cond_factor_local(ctx)) || (rc = cond_top_split(ctx, true, false, buf))) return rc;
-    ctx->bottom_factored = true;
-    return NXFX_OK;
-  }
-  auto& s = ctx->tree;
-  TreeDev t = make_tree(ctx);
-  const int nb = s.n_chunks - 1;
-  if (ctx->N == 1) {
-    NXFX_LAUNCH(ctx, bif_diag_n1_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx), t, ctx->cur->cell_rh.p);
-  } else {
-    NXFX_LAUNCH(ctx, edge_conductance_kernel, (int)cdiv(ctx->E, kThreads), kThreads, 0, ctx->E, ctx->N, ctx->cur->cell_rh.p, ctx->edge_g.p);
-    NXFX_LAUNCH(ctx, bif_diag_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx), t, ctx->edge_g.p);
-  }
-  if (nb > 0) NXFX_LAUNCH(ctx, tree_factor_kernel, nb, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, ctx->ticket.p + 1, 0,
-                          (FusedN1{make_net(ctx), nullptr, nullptr}));
-  NXFX_LAUNCH(ctx, (tree_top_kernel<true, kPartial>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, buf);
+  if ((rc = factor_bottom(ctx)) || (rc = top_split<true, kPartial>(ctx, buf))) return rc;
   ctx->bottom_factored = true;
   return NXFX_OK;
 }
@@ -1777,16 +1830,9 @@ int nxfx_pc_setup_end(nxfx_ctx* ctx, double* buf) {
   if (!ctx) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
-  if (ctx->generic) {
-    NXFX_REQUIRE(ctx, ctx->bottom_factored, "nxfx_pc_setup_begin has not been run");
-    if ((rc = cond_top_split(ctx, true, true, buf))) return rc;
-    ctx->pc_ready = true;
-    ctx->pc_mat = ctx->cur->id;
-    return NXFX_OK;
-  }
-  NXFX_LAUNCH(ctx, (tree_top_kernel<true, kFinish>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), ctx->tree.n_chunks - 1, buf);
-  ctx->pc_ready = true;
-  ctx->pc_mat = ctx->cur->id;
+  NXFX_REQUIRE(ctx, ctx->bottom_factored, "nxfx_pc_setup_begin has not been run");
+  if ((rc = top_split<true, kFinish>(ctx, buf))) return rc;
+  mark_factored(ctx);
   return NXFX_OK;
 }
 
@@ -1797,68 +1843,34 @@ int nxfx_pc_apply_begin(nxfx_ctx* ctx, const double* r, double* buf) {
   // the forward sweep of the bottom chunks only needs THEIR factors: it may run before
   // nxfx_pc_setup_end, so that setup and first application share one all-reduce
   NXFX_REQUIRE(ctx, ctx->pc_ready || ctx->bottom_factored, "nxfx_pc_setup_begin has not been run");
-  NXFX_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(r) & 15) == 0, "vectors must be 16-byte aligned");
-  if (ctx->generic) {
-    if ((rc = cond_forward_local(ctx, r, ctx->lam_weight.p))) return rc;
-    return cond_top_split(ctx, false, false, buf);
-  }
-  Net g = make_net(ctx);
-  TreeDev t = make_tree(ctx);
-  const int nb = ctx->tree.n_chunks - 1;
-  if (ctx->N == 1) {
-    NXFX_LAUNCH(ctx, bif_rhs_n1_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, r, ctx->cur->cell_rh.p, ctx->lam_weight.p);
-  } else {
-    NXFX_LAUNCH(ctx, edge_condense_kernel<false>, (int)cdiv(ctx->E, kThreads), kThreads, 0, g, ctx->cur->cell_rh.p, r, ctx->edge_c.p, ctx->edge_fn.p);
-    NXFX_LAUNCH(ctx, bif_rhs_kernel<false>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, r, ctx->edge_g.p, ctx->edge_c.p,
-                ctx->edge_fn.p, ctx->lam_weight.p);
-  }
-  if (nb > 0) NXFX_LAUNCH(ctx, tree_solve_kernel<kTreeUp>, nb, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, ctx->ticket.p + 1, 0);
-  NXFX_LAUNCH(ctx, (tree_top_kernel<false, kPartial>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, buf);
-  return NXFX_OK;
+  if ((rc = check_aligned(ctx, r)) || (rc = forward_bottom(ctx, r))) return rc;
+  return top_split<false, kPartial>(ctx, buf);
 }
 
 int nxfx_pc_apply_end(nxfx_ctx* ctx, const double* r, double* z, double* buf, int add) {
   if (!ctx || !r || !z) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
-  if (ctx->generic) {
-    NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
-    if ((rc = cond_top_split(ctx, false, true, buf))) return rc;
-    return cond_backward_local(ctx, z, add != 0);
-  }
-  Net g = make_net(ctx);
-  TreeDev t = make_tree(ctx);
-  const int nb = ctx->tree.n_chunks - 1;
-  NXFX_LAUNCH(ctx, (tree_top_kernel<false, kFinish>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, buf);
-  if (nb > 0) NXFX_LAUNCH(ctx, tree_solve_kernel<kTreeDown>, nb, kTreeThreads, tree_smem_bytes(ctx->tree.cap), t, nb, ctx->ticket.p + 1, 0);
-  const int bgrid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kThreads);
-  if (ctx->N == 1) {
-    if (add) NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<true>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, z);
-    else NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<false>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, z);
-    return NXFX_OK;
-  }
-  if (add)
-    NXFX_LAUNCH(ctx, edge_backsub_kernel<true>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, ctx->edge_g.p, ctx->edge_c.p, z);
-  else
-    NXFX_LAUNCH(ctx, edge_backsub_kernel<false>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, ctx->edge_g.p, ctx->edge_c.p, z);
-  return NXFX_OK;
+  NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
+  if ((rc = top_split<false, kFinish>(ctx, buf))) return rc;
+  return backward_bottom(ctx, r, z, add != 0);
 }
 
-// setup + first application in one pair of calls around ONE all-reduce of 3*n_top doubles.
-// N == 1: the bottom chunks are factorised while their right-hand sides are eliminated (one kernel),
+// setup + first application in one pair of calls around ONE all-reduce of [setup | apply] sections.
+// P1/DG0, N == 1: the bottom chunks are factorised while their right-hand sides are eliminated (one kernel),
 // the top chunk handles factor and solve together in each phase; otherwise the four separate phases.
 int nxfx_pc_setup_apply_begin(nxfx_ctx* ctx, const double* r, double* buf) {
   if (!ctx || !r) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
   NXFX_REQUIRE(ctx, is_assembled(ctx), "assemble the matrix before pc_setup");
-  int32_t ns, na, nr;
-  exchange_sizes(ctx, &ns, &na, &nr);
-  if (ctx->N != 1 || ctx->generic) {
+  if (!fused_split(ctx)) {
+    int32_t ns, na, nr;
+    exchange_sizes(ctx, &ns, &na, &nr);
     if ((rc = nxfx_pc_setup_begin(ctx, buf))) return rc;
     return nxfx_pc_apply_begin(ctx, r, buf + ns);
   }
-  NXFX_REQUIRE(ctx, (reinterpret_cast<uintptr_t>(r) & 15) == 0, "vectors must be 16-byte aligned");
+  if ((rc = check_aligned(ctx, r))) return rc;
   auto& s = ctx->tree;
   TreeDev t = make_tree(ctx);
   const int nb = s.n_chunks - 1;
@@ -1874,25 +1886,18 @@ int nxfx_pc_setup_apply_end(nxfx_ctx* ctx, const double* r, double* z, double* b
   if (!ctx || !r || !z) return NXFX_ERR_INVALID;
   int rc = dist_ready(ctx, buf);
   if (rc) return rc;
-  int32_t ns, na, nr;
-  exchange_sizes(ctx, &ns, &na, &nr);
-  if (ctx->N != 1 || ctx->generic) {
+  if (!fused_split(ctx)) {
+    int32_t ns, na, nr;
+    exchange_sizes(ctx, &ns, &na, &nr);
     if ((rc = nxfx_pc_setup_end(ctx, buf))) return rc;
     return nxfx_pc_apply_end(ctx, r, z, buf + ns, 0);
   }
   NXFX_REQUIRE(ctx, ctx->bottom_factored, "nxfx_pc_setup_apply_begin has not been run");
-  auto& s = ctx->tree;
-  Net g = make_net(ctx);
-  TreeDev t = make_tree(ctx);
-  const int nb = s.n_chunks - 1;
-  FusedN1 fin{g, r, ctx->cur->cell_rh.p, ctx->lam_weight.p};
-  NXFX_LAUNCH(ctx, tree_top_fs_kernel<kFinish>, 1, kTreeThreads, tree_smem_bytes_fs(s.cap), t, nb, buf, fin);
-  ctx->pc_ready = true;
-  ctx->pc_mat = ctx->cur->id;
-  if (nb > 0) NXFX_LAUNCH(ctx, tree_solve_kernel<kTreeDown>, nb, kTreeThreads, tree_smem_bytes(s.cap), t, nb, ctx->ticket.p + 1, 0);
-  const int bgrid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kThreads);
-  NXFX_LAUNCH(ctx, edge_backsub_n1_kernel<false>, bgrid, kThreads, 0, g, t, ctx->cur->cell_rh.p, r, z);
-  return NXFX_OK;
+  FusedN1 fin{make_net(ctx), r, ctx->cur->cell_rh.p, ctx->lam_weight.p};
+  NXFX_LAUNCH(ctx, tree_top_fs_kernel<kFinish>, 1, kTreeThreads, tree_smem_bytes_fs(ctx->tree.cap), make_tree(ctx),
+              ctx->tree.n_chunks - 1, buf, fin);
+  mark_factored(ctx);
+  return backward_bottom(ctx, r, z, false);
 }
 
 // ---- peer exchange over NVLink (peer.cuh) ----------------------------------------------------------
@@ -1967,62 +1972,29 @@ int nxfx_comm_connect(nxfx_ctx* ctx, const void* handles_all) {
   return NXFX_OK;
 }
 
-int nxfx_pack_shared(nxfx_ctx* ctx, const double* v, double* buf) {
-  if (!ctx || !v || !buf) return NXFX_ERR_INVALID;
-  if (ctx->n_shared > 0)
-    NXFX_LAUNCH(ctx, pack_shared_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->loff,
-                ctx->shared_lm.p, v, buf);
-  if (ctx->n_shared > 0 && ctx->generic && ctx->cond.set && ctx->cond.cont)
-    NXFX_LAUNCH(ctx, pack_nodal_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->nq,
-                ctx->shared_lm.p, ctx->cond.bif_node.p, v, buf + ctx->n_shared);
-  return NXFX_OK;
-}
-
-int nxfx_unpack_shared(nxfx_ctx* ctx, const double* buf, double* v) {
-  if (!ctx || !v || !buf) return NXFX_ERR_INVALID;
-  if (ctx->n_shared > 0)
-    NXFX_LAUNCH(ctx, unpack_shared_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->loff,
-                ctx->shared_lm.p, buf, v);
-  if (ctx->n_shared > 0 && ctx->generic && ctx->cond.set && ctx->cond.cont)
-    NXFX_LAUNCH(ctx, unpack_nodal_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->nq,
-                ctx->shared_lm.p, ctx->cond.bif_node.p, buf + ctx->n_shared, v);
-  return NXFX_OK;
-}
-
 int nxfx_residual_partial(nxfx_ctx* ctx, const double* b, const double* x, double* r, double* buf) {
   if (!ctx || !b || !x || !r || !buf) return NXFX_ERR_INVALID;
   NXFX_REQUIRE(ctx, ctx->has_pattern && ctx->lam_nonshared.p, "nxfx_set_shared has not been called");
   NXFX_REQUIRE(ctx, is_assembled(ctx), "matrix has not been assembled");
-  int rc;
-  if (ctx->generic) {
-    // [lam rows of r | P rows of r | P rows of b | norm partials without any shared row]: a plain residual, then
-    // the packs and a weighted-norm kernel that also skips the nodal pressure rows of the shared bifurcations
-    NXFX_REQUIRE(ctx, ctx->cond.set, "nxfx_set_condensation has not been called");
-    const bool cont = ctx->cond.cont && ctx->n_shared > 0;
-    if ((rc = do_residual(ctx, b, x, r, slot(ctx, 0)))) return rc;
-    if ((rc = nxfx_pack_shared(ctx, r, buf))) return rc;
-    if (cont)
-      NXFX_LAUNCH(ctx, pack_nodal_kernel, (int)cdiv(ctx->n_shared, kThreads), kThreads, 0, ctx->n_shared, (int)ctx->nq,
-                  ctx->shared_lm.p, ctx->cond.bif_node.p, b, buf + 2 * (size_t)ctx->n_shared);
-    const int n = (int)ctx->ndofs, nr = (cont ? 3 : 1) * ctx->n_shared;
-    NXFX_LAUNCH(ctx, weighted_norm2_pair_kernel, vec_grid(ctx, n), kThreads, 0, n, (int)ctx->loff, r, ctx->lam_nonshared.p,
-                b, ctx->lam_weight.p, ctx->scal.p, ctx->ticket.p, buf + nr, (int)ctx->nq, cont ? ctx->n_nodes : 0,
-                cont ? ctx->p_nonshared.p : nullptr);
-    return NXFX_OK;
-  }
-  if (ctx->pipe_ok) {  // the weighted partial norms come out of the residual kernel itself
+  NXFX_REQUIRE(ctx, !ctx->generic || ctx->cond.set, "nxfx_set_condensation has not been called");
+  if (!ctx->generic && ctx->pipe_ok) {  // the weighted partial norms come out of the residual kernel itself
     const int ntiles = (int)cdiv(ctx->ndofs, kTileRows);
     const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
     NXFX_LAUNCH(ctx, spmv_pipe_kernel<2>, grid, kTileRows, kPipeSmem, (int)ctx->ndofs, ntiles, ctx->rowptr.p,
                 ctx->colidx.p, ctx->cur->vals.p, ctx->tile_base.p, x, r, b, ctx->scal.p, ctx->ticket.p,
                 buf + ctx->n_shared, (int)ctx->loff, ctx->lam_nonshared.p, ctx->lam_weight.p);
-    return nxfx_pack_shared(ctx, r, buf);
+    return pack_shared(ctx, r, b, buf, false);
   }
-  if ((rc = do_residual(ctx, b, x, r, slot(ctx, 0)))) return rc;
-  if ((rc = nxfx_pack_shared(ctx, r, buf))) return rc;
-  const int n = (int)ctx->ndofs;
+  // [lam rows of r | (cont) P rows of r | (cont) P rows of b | norm partials without any shared row]: a plain
+  // residual, then the packs and a weighted-norm kernel that also skips the nodal pressure rows of the shared
+  // bifurcations
+  const bool cont = ctx->generic && ctx->cond.cont && ctx->n_shared > 0;
+  int rc;
+  if ((rc = do_residual(ctx, b, x, r, slot(ctx, 0))) || (rc = pack_shared(ctx, r, b, buf, cont))) return rc;
+  const int n = (int)ctx->ndofs, nr = (cont ? 3 : 1) * ctx->n_shared;
   NXFX_LAUNCH(ctx, weighted_norm2_pair_kernel, vec_grid(ctx, n), kThreads, 0, n, (int)ctx->loff, r, ctx->lam_nonshared.p,
-              b, ctx->lam_weight.p, ctx->scal.p, ctx->ticket.p, buf + ctx->n_shared);
+              b, ctx->lam_weight.p, ctx->scal.p, ctx->ticket.p, buf + nr, (int)ctx->nq, cont ? ctx->n_nodes : 0,
+              cont ? ctx->p_nonshared.p : nullptr);
   return NXFX_OK;
 }
 
@@ -2037,14 +2009,6 @@ int nxfx_residual_finish(nxfx_ctx* ctx, const double* buf, double* r, double* nr
     return NXFX_OK;
   }
   NXFX_LAUNCH(ctx, residual_finish_kernel, 1, kThreads, 0, ctx->n_shared, (int)ctx->loff, ctx->shared_lm.p, buf, r, nrm_out);
-  return NXFX_OK;
-}
-
-int nxfx_norm2_owned(nxfx_ctx* ctx, const double* v, double* out_d) {
-  if (!ctx || !v || !out_d) return NXFX_ERR_INVALID;
-  NXFX_REQUIRE(ctx, ctx->has_network, "no network");
-  NXFX_LAUNCH(ctx, weighted_norm2_kernel, vec_grid(ctx, ctx->ndofs), kThreads, 0, (int)ctx->ndofs, (int)ctx->loff, v,
-              ctx->lam_weight.p, ctx->scal.p, ctx->ticket.p, out_d);
   return NXFX_OK;
 }
 

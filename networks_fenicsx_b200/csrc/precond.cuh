@@ -1319,18 +1319,12 @@ edge_backsub_n1_kernel(Net g, TreeDev t, const double* __restrict__ cell_rh, con
 }
 
 // ---- multi-GPU helpers --------------------------------------------------------------------------
-// shared (replicated) multiplier rows of a vector <-> contiguous buffer for the all-reduce
+// shared (replicated) multiplier rows of a vector -> contiguous buffer for the all-reduce
 __global__ void __launch_bounds__(kThreads)
 pack_shared_kernel(int n_shared, int loff, const int32_t* __restrict__ shared_lm,
                    const double* __restrict__ v, double* __restrict__ buf) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_shared) buf[i] = v[loff + shared_lm[i]];
-}
-__global__ void __launch_bounds__(kThreads)
-unpack_shared_kernel(int n_shared, int loff, const int32_t* __restrict__ shared_lm,
-                     const double* __restrict__ buf, double* __restrict__ v) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n_shared) v[loff + shared_lm[i]] = buf[i];
 }
 
 // After the all-reduce of [shared rows of r | partial ||r||^2 | ||b||^2]: write the reduced shared

@@ -367,22 +367,8 @@ multi_dot_kernel(int n, const double* __restrict__ A, size_t stride, const doubl
   finish_partials<kThreads, K>(mine, partial, gridDim.x, ticket, out, red);
 }
 
-// out[0] = sum_i w_i v_i^2 with w_i = 1 for i < loff and lam_weight[i - loff] on the multiplier rows
-// (multi-GPU: replicated multipliers are counted on one rank only)
-__global__ void __launch_bounds__(kThreads)
-weighted_norm2_kernel(int n, int loff, const double* __restrict__ v, const double* __restrict__ lam_weight,
-                      double* partial, unsigned int* ticket, double* out) {
-  __shared__ double red[kThreads / 32];
-  double acc = 0.0;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const double vi = v[i];
-    acc += (i < loff || !lam_weight ? 1.0 : lam_weight[i - loff]) * vi * vi;
-  }
-  double mine[1] = {block_sum<kThreads>(acc, red)};
-  finish_partials<kThreads, 1>(mine, partial, gridDim.x, ticket, out, red);
-}
-
-// out[0] = sum w1_i r_i^2, out[1] = sum w2_i b_i^2 in one pass (weights as above; multi-GPU residual:
+// out[0] = sum w1_i r_i^2, out[1] = sum w2_i b_i^2 in one pass (weights 1 for i < loff, w[i - loff] on the
+// multiplier rows; multi-GPU residual:
 // w1 excludes every replicated multiplier row -- their partial sums are O(1) and only cancel in the
 // all-reduce, so they must never enter a local norm -- w2 counts owned rows).  pw (nullptr: none): extra weight of the rows p0 .. p0 + np - 1 in both sums -- 0 on
 // the nodal pressure rows of the shared bifurcations (continuous pressure), partial sums like the multiplier rows

@@ -27,7 +27,7 @@ def test_binding_covers_header(built_library):
 
     assert sorted(_lib.SIGNATURES) == declared_symbols()
     lib = _lib.load()
-    assert lib.nxfx_abi_version() == 1
+    assert lib.nxfx_abi_version() == 2
 
 
 def test_create_fails_loudly_without_gpu(built_library):
