@@ -318,7 +318,24 @@ int nxfx_set_shared(nxfx_ctx* ctx, int32_t n_shared, const int32_t* shared_lm_h,
 int nxfx_comm_create(nxfx_ctx* ctx, int32_t rank, int32_t nranks, void* handle_out_h,
                      int32_t* slot_doubles);
 int nxfx_comm_connect(nxfx_ctx* ctx, const void* handles_all_h);
+/* Ranks that are contexts of ONE process (one host thread each, on one GPU or on several): after
+ * nxfx_comm_create on every context, each rank calls nxfx_comm_connect_local with ctxs_h[r] = rank r's
+ * context.  Rank r's buffer is used through its device pointer (no IPC handle).  Every context must
+ * run on its own stream created with cudaStreamNonBlocking (nxfx_set_stream).
+ *   different devices: peer access is enabled (NXFX_ERR_COMM if the devices cannot reach each other)
+ *   same device: the cooperative tree grids of all ranks on it must be resident together (sum of
+ *     their blocks <= blocks per SM x SMs), else NXFX_ERR_UNSUPPORTED before anything is launched;
+ *     the back-substitution is then not launched as a programmatic dependent of the tree kernel
+ * NXFX_ERR_INVALID if nranks, the rank order or the slot size disagree between the contexts.
+ * Every rank gets the same answer: each checks all the devices of the group.                    */
+int nxfx_comm_connect_local(nxfx_ctx* ctx, nxfx_ctx* const* ctxs_h, int32_t nranks);
 int nxfx_comm_destroy(nxfx_ctx* ctx);
+/* dst_d[i] = sum over r of src_h[r][i], i < n, added in rank order 0, 1, ... (bit-identical on every
+ * rank): the in-process replacement of the SUM all-reduce between the begin/end halves below.  A
+ * kernel on the ctx's stream; src_h = nranks device pointers readable from the ctx's device (peer
+ * access to another device is enabled on first use).  The caller orders the producers of src before
+ * this call and its consumers after it (events).                                                   */
+int nxfx_group_sum(nxfx_ctx* ctx, const double* const* src_h, int32_t nranks, double* dst_d, int64_t n);
 /* doubles of the exchanged sections of the host-driven path, for either element family:
  * setup (nxfx_pc_setup_begin), apply (nxfx_pc_apply_begin; _setup_apply_* take setup + apply, the
  * application's part at offset setup) and residual (nxfx_residual_partial).  P1/DG0: 2 nt, nt and

@@ -128,7 +128,9 @@ SIGNATURES = {
     "nxfx_set_shared": (C.c_int, [C.c_void_p, C.c_int32, c_i32p, c_f64p]),
     "nxfx_comm_create": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.POINTER(C.c_int32)]),
     "nxfx_comm_connect": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "nxfx_comm_connect_local": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32]),
     "nxfx_comm_destroy": (C.c_int, [C.c_void_p]),
+    "nxfx_group_sum": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_int32, C.c_void_p, C.c_int64]),
     "nxfx_exchange_sizes": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "nxfx_pc_setup_begin": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_pc_setup_end": (C.c_int, [C.c_void_p, C.c_void_p]),

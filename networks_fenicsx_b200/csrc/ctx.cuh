@@ -83,6 +83,8 @@ struct Condensation {
 // buffers of the other ranks.
 struct PeerComm {
   bool created = false, ready = false;
+  bool in_process = false;      // connected by nxfx_comm_connect_local: base[] are plain device pointers
+  bool shared_device = false;   // another rank of the group runs on this ctx's device
   int rank = 0, nranks = 1;
   int slot = 0;                 // doubles per (channel, parity, source)
   void* local = nullptr;        // cudaMalloc'ed, exported by cudaIpcGetMemHandle
@@ -147,6 +149,7 @@ struct nxfx_ctx {
   nxfx::DevBuf<double> lam_weight, lam_nonshared;
   nxfx::DevBuf<double> p_nonshared;  // [n_nodes] continuous pressure: 0 on the shared bifurcations (partial rows)
   nxfx::PeerComm comm;
+  uint64_t peer_on = 0;  // devices this ctx's device has peer access to (bit = ordinal; nxfx_group_sum)
   // solution mirror: pinned host copy of x that nxfx_solve fills while the residual check still runs
   double* mirror_h = nullptr;
   cudaStream_t side = nullptr;

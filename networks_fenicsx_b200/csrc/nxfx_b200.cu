@@ -671,7 +671,9 @@ int do_pc_setup_apply(nxfx_ctx* ctx, const double* r, double* z, bool add = fals
   NXFX_CUDA(ctx, le);
   ctx->launches++;
   mark_factored(ctx);
-  return edge_backsub(ctx, r, z, add, true);
+  // ranks sharing this device: a back-substitution that moved in early would hold SMs while the tree kernel
+  // waits for a peer whose cooperative grid still has to become resident (DESIGN §6)
+  return edge_backsub(ctx, r, z, add, !ctx->comm.shared_device);
 }
 
 int do_pc_apply(nxfx_ctx* ctx, int pc_type, const double* r, double* z, bool add = false) {
@@ -1911,7 +1913,7 @@ int nxfx_comm_destroy(nxfx_ctx* ctx) {
   if (!c.created) return NXFX_OK;
   cudaStreamSynchronize(ctx->stream);
   for (int r = 0; r < c.nranks; ++r)
-    if (r != c.rank && c.base[r]) cudaIpcCloseMemHandle(c.base[r]);
+    if (r != c.rank && c.base[r] && !c.in_process) cudaIpcCloseMemHandle(c.base[r]);
   if (c.local) cudaFree(c.local);
   if (c.err_h) cudaFreeHost(c.err_h);
   c.lam_scratch.release();
@@ -1969,6 +1971,108 @@ int nxfx_comm_connect(nxfx_ctx* ctx, const void* handles_all) {
     }
   }
   c.ready = true;
+  return NXFX_OK;
+}
+
+// peer access from ctx's device to `device` (idempotent; NXFX_ERR_COMM if the devices cannot reach each other)
+static int enable_peer(nxfx_ctx* ctx, int device) {
+  if (device == ctx->device || (device < 64 && (ctx->peer_on >> device) & 1u)) return NXFX_OK;
+  int can = 0;
+  NXFX_CUDA(ctx, cudaDeviceCanAccessPeer(&can, ctx->device, device));
+  if (!can) return fail(ctx, NXFX_ERR_COMM, "device %d cannot access the memory of device %d (no peer access)", ctx->device, device);
+  NXFX_CUDA(ctx, cudaSetDevice(ctx->device));
+  const cudaError_t e = cudaDeviceEnablePeerAccess(device, 0);
+  if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+  else NXFX_CUDA(ctx, e);
+  if (device < 64) ctx->peer_on |= 1ull << device;
+  return NXFX_OK;
+}
+
+int nxfx_comm_connect_local(nxfx_ctx* ctx, nxfx_ctx* const* ctxs, int32_t nranks) {
+  if (!ctx || !ctxs) return NXFX_ERR_INVALID;
+  PeerComm& c = ctx->comm;
+  NXFX_REQUIRE(ctx, c.created && !c.ready, "nxfx_comm_create has not been called (or the communicator is already connected)");
+  NXFX_REQUIRE(ctx, nranks == c.nranks && ctxs[c.rank] == ctx, "nranks or this context's rank disagree with nxfx_comm_create");
+  for (int r = 0; r < nranks; ++r) {
+    const nxfx_ctx* o = ctxs[r];
+    if (!o || !o->comm.created || o->comm.rank != r || o->comm.nranks != nranks || o->comm.slot != c.slot)
+      return fail(ctx, NXFX_ERR_INVALID, "nxfx_comm_connect_local: context %d is not rank %d of the same %d-rank group "
+                  "(nxfx_comm_create with the same nranks and slot size on every context)", r, r, nranks);
+  }
+  unsigned int flags = 0;
+  NXFX_CUDA(ctx, cudaStreamGetFlags(ctx->stream, &flags));
+  NXFX_REQUIRE(ctx, flags & cudaStreamNonBlocking,
+               "in-process ranks need a stream created with cudaStreamNonBlocking (the legacy stream serialises them)");
+  // Ranks on one device wait for each other inside the cooperative tree kernel: the grids of all of them must be
+  // resident together, or a waiting grid holds the SMs its peer needs.  Same calculation as the single-rank check
+  // (blocks per SM x SMs, tree.coop_fs_blocks), summed over the ranks of each device; every rank checks every
+  // device, so all ranks reach the same verdict.
+  bool shared = false;
+  for (int r = 0; r < nranks; ++r) {
+    int sum = 0, cap = INT32_MAX, k = 0;
+    char list[160] = "";
+    for (int q = 0; q < nranks; ++q) {
+      if (ctxs[q]->device != ctxs[r]->device) continue;
+      if (q < r) { k = -1; break; }  // device counted at its first rank
+      const TreeSchedule& s = ctxs[q]->tree;
+      const int grid = std::min(s.n_chunks - 1, s.coop_fs_blocks - 1) + 1;  // as do_pc_setup_apply launches it
+      sum += grid;
+      cap = std::min(cap, s.coop_fs_blocks);
+      const size_t len = std::strlen(list);
+      if (len + 16 < sizeof list) std::snprintf(list + len, sizeof list - len, "%s%d", k ? " + " : "", grid);
+      ++k;
+    }
+    if (k < 2) continue;
+    if (ctxs[r]->device == ctx->device) shared = true;
+    if (sum > cap)
+      return fail(ctx, NXFX_ERR_UNSUPPORTED, "the cooperative tree grids of the %d ranks on device %d are not resident together: "
+                  "%s = %d blocks > %d (blocks per SM x SMs); use the split phases (nxfx_pc_*_begin/_end) instead",
+                  k, ctxs[r]->device, list, sum, cap);
+  }
+  for (int r = 0; r < nranks; ++r) {
+    int rc = enable_peer(ctx, ctxs[r]->device);
+    if (rc) return rc;
+  }
+  // Everything the step needs from the driver happens now, not while a peer's kernel waits: the solve workspace is
+  // allocated, and every kernel the step can launch is loaded (with lazy module loading, the first launch of a
+  // kernel loads it under a lock that stalls the other ranks' threads -- measured on a B200: a peer's cooperative
+  // grid was never launched and the exchange timed out)
+  int rc = ensure_work(ctx, 3);
+  if (rc) return rc;
+  const void* step_kernels[] = {
+      reinterpret_cast<const void*>(tree_factor_solve_coop_kernel<true, false>),
+      reinterpret_cast<const void*>(tree_factor_solve_coop_kernel<true, true>),
+      reinterpret_cast<const void*>(edge_backsub_n1_kernel<false>), reinterpret_cast<const void*>(edge_backsub_n1_kernel<true>),
+      reinterpret_cast<const void*>(edge_backsub_kernel<false>), reinterpret_cast<const void*>(edge_backsub_kernel<true>),
+      reinterpret_cast<const void*>(edge_condense_kernel<true>), reinterpret_cast<const void*>(bif_rhs_kernel<true>),
+      reinterpret_cast<const void*>(spmv_pipe_kernel<3>)};
+  for (const void* k : step_kernels) {
+    cudaFuncAttributes fa;
+    NXFX_CUDA(ctx, cudaFuncGetAttributes(&fa, k));
+  }
+  for (int r = 0; r < nranks; ++r) c.base[r] = ctxs[r]->comm.local;
+  c.in_process = true;
+  c.shared_device = shared;
+  c.ready = true;
+  return NXFX_OK;
+}
+
+int nxfx_group_sum(nxfx_ctx* ctx, const double* const* src, int32_t nranks, double* dst, int64_t n) {
+  if (!ctx || !src || !dst || n < 0) return NXFX_ERR_INVALID;
+  NXFX_REQUIRE(ctx, nranks >= 1 && nranks <= kMaxPeers, "nranks out of range");
+  GroupSrc g = {};
+  for (int r = 0; r < nranks; ++r) {
+    NXFX_REQUIRE(ctx, src[r], "null source buffer");
+    g.p[r] = src[r];
+    cudaPointerAttributes a;
+    NXFX_CUDA(ctx, cudaPointerGetAttributes(&a, src[r]));
+    NXFX_REQUIRE(ctx, a.type == cudaMemoryTypeDevice, "sources must be device memory");
+    int rc = enable_peer(ctx, a.device);
+    if (rc) return rc;
+  }
+  if (n == 0) return NXFX_OK;
+  NXFX_LAUNCH(ctx, group_sum_kernel, (int)std::min<int64_t>(cdiv(n, kGroupSumThreads), (int64_t)ctx->sm_count * 4),
+              kGroupSumThreads, 0, g, (int)nranks, dst, n);
   return NXFX_OK;
 }
 

@@ -81,4 +81,25 @@ __device__ __forceinline__ double peer_ll_recv(const PeerDev& c, int ch, int src
   return __longlong_as_double((long long)((w0 & 0xFFFFFFFF00000000ull) | (w1 >> 32)));
 }
 
+// ---- in-process all-reduce (nxfx_group_sum) ----------------------------------------------------------
+// Ranks that are threads of one process reduce the split phases' buffers by reading each other's device
+// memory directly; the host orders producers and consumers with events.  Every rank adds the
+// contributions in rank order, so all ranks hold bit-identical sums.
+struct GroupSrc {
+  const double* p[kMaxPeers];
+};
+
+constexpr int kGroupSumThreads = 256;
+
+__global__ void __launch_bounds__(kGroupSumThreads)
+group_sum_kernel(GroupSrc src, int nranks, double* __restrict__ dst, int64_t n) {
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    double s = src.p[0][i];
+#pragma unroll
+    for (int r = 1; r < kMaxPeers; ++r)  // static indices: the pointers stay in the parameter bank (no stack copy)
+      if (r < nranks) s += src.p[r][i];
+    dst[i] = s;
+  }
+}
+
 }  // namespace nxfx

@@ -17,13 +17,20 @@ diagonal blocks, coupling blocks and nodal right-hand sides are exchanged), and 
 pressure the nodal pressure rows of the shared bifurcations are partial sums like their multiplier
 rows.  The section sizes come from the library (``nxfx_exchange_sizes``).
 
-Host code (NumPy) in this file; collectives through ``torch.distributed`` (NCCL on GPUs, gloo in
-the CPU tests).
+Host code (NumPy) in this file; collectives through one small seam: ``TorchDistGroup``
+(``torch.distributed``: NCCL on GPUs, gloo in the CPU tests; one process per rank) or ``ThreadGroup``
+(ranks that are threads of one process: ``PartitionedSolver``).
 """
 
 from __future__ import annotations
 
+import ctypes as C
 import dataclasses
+import functools
+import gc
+import queue
+import threading
+import weakref
 
 import numpy as np
 
@@ -133,9 +140,134 @@ def partition_tree(graph: ArrayGraph, world: int, rank: int, chunk_nodes: int = 
                          int(shared_bif.sum()), n_bif)
 
 
+class TorchDistGroup:
+    """The collectives of :class:`DistributedSolver` over ``torch.distributed`` (one process per rank)."""
+
+    def __init__(self, group=None):
+        import torch.distributed as dist
+
+        self._dist, self.group = dist, group
+        self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+
+    def all_reduce(self, t) -> None:
+        self._dist.all_reduce(t, group=self.group)
+
+    def all_reduce_scalar(self, v: float, device) -> float:
+        import torch
+
+        t = torch.tensor([float(v)], dtype=torch.float64, device=device)
+        self._dist.all_reduce(t, group=self.group)
+        return float(t.item())
+
+    def all_gather(self, out: list, t) -> None:
+        self._dist.all_gather(out, t, group=self.group)
+
+    def barrier(self) -> None:
+        self._dist.barrier(group=self.group)
+
+
+@dataclasses.dataclass
+class _ThreadShared:
+    barrier: threading.Barrier
+    slots: list  # two rounds of per-rank slots, used alternately
+
+
+class ThreadGroup:
+    """The collectives of :class:`DistributedSolver` for ranks that are threads of ONE process (one
+    ``ThreadGroup`` per rank, from :meth:`create`).
+
+    * ``barrier``: a ``threading.Barrier`` with a timeout; :meth:`abort` (called when a rank raises) breaks it,
+      so the other ranks raise ``threading.BrokenBarrierError`` instead of waiting.
+    * ``all_reduce`` of a float64 CUDA tensor: every rank records an event on its stream, the ranks swap
+      (pointer, event), each stream waits for all the events and ``nxfx_group_sum`` adds the inputs in rank
+      order into a scratch buffer (bit-identical on every rank); a second swap of events keeps every input
+      alive until all ranks have read it, then the sum is copied back.  The rank's torch current stream must
+      be its library stream (``PartitionedSolver`` sets both).  A CPU tensor is summed on the host, in rank order.
+    * scalars, ``all_gather`` and :meth:`gather_object`: plain Python.
+
+    Every call is collective: all ranks make the same calls in the same order."""
+
+    def __init__(self, shared: _ThreadShared, rank: int, world: int, timeout: float):
+        self._sh, self.rank, self.world, self.timeout = shared, rank, world, timeout
+        self._round = 0
+        self._dev = None  # Device of this rank (bind), for nxfx_group_sum
+        self._events = None
+        self._scratch = None
+
+    @classmethod
+    def create(cls, world: int, timeout: float = 300.0) -> list["ThreadGroup"]:
+        shared = _ThreadShared(threading.Barrier(world), [[None] * world, [None] * world])
+        return [cls(shared, r, world, timeout) for r in range(world)]
+
+    def bind(self, dev) -> None:
+        self._dev = dev
+
+    def barrier(self) -> None:
+        self._sh.barrier.wait(self.timeout)
+
+    def abort(self) -> None:
+        self._sh.barrier.abort()
+
+    def _swap(self, obj) -> list:
+        """Every rank's ``obj``, in rank order.  Two alternating slot rounds: a rank can only come back to
+        a round after every rank has passed the barrier of the round in between, i.e. has read this one."""
+        slots = self._sh.slots[self._round & 1]
+        self._round += 1
+        slots[self.rank] = obj
+        self.barrier()
+        return list(slots)
+
+    def gather_object(self, obj) -> list:
+        return self._swap(obj)
+
+    def all_reduce_scalar(self, v: float, device=None) -> float:
+        total = 0.0
+        for x in self._swap(float(v)):
+            total += x
+        return total
+
+    def all_gather(self, out: list, t) -> None:
+        for o, x in zip(out, self._swap(t.detach().cpu().clone())):
+            o.copy_(x)
+
+    def all_reduce(self, t) -> None:
+        import torch
+
+        if not t.is_cuda:
+            parts = self._swap(t.detach().clone())
+            total = parts[0].clone()
+            for x in parts[1:]:
+                total += x
+            t.copy_(total)
+            return
+        assert t.dtype == torch.float64 and t.is_contiguous(), "all_reduce: contiguous float64 tensors only"
+        n = t.numel()
+        stream = torch.cuda.current_stream(t.device)
+        if self._events is None:
+            self._events = (torch.cuda.Event(), torch.cuda.Event())
+        if self._scratch is None or self._scratch.numel() < n:
+            self._scratch = torch.empty(max(n, 1), dtype=torch.float64, device=t.device)
+        ready, done = self._events
+        ready.record(stream)
+        inputs = self._swap((t.data_ptr(), ready))
+        for _, ev in inputs:
+            stream.wait_event(ev)
+        ptrs = (C.c_void_p * self.world)(*[p for p, _ in inputs])
+        self._dev.call("nxfx_group_sum", ptrs, self.world, C.c_void_p(self._scratch.data_ptr()), n)
+        done.record(stream)
+        for ev in self._swap(done):
+            stream.wait_event(ev)  # nobody overwrites an input another rank still reads
+        t.copy_(self._scratch[:n])
+
+
+def _collectives(group):
+    return group if isinstance(group, ThreadGroup) else TorchDistGroup(group)
+
+
 class DistributedSolver:
     """Assemble + solve of ONE network cut over the ranks of ``torch.distributed`` (one process per
-    GPU).  Mirrors ``Solver`` for the default options (network-Schur direct solve + iterative
+    GPU), or over the threads of one process (``group`` a :class:`ThreadGroup`; see :class:`PartitionedSolver`).
+    Mirrors ``Solver`` for the default options (network-Schur direct solve + iterative
     refinement); the collectives are three kinds of small SUM all-reduces (see module docstring).
 
     Args:
@@ -149,47 +281,46 @@ class DistributedSolver:
             per GPU); ``"nccl"``: split phases around ``torch.distributed`` all-reduces;
             ``"auto"``: peer when available.
         device: CUDA ordinal of this rank.
+        group: a ``torch.distributed`` process group (None: the default one) or this rank's :class:`ThreadGroup`.
         flux_degree, pressure_degree: element degrees as in :class:`HydraulicNetworkAssembler` (the peer
             exchange is implemented for 1 / 0 only: other degrees use the all-reduces).
+        stream: ``cudaStream_t`` (as an int) the library runs this rank on; None: the legacy default stream.
     """
 
     def __init__(self, graph: ArrayGraph, N: int, p_bc_ex, f=None, R=None, device: int = 0,
                  color_strategy="smallest_last", chunk_nodes: int = CHUNK_NODES, group=None,
-                 exchange: str = "auto", flux_degree: int = 1, pressure_degree: int = 0):
-        import torch.distributed as dist
-
+                 exchange: str = "auto", flux_degree: int = 1, pressure_degree: int = 0, stream: int | None = None):
         from .assembly import HydraulicNetworkAssembler
         from .mesh import NetworkMesh, SerialComm
         from .solver import Solver
 
-        rank, world = dist.get_rank(group), dist.get_world_size(group)
-        self.part = part = partition_tree(graph, world, rank, chunk_nodes)
+        comm = _collectives(group)
+        self.part = part = partition_tree(graph, comm.world, comm.rank, chunk_nodes)
         # the sub-network is handed over explicitly (comm = serial): no second partitioning inside
         mesh = NetworkMesh(part.graph, N=N, color_strategy=color_strategy, device=device,
                            node_degree=part.node_degree, comm=SerialComm())
+        if stream is not None:
+            mesh.device.call("nxfx_set_stream", C.c_void_p(stream))
         assembler = HydraulicNetworkAssembler(mesh, flux_degree=flux_degree, pressure_degree=pressure_degree)
         assembler.compute_forms(p_bc_ex=p_bc_ex, f=self._restrict(f, N, graph), R=self._restrict(R, N, graph))
         solver = Solver(assembler, schedule=part.schedule)
-        self._attach(part, mesh, assembler, solver, group, exchange)
+        self._attach(part, mesh, assembler, solver, comm, exchange)
 
     @classmethod
     def from_solver(cls, solver, part: TreePartition, group=None, exchange: str = "auto") -> "DistributedSolver":
         """Distributed layer for an existing ``Solver`` on one rank's part of a partitioned network
         (``NetworkMesh(G, N, comm=TorchDistComm())`` under torchrun: the reference-API path)."""
         self = cls.__new__(cls)
-        self._attach(part, solver.assembler.network, solver.assembler, solver, group, exchange)
+        self._attach(part, solver.assembler.network, solver.assembler, solver, _collectives(group), exchange)
         return self
 
-    def _attach(self, part: TreePartition, mesh, assembler, solver, group, exchange: str) -> None:
-        import ctypes as C
-
+    def _attach(self, part: TreePartition, mesh, assembler, solver, comm, exchange: str) -> None:
         import torch
-        import torch.distributed as dist
 
         from . import _lib
 
-        self._C, self._torch, self._dist, self._group = C, torch, dist, group
-        self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+        self._C, self._torch, self._comm = C, torch, comm
+        self.rank, self.world = comm.rank, comm.world
         self.part = part
         self.mesh, self.assembler, self.solver = mesh, assembler, solver
         N = mesh.cells_per_edge
@@ -197,6 +328,8 @@ class DistributedSolver:
         assert np.array_equal(part.global_nodes[self.mesh.bifurcation_values], part.global_nodes[
             np.flatnonzero(part.node_degree > 1)])
         self.dev = self.mesh.device
+        if isinstance(comm, ThreadGroup):
+            comm.bind(self.dev)
         shared = np.ascontiguousarray(part.shared_lm, dtype=np.int32)
         weight = np.ascontiguousarray(part.lam_weight, dtype=np.float64)
         self.dev.call("nxfx_set_shared", shared.size, _lib.as_i32p(shared), _lib.as_f64p(weight))
@@ -220,10 +353,11 @@ class DistributedSolver:
 
     def _connect_peers(self, required: bool) -> None:
         """Peer exchange over NVLink (``peer.cuh``): every rank exports its exchange buffer as a CUDA IPC
-        handle, the handles are all-gathered with torch.distributed (the only use of the process group
-        on this path) and mapped.  All ranks agree on the outcome; any failure falls back to the
-        host-driven NCCL all-reduces unless ``required``."""
-        C, torch, dist = self._C, self._torch, self._dist
+        handle, the handles are all-gathered (the only use of the group on this path) and mapped; ranks
+        that are threads of one process (``ThreadGroup``) swap their contexts instead and use each other's
+        buffers directly.  All ranks agree on the outcome; any failure falls back to the host-driven
+        all-reduces unless ``required``."""
+        C, torch = self._C, self._torch
         handle = (C.c_ubyte * 64)()
         slot = C.c_int32(0)
         ok = 1
@@ -235,12 +369,16 @@ class DistributedSolver:
         mine = torch.tensor(list(bytes(handle)) + [slot.value & 0xFF, (slot.value >> 8) & 0xFF, (slot.value >> 16) & 0xFF, ok],
                             dtype=torch.uint8, device=cuda)
         allh = [torch.empty_like(mine) for _ in range(self.world)]
-        dist.all_gather(allh, mine, group=self._group)
+        self._comm.all_gather(allh, mine)
         table = np.stack([t.cpu().numpy() for t in allh])
         if ok and table[:, 67].all() and (table[:, 64:67] == table[0, 64:67]).all():
             blob = np.ascontiguousarray(table[:, :64]).tobytes()
             try:
-                self.dev.call("nxfx_comm_connect", C.c_char_p(blob))
+                if isinstance(self._comm, ThreadGroup):
+                    ctxs = self._comm.gather_object(self.dev.handle.value)
+                    self.dev.call("nxfx_comm_connect_local", (C.c_void_p * self.world)(*ctxs), self.world)
+                else:
+                    self.dev.call("nxfx_comm_connect", C.c_char_p(blob))
             except RuntimeError as exc:
                 ok, err = 0, str(exc)
         else:  # keep this rank's own reason when it has one (e.g. a higher-order context)
@@ -248,7 +386,7 @@ class DistributedSolver:
             ok = 0
         if self._allreduce_scalar(float(ok)) == float(self.world):
             self.exchange = "peer"
-            dist.barrier(group=self._group)  # every buffer is mapped and zeroed before the first flag is written
+            self._comm.barrier()  # every buffer is mapped and zeroed before the first flag is written
             return
         self.dev.call("nxfx_comm_destroy")
         if required:
@@ -274,9 +412,7 @@ class DistributedSolver:
         return int(self.assembler.num_dofs - n_sh + (n_sh if self.rank == 0 else 0))
 
     def _allreduce_scalar(self, v: float) -> float:
-        t = self._torch.tensor([float(v)], dtype=self._torch.float64, device=self._top.device)
-        self._dist.all_reduce(t, group=self._group)
-        return float(t.item())
+        return self._comm.all_reduce_scalar(v, self._top.device)
 
     def _ptr(self, t, offset: int = 0):
         return self._C.c_void_p(t.data_ptr() + 8 * offset)
@@ -287,7 +423,7 @@ class DistributedSolver:
     def _apply(self, r_ptr, z_ptr, add: int) -> None:
         top = self._ptr(self._top)
         self.dev.call("nxfx_pc_apply_begin", r_ptr, top)
-        self._dist.all_reduce(self._top[: self._n_apply], group=self._group)
+        self._comm.all_reduce(self._top[: self._n_apply])
         self.dev.call("nxfx_pc_apply_end", r_ptr, z_ptr, top, add)
 
     def solve(self, refine_steps: int = 1, final_residual: bool = False, refine_rtol: float = 1e-13):
@@ -305,7 +441,7 @@ class DistributedSolver:
         # chunks only needs their own factors
         top = self._ptr(self._top)  # [setup: partial pivots / blocks, link couplings | apply: partial rhs]
         dev.call("nxfx_pc_setup_apply_begin", b, top)
-        self._dist.all_reduce(self._top, group=self._group)
+        self._comm.all_reduce(self._top)
         dev.call("nxfx_pc_setup_apply_end", b, x, top)
         self.history = []
         applied = 0
@@ -359,7 +495,7 @@ class DistributedSolver:
         dev = self.dev
         sh = self._ptr(self._sh)
         dev.call("nxfx_residual_partial", b, x, self._r.c_ptr, sh)
-        self._dist.all_reduce(self._sh, group=self._group)
+        self._comm.all_reduce(self._sh)
         dev.call("nxfx_residual_finish", sh, self._r.c_ptr, self._ptr(self._nrm, 2 * k))
 
     # ---- results -------------------------------------------------------------------------------
@@ -420,3 +556,140 @@ class DistributedSolver:
         own_lm = self.part.lam_weight > 0
         return {"edges": ge, "flux": flux, "pressure": pressure, "nodes": nodes, "node_pressure": node_p,
                 "multipliers": self.part.global_bif[own_lm], "lam": x[loff:][own_lm]}
+
+
+class _Worker:
+    """One persistent thread of a :class:`PartitionedSolver`: the rank's device is current and its own
+    non-blocking torch stream is the current stream for everything the thread runs."""
+
+    def __init__(self, rank: int, device: int, on_error):
+        self.rank, self.device, self._on_error = rank, device, on_error
+        self.tasks: queue.SimpleQueue = queue.SimpleQueue()
+        self.stream = None
+        self.thread = threading.Thread(target=self._loop, name=f"nxfx-rank{rank}", daemon=True)
+        self.thread.start()
+
+    def _loop(self) -> None:
+        setup_error = None
+        try:
+            import torch
+
+            torch.cuda.set_device(self.device)
+            # torch pool streams are created with cudaStreamNonBlocking: no implicit synchronisation with the legacy
+            # stream of another thread (nxfx_comm_connect_local checks the flag)
+            self.stream = torch.cuda.Stream(self.device)
+            torch.cuda.set_stream(self.stream)
+        except BaseException as exc:  # reported by every task
+            setup_error = exc
+        while True:
+            item = self.tasks.get()
+            if item is None:
+                return
+            fn, done = item
+            if setup_error is not None:
+                self._on_error()
+                done.put((None, setup_error))
+                continue
+            try:
+                done.put((fn(), None))
+            except BaseException as exc:
+                self._on_error()  # the other ranks leave their barriers instead of waiting for this one
+                done.put((None, exc))
+
+
+def _stop_workers(workers) -> None:
+    for w in workers:
+        w.tasks.put(None)
+    for w in workers:
+        w.thread.join()
+
+
+class PartitionedSolver:
+    """ONE network cut into ``len(devices)`` parts and solved from one process, without a launcher: one
+    persistent worker thread per part, each with a :class:`DistributedSolver` on its own non-blocking stream
+    of ``cuda:devices[rank]``, the ranks' collectives through a :class:`ThreadGroup`.  An entry of ``devices``
+    may repeat (``devices=[0, 0]``: two parts on one GPU).
+
+    ``exchange``: ``"peer"`` -- the kernels exchange the partial sums through each other's device memory (the
+    single-GPU launch sequence; ranks on one device need their cooperative tree grids resident together);
+    ``"nccl"`` -- the split phases around the group's all-reduce (``nxfx_group_sum``); ``"auto"`` -- peer when
+    available.  :attr:`exchange` reports the mode the ranks agreed on.
+
+    ``assemble()`` / ``solve()`` run on every rank at once; ``solve`` returns rank 0's residual history (identical
+    on every rank).  An exception in any rank stops every thread and is re-raised here.  Use as a context
+    manager or call :meth:`close`."""
+
+    def __init__(self, graph: ArrayGraph, N: int, p_bc_ex, f=None, R=None, devices=(0, 1), flux_degree: int = 1,
+                 pressure_degree: int = 0, exchange: str = "auto", chunk_nodes: int = CHUNK_NODES,
+                 timeout: float = 300.0):
+        devices = [int(d) for d in devices]
+        if not devices:
+            raise ValueError("devices must name at least one GPU")
+        groups = ThreadGroup.create(len(devices), timeout)
+        self._workers = [_Worker(r, d, groups[0].abort) for r, d in enumerate(devices)]
+        self._finalizer = weakref.finalize(self, _stop_workers, self._workers)
+        self.devices = devices
+        self.solvers: list[DistributedSolver | None] = [None] * len(devices)
+
+        def build(rank):
+            w = self._workers[rank]
+            self.solvers[rank] = DistributedSolver(
+                graph, N, p_bc_ex, f=f, R=R, device=w.device, chunk_nodes=chunk_nodes, group=groups[rank],
+                exchange=exchange, flux_degree=flux_degree, pressure_degree=pressure_degree,
+                stream=w.stream.cuda_stream)
+
+        self._run(build)
+
+    def _run(self, fn) -> list:
+        """fn(rank) on every rank's thread at once; the results in rank order."""
+        if not self._finalizer.alive:
+            raise RuntimeError("PartitionedSolver is closed")
+        done = [queue.SimpleQueue() for _ in self._workers]
+        for w, d in zip(self._workers, done):
+            w.tasks.put((functools.partial(fn, w.rank), d))
+        results = [d.get() for d in done]
+        errors = [e for _, e in results if e is not None]
+        if errors:
+            self.close()
+            # the first failure, not the broken barriers it caused in the other ranks
+            raise next((e for e in errors if not isinstance(e, threading.BrokenBarrierError)), errors[0])
+        return [r for r, _ in results]
+
+    def map(self, fn) -> list:
+        """fn(DistributedSolver) on every rank's thread (its device and stream current); the results in rank order."""
+        return self._run(lambda rank: fn(self.solvers[rank]))
+
+    @property
+    def exchange(self) -> str:
+        return self.solvers[0].exchange
+
+    def assemble(self) -> None:
+        self.map(lambda s: s.assemble())
+
+    def solve(self, refine_steps: int = 1, final_residual: bool = False, refine_rtol: float = 1e-13) -> list[float]:
+        return self.map(lambda s: s.solve(refine_steps, final_residual, refine_rtol))[0]
+
+    def dof_values(self) -> list[dict]:
+        """Every rank's :meth:`DistributedSolver.dof_values` (global edge, node and multiplier ids)."""
+        return self.map(lambda s: s.dof_values())
+
+    def close(self) -> None:
+        """Release every rank's solver on its own thread, then stop and join the threads."""
+        if not self._finalizer.alive:
+            return
+        done = [queue.SimpleQueue() for _ in self._workers]
+        for w, d in zip(self._workers, done):
+            w.tasks.put((functools.partial(self._release, w.rank), d))
+        for d in done:
+            d.get()
+        self._finalizer()
+
+    def _release(self, rank: int) -> None:
+        self.solvers[rank] = None
+        gc.collect()
+
+    def __enter__(self) -> "PartitionedSolver":
+        return self
+
+    def __exit__(self, *exc) -> None:
+        self.close()
