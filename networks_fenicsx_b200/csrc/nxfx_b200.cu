@@ -543,7 +543,7 @@ int node_diag(nxfx_ctx* ctx, bool bif) {
     if (bif) NXFX_LAUNCH(ctx, bif_diag_n1_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx), make_tree(ctx), ctx->cur->cell_rh.p);
     return NXFX_OK;
   }
-  NXFX_LAUNCH(ctx, edge_conductance_kernel, (int)cdiv(ctx->E, kThreads), kThreads, 0, ctx->E, ctx->N, ctx->cur->cell_rh.p, ctx->edge_g.p);
+  NXFX_LAUNCH(ctx, edge_conductance_kernel, (int)cdiv(ctx->E, kThreads), kThreads, 0, make_net(ctx), ctx->cur->cell_rh.p, ctx->edge_g.p);
   if (bif) NXFX_LAUNCH(ctx, bif_diag_kernel, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, make_net(ctx), make_tree(ctx), ctx->edge_g.p);
   return NXFX_OK;
 }

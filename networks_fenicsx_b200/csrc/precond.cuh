@@ -190,14 +190,22 @@ t_inc_fill_kernel(int n_bif, const int32_t* __restrict__ bif_of_t, const int32_t
   }
 }
 
+// R h of the cells of edge e start at cell_rh + rh_base(g, e): the one-cell-per-edge assembly stores them in flux-slot
+// order (assemble.cuh), otherwise they are in cell order.  (The N == 1 kernels below index by slot themselves; the
+// general kernels also run with N == 1 when the schedule does not fit the shared-memory sweeps.)
+__device__ __forceinline__ size_t rh_base(const Net& g, int e) {
+  return g.N == 1 ? (size_t)g.edge_slot[e] : (size_t)e * g.N;
+}
+
 // g_e = 1 / sum_j R_j h_j
 __global__ void __launch_bounds__(kThreads)
-edge_conductance_kernel(int E, int N, const double* __restrict__ cell_rh, double* __restrict__ g) {
+edge_conductance_kernel(Net g, const double* __restrict__ cell_rh, double* __restrict__ edge_g) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= E) return;
+  if (e >= g.E) return;
+  const double* rh = cell_rh + rh_base(g, e);
   double W = 0.0;
-  for (int j = 0; j < N; ++j) W += cell_rh[(size_t)e * N + j];
-  g[e] = 1.0 / W;
+  for (int j = 0; j < g.N; ++j) W += rh[j];
+  edge_g[e] = 1.0 / W;
 }
 
 __global__ void __launch_bounds__(kThreads)
@@ -1154,7 +1162,7 @@ edge_condense_kernel(Net g, const double* __restrict__ cell_rh, const double* __
   const int N = g.N;
   const double* rq = r + (size_t)g.edge_slot[e] * (N + 1);
   const double* rp = r + g.poff + (size_t)e * N;
-  const double* rh = cell_rh + (size_t)e * N;
+  const double* rh = cell_rh + rh_base(g, e);
   double s = 0.0, F = 0.0, wF = 0.0, hl = 0.0, W = 0.0;
   for (int a = 0; a <= N; ++a) {
     s += rq[a];
@@ -1222,7 +1230,7 @@ edge_backsub_kernel(Net g, TreeDev t, const double* __restrict__ cell_rh,
   const double lv = uv.w >= 0 ? t.lam_nat[uv.w] : 0.0;
   const double* rq = r + (size_t)slot * (N + 1);
   const double* rp = r + g.poff + (size_t)e * N;
-  const double* rh = cell_rh + (size_t)e * N;
+  const double* rh = cell_rh + rh_base(g, e);
   double* zq = z + (size_t)slot * (N + 1);
   double* zp = z + g.poff + (size_t)e * N;
   const double q0 = edge_g[e] * (edge_c[e] + lu - lv);

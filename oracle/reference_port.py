@@ -379,6 +379,86 @@ class OracleNetwork:
         """Direct solve (SuperLU as the MUMPS stand-in) -- solver.py:58-65,127."""
         return spla.splu(A.tocsc()).solve(b)
 
+    @staticmethod
+    def solve_exact(A, r, rounds=4):
+        """``A^{-1} r`` to well below float64 rounding, as ``np.longdouble`` (test reference for operators that are
+        meant to be exact solves).  SuperLU in float64, then ``rounds`` steps of iterative refinement whose residual
+        ``r - A x`` is formed in extended precision (x86 long double: 64-bit mantissa, eps 1.1e-19).  Each step gains
+        about -log10(eps_64 cond(A)) digits until the extended residual's own rounding is reached.  ``r`` may be
+        ``[n]`` or ``[n, k]``."""
+        lu = spla.splu(sp.csc_matrix(A, dtype=np.float64))
+        Ald = sp.csr_matrix(A).astype(np.longdouble)
+        rld = np.asarray(r).astype(np.longdouble)
+        x = lu.solve(np.asarray(r, dtype=np.float64)).astype(np.longdouble)
+        for _ in range(rounds):
+            res = rld - Ald @ x
+            x += lu.solve(res.astype(np.float64))
+        return x
+
+    @staticmethod
+    def gmres_reference(A, b, minv_diag, m, k_max):
+        """Right-preconditioned GMRES(m) from x0 = 0 in ``np.longdouble``: Arnoldi with modified Gram-Schmidt and
+        one re-orthogonalisation, Givens rotations.  ``minv_diag``: the preconditioner as a diagonal (None: the
+        identity).  Returns ``(rho, beta, x)``: ``rho[k]`` the minimal residual norm after k iterations (k = 0 ..
+        k_max; within a cycle the least-squares residual, at a restart the true residual of the updated iterate),
+        ``beta[c]`` the true residual norm at the start of cycle c (one more entry after the last cycle), and the
+        final iterate."""
+        ld = np.longdouble
+        n = b.size
+        Ald = sp.csr_matrix(A).astype(ld)
+        bl = np.asarray(b).astype(ld)
+        dinv = np.ones(n, dtype=ld) if minv_diag is None else np.asarray(minv_diag).astype(ld)
+        x = np.zeros(n, dtype=ld)
+        rho, beta = [], []
+        its = 0
+        while True:
+            r = bl - Ald @ x
+            bt = np.sqrt(np.sum(r * r))
+            beta.append(bt)
+            if its == 0:
+                rho.append(bt)
+            else:
+                rho[-1] = bt  # the true residual of the restarted iterate replaces the estimate
+            if its >= k_max or bt == 0:
+                break
+            V = np.zeros((m + 1, n), dtype=ld)
+            H = np.zeros((m + 1, m), dtype=ld)
+            cs, sn = np.zeros(m, dtype=ld), np.zeros(m, dtype=ld)
+            g = np.zeros(m + 1, dtype=ld)
+            g[0] = bt
+            V[0] = r / bt
+            k = 0
+            while k < m and its < k_max:
+                w = Ald @ (dinv * V[k])
+                for _ in range(2):  # MGS, then once more
+                    for i in range(k + 1):
+                        h = np.sum(V[i] * w)
+                        H[i, k] += h
+                        w -= h * V[i]
+                H[k + 1, k] = np.sqrt(np.sum(w * w))
+                breakdown = not H[k + 1, k] > 0  # the Krylov space is invariant: the iterate below is exact
+                if not breakdown:
+                    V[k + 1] = w / H[k + 1, k]
+                for i in range(k):
+                    t = cs[i] * H[i, k] + sn[i] * H[i + 1, k]
+                    H[i + 1, k] = -sn[i] * H[i, k] + cs[i] * H[i + 1, k]
+                    H[i, k] = t
+                den = np.hypot(H[k, k], H[k + 1, k])
+                cs[k], sn[k] = (H[k, k] / den, H[k + 1, k] / den) if den > 0 else (ld(1), ld(0))
+                H[k, k] = den
+                g[k + 1] = -sn[k] * g[k]
+                g[k] = cs[k] * g[k]
+                rho.append(abs(g[k + 1]))
+                k += 1
+                its += 1
+                if breakdown:
+                    break
+            y = np.zeros(k, dtype=ld)
+            for i in range(k - 1, -1, -1):
+                y[i] = (g[i] - H[i, i + 1:k] @ y[i + 1:]) / H[i, i]
+            x += dinv * (V[:k].T @ y)
+        return np.asarray(rho, dtype=ld), np.asarray(beta, dtype=ld), x
+
     def split(self, x):
         """Split the blocked vector as fem.petsc.assign does -- solver.py:120-134."""
         bounds = np.concatenate([[0], np.cumsum(self.block_sizes)])

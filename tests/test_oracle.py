@@ -244,3 +244,103 @@ def test_vectorised_assembly_equals_the_cellwise_quadrature_assembly(fd, pd):
         Ad, bd = ffcx_literal.assemble_cellwise(net, pbc, R=R, f=f)
         np.testing.assert_allclose(A.toarray(), Ad, rtol=1e-12, atol=1e-13)
         np.testing.assert_allclose(b, bd, rtol=1e-12, atol=1e-13)
+
+
+# ---- the high-precision references the GPU operator tests compare against ---------------------------------------
+def _fraction_solve(A, b):
+    """Exact solution of A x = b by Gaussian elimination over the rationals (A, b: float64 entries, taken exactly)."""
+    from fractions import Fraction
+
+    n = A.shape[0]
+    M = [[Fraction(float(v)) for v in row] + [Fraction(float(bi))] for row, bi in zip(A.toarray(), b)]
+    for c in range(n):
+        p = next(i for i in range(c, n) if M[i][c] != 0)
+        M[c], M[p] = M[p], M[c]
+        piv = M[c]
+        for i in range(c + 1, n):
+            if M[i][c] != 0:
+                f = M[i][c] / piv[c]
+                M[i] = [a - f * bb for a, bb in zip(M[i], piv)] if f else M[i]
+    x = [Fraction(0)] * n
+    for i in range(n - 1, -1, -1):
+        x[i] = (M[i][n] - sum(M[i][j] * x[j] for j in range(i + 1, n))) / M[i][i]
+    return x
+
+
+def _block_errors(net, x, x_exact):
+    """Per block (flux, pressure, multipliers): ||x - x_exact|| / ||x_exact||, with x_exact rational and the
+    difference formed exactly."""
+    from fractions import Fraction
+
+    out = []
+    for lo, hi in ((0, net.poff), (net.poff, net.loff), (net.loff, net.n_dofs)):
+        d = [Fraction(*np.longdouble(x[i]).as_integer_ratio()) - x_exact[i] for i in range(lo, hi)]
+        num = float(sum(v * v for v in d))
+        den = float(sum(x_exact[i] * x_exact[i] for i in range(lo, hi)))
+        out.append(np.sqrt(num / den))
+    return np.asarray(out)
+
+
+@pytest.mark.parametrize("graph", ["Y", "double_Y"])
+@pytest.mark.parametrize("N", [1, 3])
+def test_solve_exact_against_rational_elimination(graph, N):
+    """solve_exact (float64 SuperLU + refinement with an extended-precision residual) agrees with exact rational
+    Gaussian elimination to far below float64 rounding, block by block, on the Y and double-Y systems with a source:
+    it is a reference the float64 solvers can be measured against."""
+    G = golden_graph("tree_n2_H1_W3_d3") if graph == "Y" else helpers.double_junction_graph()
+    net, _ = oracle_net(G, N, "smallest_last")
+    rng = np.random.default_rng(7 * N + len(graph))
+    nc = net.cells.shape[0]
+    A, b = net.assemble(net.eval_pbc(lambda x: x[1] - 0.4 * x[0]), R=rng.uniform(0.5, 2.0, nc), f=rng.normal(size=nc))
+    assert np.count_nonzero(b[net.poff:net.loff]) == nc  # f != 0: every pressure row is populated
+    x_exact = _fraction_solve(A, b)
+    err = _block_errors(net, rp.OracleNetwork.solve_exact(A, b), x_exact)
+    err64 = _block_errors(net, net.solve(A, b), x_exact)
+    assert err.max() <= 1e-17, err
+    assert err64.max() <= 1e-13, err64
+
+
+def _krylov_min_residual(A, b, dinv, k):
+    """min over y in K_k(A D, b) of ||b - A D y||, by a dense float64 least-squares solve on an explicit (column-
+    normalised) Krylov basis: an independent statement of what GMRES minimises."""
+    cols = [b / np.linalg.norm(b)]
+    for _ in range(k - 1):
+        v = A @ (dinv * cols[-1])
+        cols.append(v / np.linalg.norm(v))
+    AK = np.column_stack([A @ (dinv * c) for c in cols])
+    y = np.linalg.lstsq(AK, b, rcond=None)[0]
+    return np.linalg.norm(b - AK @ y)
+
+
+@pytest.mark.parametrize("pc", ["none", "jacobi"])
+def test_gmres_reference(pc):
+    """gmres_reference: the minimal residuals never increase (also across restarts), reach zero at k = n on a small
+    system, agree with a least-squares minimisation over an explicit Krylov basis for small k, and the returned
+    iterate has the residual it reports."""
+    G = golden_graph("tree_n2_H1_W3_d3")
+    net, _ = oracle_net(G, 2)
+    rng = np.random.default_rng(3)
+    nc = net.cells.shape[0]
+    A, b = net.assemble(net.eval_pbc(lambda x: x[1]), R=rng.uniform(0.5, 2.0, nc), f=rng.normal(size=nc))
+    n = net.n_dofs
+    dinv = np.ones(n)
+    if pc == "jacobi":
+        dinv[:net.poff] = 1.0 / A.diagonal()[:net.poff]
+    minv = None if pc == "none" else dinv
+    nb = np.linalg.norm(b)
+    rho, beta, x = rp.OracleNetwork.gmres_reference(A, b, minv, n, n)
+    assert rho.size == n + 1 and beta.size == 2
+    assert np.all(np.diff(rho.astype(np.float64)) <= 1e-15 * nb)
+    assert rho[-1] <= 1e-14 * nb and beta[-1] <= 1e-14 * nb
+    for k in range(1, 6):
+        np.testing.assert_allclose(float(rho[k]), _krylov_min_residual(A, b, dinv, k), rtol=1e-8)
+    # restarted: the iterate of each cycle is the start of the next, the residuals keep decreasing
+    m, k_max = 3, 12
+    rho_r, beta_r, x_r = rp.OracleNetwork.gmres_reference(A, b, minv, m, k_max)
+    assert rho_r.size == k_max + 1 and beta_r.size == k_max // m + 1
+    assert np.all(np.diff(rho_r.astype(np.float64)) <= 1e-15 * nb)
+    np.testing.assert_allclose(rho_r[:m + 1].astype(np.float64), rho[:m + 1].astype(np.float64), rtol=1e-12)
+    np.testing.assert_allclose(beta_r.astype(np.float64), rho_r[::m].astype(np.float64), rtol=1e-12)
+    res = b.astype(np.longdouble) - A.astype(np.longdouble) @ x_r
+    np.testing.assert_allclose(float(np.sqrt(np.sum(res * res))), float(rho_r[-1]), rtol=1e-12)
+    assert float(rho_r[-1]) > float(rho[k_max])  # restarting costs: GMRES(3) is slower than full GMRES
