@@ -246,17 +246,20 @@ int build_vertices(nxfx_ctx* ctx) {
 }
 
 // ---- solver building blocks ------------------------------------------------------------------
-constexpr size_t kPipeSmem = kStages * sizeof(SpmvStage) + kStages * sizeof(uint64_t);
-#ifndef NXFX_SPMV_BLOCKS
-#define NXFX_SPMV_BLOCKS 5
-#endif
-constexpr int kPipeBlocksPerSM = NXFX_SPMV_BLOCKS;
+// launch shape of spmv_pipe_kernel: persistent blocks (their partials stay within kMaxPartials)
+struct PipeShape {
+  int ntiles, grid;
+};
+PipeShape pipe_shape(const nxfx_ctx* ctx) {
+  const int ntiles = (int)cdiv(ctx->ndofs, kTileRows);
+  return {ntiles, std::min({ntiles, ctx->sm_count * kPipeBlocksPerSM, kMaxPartials})};
+}
 
 int do_spmv(nxfx_ctx* ctx, const double* x, double* y) {
   const int ntiles = (int)cdiv(ctx->ndofs, kTileRows);
   if (ctx->pipe_ok) {
-    const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
-    NXFX_LAUNCH(ctx, spmv_pipe_kernel<0>, grid, kTileRows, kPipeSmem, (int)ctx->ndofs, ntiles,
+    const PipeShape ps = pipe_shape(ctx);
+    NXFX_LAUNCH(ctx, spmv_pipe_kernel<0>, ps.grid, kPipeThreads, kPipeSmem, (int)ctx->ndofs, ps.ntiles,
                 ctx->rowptr.p, ctx->colidx.p, ctx->cur->vals.p, ctx->tile_base.p, x, y, nullptr, nullptr,
                 nullptr, nullptr);
     return NXFX_OK;
@@ -274,10 +277,10 @@ int do_residual(nxfx_ctx* ctx, const double* b, const double* x, double* r, doub
     // partitioned network: the kernel itself exchanges the shared rows and the norm partials with the
     // other ranks over NVLink; norm2_d receives the GLOBAL [||r||^2, ||b||^2], identical on all ranks
     NXFX_REQUIRE(ctx, ctx->pipe_ok && ctx->lam_nonshared.p, "the fused partitioned residual needs the pipelined SpMV and nxfx_set_shared");
-    const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
+    const PipeShape ps = pipe_shape(ctx);
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(kTileRows);
+    cfg.gridDim = dim3(ps.grid);
+    cfg.blockDim = dim3(kPipeThreads);
     cfg.dynamicSmemBytes = kPipeSmem;
     cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
@@ -285,7 +288,7 @@ int do_residual(nxfx_ctx* ctx, const double* b, const double* x, double* r, doub
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = pdl ? 1 : 0;
-    NXFX_CUDA(ctx, cudaLaunchKernelEx(&cfg, spmv_pipe_kernel<3>, (int)ctx->ndofs, ntiles, (const int32_t*)ctx->rowptr.p,
+    NXFX_CUDA(ctx, cudaLaunchKernelEx(&cfg, spmv_pipe_kernel<3>, (int)ctx->ndofs, ps.ntiles, (const int32_t*)ctx->rowptr.p,
                                       (const int32_t*)ctx->colidx.p, (const double*)ctx->cur->vals.p,
                                       (const int32_t*)ctx->tile_base.p, x, r, b, ctx->scal.p, ctx->ticket.p, norm2_d,
                                       (int)ctx->loff, (const double*)ctx->lam_nonshared.p, (const double*)ctx->lam_weight.p,
@@ -295,19 +298,19 @@ int do_residual(nxfx_ctx* ctx, const double* b, const double* x, double* r, doub
     return NXFX_OK;
   }
   if (ctx->pipe_ok && !pdl) {
-    const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
-    NXFX_LAUNCH(ctx, spmv_pipe_kernel<1>, grid, kTileRows, kPipeSmem, (int)ctx->ndofs, ntiles,
+    const PipeShape ps = pipe_shape(ctx);
+    NXFX_LAUNCH(ctx, spmv_pipe_kernel<1>, ps.grid, kPipeThreads, kPipeSmem, (int)ctx->ndofs, ps.ntiles,
                 ctx->rowptr.p, ctx->colidx.p, ctx->cur->vals.p, ctx->tile_base.p, x, r, b, ctx->scal.p,
                 ctx->ticket.p, norm2_d);
     return NXFX_OK;
   }
   if (ctx->pipe_ok) {
-    const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
-    // programmatic dependent launch: the blocks set up their pipeline and prefetch matrix tiles
+    const PipeShape ps = pipe_shape(ctx);
+    // programmatic dependent launch: the blocks set up their ring and prefetch matrix tiles
     // while the preceding kernel (normally the back-substitution producing x) drains
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(kTileRows);
+    cfg.gridDim = dim3(ps.grid);
+    cfg.blockDim = dim3(kPipeThreads);
     cfg.dynamicSmemBytes = kPipeSmem;
     cfg.stream = ctx->stream;
     cudaLaunchAttribute attr[1];
@@ -315,7 +318,7 @@ int do_residual(nxfx_ctx* ctx, const double* b, const double* x, double* r, doub
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    NXFX_CUDA(ctx, cudaLaunchKernelEx(&cfg, spmv_pipe_kernel<1>, (int)ctx->ndofs, ntiles, (const int32_t*)ctx->rowptr.p,
+    NXFX_CUDA(ctx, cudaLaunchKernelEx(&cfg, spmv_pipe_kernel<1>, (int)ctx->ndofs, ps.ntiles, (const int32_t*)ctx->rowptr.p,
                                       (const int32_t*)ctx->colidx.p, (const double*)ctx->cur->vals.p,
                                       (const int32_t*)ctx->tile_base.p, x, r, b, ctx->scal.p, ctx->ticket.p, norm2_d, 0,
                                       (const double*)nullptr, (const double*)nullptr, PeerDev{}, (const int32_t*)nullptr, 0,
@@ -1000,11 +1003,15 @@ int setup_spmv_tiles(nxfx_ctx* ctx) {
   NXFX_CUDA(ctx, cudaMemcpyAsync(&max_tile_h, max_tile, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
   NXFX_CUDA(ctx, cudaMemsetAsync(ctx->ticket.p, 0, sizeof(unsigned int), ctx->stream));
   NXFX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  ctx->pipe_ok = max_tile_h + 8 <= kPipeCap;
+  // every tile, widened to 16-byte boundaries (up to 3 entries on each side), fits the ring at once
+  ctx->pipe_ok = pipe_tile_bytes(kTileRows, max_tile_h + 6) <= kRingBytes;
   if (ctx->pipe_ok) {
-    NXFX_CUDA(ctx, cudaFuncSetAttribute(spmv_pipe_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmem));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute(spmv_pipe_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmem));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute(spmv_pipe_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmem));
+    const void* modes[] = {reinterpret_cast<const void*>(spmv_pipe_kernel<0>), reinterpret_cast<const void*>(spmv_pipe_kernel<1>),
+                           reinterpret_cast<const void*>(spmv_pipe_kernel<2>), reinterpret_cast<const void*>(spmv_pipe_kernel<3>)};
+    for (const void* k : modes) {
+      NXFX_CUDA(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPipeSmem));
+      NXFX_CUDA(ctx, cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
+    }
   }
   return NXFX_OK;
 }
@@ -2082,9 +2089,8 @@ int nxfx_residual_partial(nxfx_ctx* ctx, const double* b, const double* x, doubl
   NXFX_REQUIRE(ctx, is_assembled(ctx), "matrix has not been assembled");
   NXFX_REQUIRE(ctx, !ctx->generic || ctx->cond.set, "nxfx_set_condensation has not been called");
   if (!ctx->generic && ctx->pipe_ok) {  // the weighted partial norms come out of the residual kernel itself
-    const int ntiles = (int)cdiv(ctx->ndofs, kTileRows);
-    const int grid = std::min(ntiles, ctx->sm_count * kPipeBlocksPerSM);
-    NXFX_LAUNCH(ctx, spmv_pipe_kernel<2>, grid, kTileRows, kPipeSmem, (int)ctx->ndofs, ntiles, ctx->rowptr.p,
+    const PipeShape ps = pipe_shape(ctx);
+    NXFX_LAUNCH(ctx, spmv_pipe_kernel<2>, ps.grid, kPipeThreads, kPipeSmem, (int)ctx->ndofs, ps.ntiles, ctx->rowptr.p,
                 ctx->colidx.p, ctx->cur->vals.p, ctx->tile_base.p, x, r, b, ctx->scal.p, ctx->ticket.p,
                 buf + ctx->n_shared, (int)ctx->loff, ctx->lam_nonshared.p, ctx->lam_weight.p);
     return pack_shared(ctx, r, b, buf, false);

@@ -1,12 +1,13 @@
 // CSR SpMV and fused vector kernels for the Krylov solve (solver.py:127 replaces KSPSolve).
 //
 // A block owns tiles of kTileRows consecutive rows: the tile's (value, column) pairs are streamed
-// from HBM, x is gathered from L2 (x is 8*n_dofs bytes, far below the 126 MB L2), the products are
-// parked in shared memory and every row is reduced sequentially in ascending column order.  The
+// from HBM, x is gathered from L2 (x is 8*n_dofs bytes, far below the 126 MB L2) and every row is
+// reduced sequentially in ascending column order.  The
 // row sum is therefore deterministic and bit-identical to a sequential CSR product (mul then add,
 // no FMA).  MODE 1 fuses r = b - A x with the block partials of ||r||^2 and ||b||^2.
-//   spmv_pipe_kernel  persistent blocks, TMA bulk copies (cp.async.bulk) + mbarrier pipeline,
-//                     L2 evict-first hint on the matrix stream -- the production kernel;
+//   spmv_pipe_kernel  persistent blocks, a producer thread streaming tiles into a shared-memory ring
+//                     with TMA bulk copies (cp.async.bulk) + mbarriers, L2 evict-first hint on the
+//                     matrix stream, rows summed from registers -- the production kernel;
 //   spmv_kernel       plain loads, any tile size -- fallback for very long rows.
 #pragma once
 
@@ -137,23 +138,29 @@ spmv_kernel(int n, int ntiles, const int32_t* __restrict__ rowptr,
   }
 }
 
-// ---- pipelined SpMV (TMA bulk copies + mbarrier) -----------------------------------------------
-// Persistent blocks walk over row tiles; thread 0 keeps kStages-1 tiles in flight with
-// cp.async.bulk (the TMA engine, SASS UBLKCP): the tile's values, column indices and row pointers
-// land in a shared-memory stage and signal an mbarrier with their byte count.  The other threads
-// only gather x, multiply in place and reduce rows, so HBM streaming never waits for the gather /
-// reduce phases of the same block.
-constexpr int kPipeCap = 1792;  // entries per stage = 7 * kTileRows
-#ifndef NXFX_SPMV_STAGES
-#define NXFX_SPMV_STAGES 2
-#endif
-constexpr int kStages = NXFX_SPMV_STAGES;
+// ---- pipelined SpMV (TMA bulk copies + mbarrier ring) -------------------------------------------
+// Persistent blocks walk over row tiles.  One producer thread keeps a byte ring in dynamic shared memory
+// filled with cp.async.bulk (the TMA engine, SASS UBLKCP): a tile's row pointers, column indices and
+// values land back to back, packed at their actual size, and signal the tile's full mbarrier with their
+// byte count.  The 256 consumer threads (one row each) copy their row's (column, value) pairs into
+// registers and release the tile on its empty mbarrier before they gather x and sum: a tile occupies
+// the ring only while it loads and while its entries are read out, so several tiles per block are in
+// flight from HBM while the rows of earlier ones are summed.  Rows longer than kRowRegs entries are summed
+// straight from the ring before the release (correct, slower; the headline rows hold 2-6 entries).
+constexpr int kPipeThreads = kTileRows + 32;  // 8 consumer warps + 1 producer warp
+constexpr int kPipeBlocksPerSM = 3;  // 72 registers per thread without spills (4 blocks: 56, spilling)
+constexpr int kRowRegs = 8;       // entries of a row copied into registers
+constexpr int kRingDescs = 8;     // tiles a block can have in the ring at once
+// kPipeBlocksPerSM x (ring + header + static shared memory + 1 KB reserved per block) within the 228 KB of an SM
+constexpr uint32_t kRingBytes = (228 * 1024 / kPipeBlocksPerSM - 2048) & ~15;
+constexpr size_t kPipeHeader = kRingDescs * (3 * sizeof(uint64_t) + sizeof(uint32_t));  // full, empty, end, offset
+constexpr size_t kPipeSmem = kRingBytes + kPipeHeader;
 
-struct alignas(128) SpmvStage {
-  double vals[kPipeCap];
-  int cols[kPipeCap];
-  int rows[kTileRows + 8];
-};
+// ring bytes of a tile of nr rows whose entries, widened to 16-byte boundaries, number cnt4:
+// [row pointers, padded to 16 B][cnt4 columns][cnt4 values]
+__host__ __device__ constexpr uint32_t pipe_tile_bytes(int nr, int cnt4) {
+  return (uint32_t)((((nr + 1) * 4 + 15) & ~15) + cnt4 * 12);
+}
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return (uint32_t)__cvta_generic_to_shared(p);
@@ -192,6 +199,10 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+
 // tile_base[t] = rowptr[t * kTileRows], tile_base[ntiles] = nnz
 __global__ void __launch_bounds__(kThreads)
 tile_base_kernel(int n, int ntiles, const int32_t* __restrict__ rowptr, int32_t* __restrict__ tile_base,
@@ -204,8 +215,60 @@ tile_base_kernel(int n, int ntiles, const int32_t* __restrict__ rowptr, int32_t*
   if (t < ntiles) atomicMax(max_tile_nnz, rowptr[min(r + kTileRows, n)] - b);
 }
 
+// Producer of spmv_pipe_kernel: issues the block's tiles in order into the ring.  A tile never wraps
+// around the ring's end (the rest of the ring is skipped); space and descriptors are reclaimed in issue
+// order from the empty barriers.  Only the matrix is touched until the ring is full, then the producer
+// waits for the preceding kernel like every other thread (programmatic dependent launch).
+__device__ __forceinline__ void spmv_produce(int n, int ntiles, const int32_t* __restrict__ rowptr,
+                                             const int32_t* __restrict__ colidx, const double* __restrict__ vals,
+                                             const int32_t* __restrict__ tile_base, unsigned char* ring,
+                                             uint64_t* full, uint64_t* empty, uint64_t* end, uint32_t* slot_off) {
+  const uint64_t policy = l2_evict_first_policy();
+  uint64_t head = 0, released = 0;  // ring bytes issued so far / free again below released + kRingBytes
+  bool waited = false;
+  int oldest = 0, k = 0;  // oldest tile not yet reclaimed, tile being issued (block-local counts)
+  for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++k) {
+    const int r0 = tile * kTileRows;
+    const int nr = min(kTileRows, n - r0);
+    const int sb = tile_base[tile], se = tile_base[tile + 1];
+    const int s4 = sb & ~3;
+    const int cnt4 = ((se + 3) & ~3) - s4;
+    const uint32_t rbytes = pipe_tile_bytes(nr, 0), bytes = pipe_tile_bytes(nr, cnt4);
+    uint64_t start = head;
+    const uint32_t pos = (uint32_t)(head % kRingBytes);
+    if (pos + bytes > kRingBytes) start += kRingBytes - pos;
+    while (true) {
+      if (oldest == k) {  // nothing in flight: the whole ring is free
+        released = start;
+        break;
+      }
+      if (start + bytes <= released + kRingBytes && k - oldest < kRingDescs) break;
+      if (!waited) {
+        asm volatile("griddepcontrol.wait;" ::: "memory");
+        waited = true;
+      }
+      const int d = oldest % kRingDescs;
+      mbar_wait(empty + d, (uint32_t)((oldest / kRingDescs) & 1));
+      released = end[d];
+      ++oldest;
+    }
+    head = start + bytes;
+    const int d = k % kRingDescs;
+    const uint32_t o = (uint32_t)(start % kRingBytes);
+    end[d] = head;
+    slot_off[d] = o;
+    mbar_expect_tx(full + d, bytes);
+    if (cnt4 > 0) {
+      bulk_g2s_stream(ring + o + rbytes, colidx + s4, (uint32_t)cnt4 * 4u, full + d, policy);
+      bulk_g2s_stream(ring + o + rbytes + (uint32_t)cnt4 * 4u, vals + s4, (uint32_t)cnt4 * 8u, full + d, policy);
+    }
+    bulk_g2s_stream(ring + o, rowptr + r0, rbytes, full + d, policy);
+  }
+  if (!waited) asm volatile("griddepcontrol.wait;" ::: "memory");
+}
+
 template <int MODE>
-__global__ void __launch_bounds__(kTileRows)
+__global__ void __launch_bounds__(kPipeThreads, kPipeBlocksPerSM)
 spmv_pipe_kernel(int n, int ntiles, const int32_t* __restrict__ rowptr,
                  const int32_t* __restrict__ colidx, const double* __restrict__ vals,
                  const int32_t* __restrict__ tile_base, const double* __restrict__ x,
@@ -215,85 +278,72 @@ spmv_pipe_kernel(int n, int ntiles, const int32_t* __restrict__ rowptr,
                  PeerDev pc = PeerDev{}, const int32_t* __restrict__ shared_lm = nullptr, int n_shared = 0,
                  double* lam_scratch = nullptr) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  SpmvStage* st = reinterpret_cast<SpmvStage*>(smem_raw);
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + kStages * sizeof(SpmvStage));
-  __shared__ double red[kTileRows / 32];
+  unsigned char* ring = smem_raw;
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + kRingBytes);
+  uint64_t* empty = full + kRingDescs;
+  uint64_t* end = empty + kRingDescs;
+  uint32_t* slot_off = reinterpret_cast<uint32_t*>(end + kRingDescs);
+  __shared__ double red[kPipeThreads / 32];
   const int tid = threadIdx.x;
   if (tid == 0) {
-    for (int s = 0; s < kStages; ++s) mbar_init(full + s, 1);
+    for (int d = 0; d < kRingDescs; ++d) {
+      mbar_init(full + d, 1);
+      mbar_init(empty + d, kTileRows);
+    }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   }
   __syncthreads();
-  const uint64_t stream_policy = l2_evict_first_policy();
-  auto issue = [&](int tile, int s) {
-    const int r0 = tile * kTileRows;
-    const int nr = min(kTileRows, n - r0);
-    const int sb = tile_base[tile], se = tile_base[tile + 1];
-    const int s4 = sb & ~3;
-    const int cnt4 = ((se + 3) & ~3) - s4;
-    const uint32_t rbytes = (uint32_t)(((nr + 1) * 4 + 15) & ~15);
-    mbar_expect_tx(full + s, (uint32_t)cnt4 * 12u + rbytes);
-    if (cnt4 > 0) {
-      bulk_g2s_stream(st[s].vals, vals + s4, (uint32_t)cnt4 * 8u, full + s, stream_policy);
-      bulk_g2s_stream(st[s].cols, colidx + s4, (uint32_t)cnt4 * 4u, full + s, stream_policy);
-    }
-    bulk_g2s_stream(st[s].rows, rowptr + r0, rbytes, full + s, stream_policy);
-  };
-  if (tid == 0) {
-    for (int k = 0; k < kStages - 1; ++k) {
-      const int tile = blockIdx.x + k * gridDim.x;
-      if (tile < ntiles) issue(tile, k);
-    }
-  }
-  // Programmatic dependent launch: everything above only touches the matrix (complete long before
-  // the preceding kernel started); x, b, y and the reduction scratch are used below.  A no-op when
-  // the kernel was launched without the attribute.
-  asm volatile("griddepcontrol.wait;" ::: "memory");
   double nrm = 0.0, nrb = 0.0;
-  int it = 0;
-  for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++it) {
-    const int s = it % kStages;
-    if (tid == 0) {
-      const int pre = tile + (kStages - 1) * gridDim.x;
-      if (pre < ntiles) {
-        // the stage being refilled was multiplied in place by generic-proxy stores
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        issue(pre, (it + kStages - 1) % kStages);
+  if (tid >= kTileRows) {
+    if (tid == kTileRows)
+      spmv_produce(n, ntiles, rowptr, colidx, vals, tile_base, ring, full, empty, end, slot_off);
+    else
+      asm volatile("griddepcontrol.wait;" ::: "memory");
+  } else {
+    // Programmatic dependent launch: x, b, y and the reduction scratch are only touched after this (a
+    // no-op when the kernel was launched without the attribute); the producer streams the matrix meanwhile.
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    int k = 0;
+    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++k) {
+      const int d = k % kRingDescs;
+      const int r0 = tile * kTileRows;
+      const int nr = min(kTileRows, n - r0);
+      double bi = 0.0;
+      if (MODE >= 1 && tid < nr) bi = __ldcs(b + r0 + tid);
+      mbar_wait(full + d, (uint32_t)((k / kRingDescs) & 1));
+      const unsigned char* t = ring + slot_off[d];
+      const int32_t* rows = reinterpret_cast<const int32_t*>(t);
+      const int base = rows[0];
+      const int cnt4 = ((rows[nr] + 3) & ~3) - (base & ~3);
+      const int32_t* cols = reinterpret_cast<const int32_t*>(t + pipe_tile_bytes(nr, 0)) + (base & 3);
+      const double* vv = reinterpret_cast<const double*>(t + pipe_tile_bytes(nr, 0) + cnt4 * 4) + (base & 3);
+      if (tid >= nr) {
+        mbar_arrive(empty + d);
+        continue;
       }
-    }
-    const int r0 = tile * kTileRows;
-    const int nr = min(kTileRows, n - r0);
-    double bi = 0.0;
-    if (MODE >= 1 && tid < nr) bi = __ldcs(b + r0 + tid);
-    mbar_wait(full + s, (uint32_t)((it / kStages) & 1));
-    SpmvStage& S = st[s];
-    const int base = S.rows[0];
-    const int off = base & 3;
-    const int tnnz = S.rows[nr] - base;
-    constexpr int kPer = kPipeCap / kTileRows;
-    int c[kPer];
-    double xv[kPer];
-#pragma unroll
-    for (int k = 0; k < kPer; ++k) {
-      const int idx = tid + k * kTileRows;
-      if (idx < tnnz) c[k] = S.cols[off + idx];
-    }
-#pragma unroll
-    for (int k = 0; k < kPer; ++k) {
-      const int idx = tid + k * kTileRows;
-      if (idx < tnnz) xv[k] = x[c[k]];
-    }
-#pragma unroll
-    for (int k = 0; k < kPer; ++k) {
-      const int idx = tid + k * kTileRows;
-      if (idx < tnnz) S.vals[off + idx] = __dmul_rn(S.vals[off + idx], xv[k]);
-    }
-    __syncthreads();
-    if (tid < nr) {
-      const int rs = S.rows[tid] - base + off, re = S.rows[tid + 1] - base + off;
+      const int rs = rows[tid] - base, len = rows[tid + 1] - rows[tid];
       double acc = 0.0;
-      for (int k = rs; k < re; ++k) acc = __dadd_rn(acc, S.vals[k]);
+      if (len <= kRowRegs) {
+        int c[kRowRegs];
+        double v[kRowRegs], xv[kRowRegs];
+#pragma unroll
+        for (int j = 0; j < kRowRegs; ++j)
+          if (j < len) {
+            c[j] = cols[rs + j];
+            v[j] = vv[rs + j];
+          }
+        mbar_arrive(empty + d);
+#pragma unroll
+        for (int j = 0; j < kRowRegs; ++j)
+          if (j < len) xv[j] = x[c[j]];
+#pragma unroll
+        for (int j = 0; j < kRowRegs; ++j)
+          if (j < len) acc = __dadd_rn(acc, __dmul_rn(v[j], xv[j]));
+      } else {
+        for (int j = 0; j < len; ++j) acc = __dadd_rn(acc, __dmul_rn(vv[rs + j], x[cols[rs + j]]));
+        mbar_arrive(empty + d);
+      }
       if (MODE == 0) {
         y[r0 + tid] = acc;
       } else {
@@ -311,29 +361,26 @@ spmv_pipe_kernel(int n, int ntiles, const int32_t* __restrict__ rowptr,
         }
       }
     }
-    // order this thread's generic-proxy accesses to the stage before the TMA refill
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    __syncthreads();
   }
   if (MODE >= 1 && MODE < 3) {
-    double mine[2] = {block_sum<kTileRows>(nrm, red), block_sum<kTileRows>(nrb, red)};
-    finish_partials<kTileRows, 2>(mine, partial, gridDim.x, ticket, norm2_out, red);
+    double mine[2] = {block_sum<kPipeThreads>(nrm, red), block_sum<kPipeThreads>(nrb, red)};
+    finish_partials<kPipeThreads, 2>(mine, partial, gridDim.x, ticket, norm2_out, red);
   }
   if (MODE == 3) {
     __shared__ double loc[2];
-    double mine[2] = {block_sum<kTileRows>(nrm, red), block_sum<kTileRows>(nrb, red)};
-    if (!finish_partials<kTileRows, 2>(mine, partial, gridDim.x, ticket, loc, red)) return;
+    double mine[2] = {block_sum<kPipeThreads>(nrm, red), block_sum<kPipeThreads>(nrb, red)};
+    if (!finish_partials<kPipeThreads, 2>(mine, partial, gridDim.x, ticket, loc, red)) return;
     __syncthreads();  // loc[] written by thread 0
     peer_ll_send(pc, 1, n_shared + 2,
                  [&](int i) { return i < n_shared ? __ldcg(lam_scratch + shared_lm[i]) : loc[i - n_shared]; });
     double acc = 0.0;
-    for (int i = tid; i < n_shared; i += kTileRows) {
+    for (int i = tid; i < n_shared; i += kPipeThreads) {
       double v = 0.0;
       for (int src = 0; src < pc.nranks; ++src) v += peer_ll_recv(pc, 1, src, i);  // rank order
       if (y) y[loff + shared_lm[i]] = v;
       acc += v * v;
     }
-    acc = block_sum<kTileRows>(acc, red);
+    acc = block_sum<kPipeThreads>(acc, red);
     if (tid == 0) {
       double s0 = acc, s1 = 0.0;
       for (int src = 0; src < pc.nranks; ++src) {
