@@ -116,6 +116,16 @@ int nxfx_matrix_destroy(nxfx_ctx* ctx, int64_t mat_id);
 int nxfx_matrix_bind(nxfx_ctx* ctx, int64_t mat_id);
 int nxfx_matrix_zero(nxfx_ctx* ctx);                    /* MatZeroEntries on the bound matrix */
 int nxfx_matrix_info(nxfx_ctx* ctx, int64_t* mat_id, int32_t* assembled, int32_t* acc_count);
+/* Pattern-only entries.  With flux degree 1 / pressure degree 0 the pressure rows ({-1, +1}) and the
+ * multiplier rows ((0, +1) / (-1, 0)) of the matrix depend on the pattern alone.  After a non-accumulating
+ * lhs nxfx_assemble the bound matrix remembers that its values hold them, and the next non-accumulating
+ * assembly writes only the flux rows (and b).  nxfx_matrix_zero, an accumulating assembly and a new pattern
+ * forget it.  A caller that writes the values itself through the pointer of nxfx_csr_device (or any copy of
+ * it) must bind that matrix and call nxfx_matrix_touch after the write and before the next nxfx_assemble --
+ * as PETSc's MatSeqAIJGetArray is followed by MatSeqAIJRestoreArray.  nxfx_matrix_static_valid reports the
+ * state (1: the next overwrite skips those rows).                                                 */
+int nxfx_matrix_touch(nxfx_ctx* ctx);
+int nxfx_matrix_static_valid(nxfx_ctx* ctx, int32_t* valid);
 
 /* ---- (3) numeric assembly ----------------------------------------------------------------- *
  * Replaces fem.petsc.assemble_matrix + A.assemble() + assemble_vector + ghost update:

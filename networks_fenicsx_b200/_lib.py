@@ -88,6 +88,8 @@ SIGNATURES = {
     "nxfx_matrix_info": (
         C.c_int, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
     ),
+    "nxfx_matrix_touch": (C.c_int, [C.c_void_p]),
+    "nxfx_matrix_static_valid": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
     "nxfx_set_boundary_pressure": (C.c_int, [C.c_void_p, C.c_void_p]),
     "nxfx_assemble": (
         C.c_int,

@@ -51,6 +51,7 @@ struct Net {
   int32_t nq, poff, loff, ndofs;
   FastDiv div_np1, div_n;  // divide by N+1 / N (valid when N >= 2)
   const int4* __restrict__ slot_uvl;
+  const int2* __restrict__ slot_lm;  // [E] {lm(u), lm(v)} in slot order (N == 1 back-substitution: 8 instead of 16 bytes)
   const int32_t* __restrict__ slot_edge;
   const int32_t* __restrict__ edge_slot;
   const int32_t* __restrict__ bif_ptr;
@@ -515,7 +516,8 @@ __device__ __forceinline__ void flux_tile_gen(const Net& g, const Coef& c, const
   }
 }
 
-// pressure tile: a[P][i] = +int phi dq/ds: B = [-1, +1] (assembly.py:254); L[P] = int f phi (:262)
+// pressure tile: a[P][i] = +int phi dq/ds: B = [-1, +1] (assembly.py:254); L[P] = int f phi (:262).
+// lhs == 0 (rhs only, or the values are already in place: see MatState::static_valid) writes b alone.
 template <bool ACC, bool N1>
 __device__ __forceinline__ void pressure_tile(const Net& g, const Coef& c, const int32_t* __restrict__ rowptr,
                                               double* __restrict__ vals, double* __restrict__ b, int lhs,
@@ -562,10 +564,12 @@ __device__ __forceinline__ void lambda_tile(const Net& g, const int32_t* __restr
     for (int i = i0 + threadIdx.x; i < i1; i += blockDim.x) NXFX_STB1(b + g.loff + i, 0.0);
 }
 
+// write_static == 0: the pressure and multiplier rows of vals already hold what this assembly would store
+// there (a re-assembly without ADD_VALUES, MatState::static_valid); their tiles then write b only.
 template <bool ACC, bool N1>
 __global__ void __launch_bounds__(kTileRows)
 assemble_tiles_kernel(Net g, Coef c, const int32_t* __restrict__ rowptr, double* __restrict__ vals,
-                      double* __restrict__ b, int lhs, int rhs, int n_flux_tiles, int n_pres_tiles) {
+                      double* __restrict__ b, int lhs, int rhs, int write_static, int n_flux_tiles, int n_pres_tiles) {
   __shared__ __align__(16) double sm[kAsmCap + 2];
   // a kernel launched as programmatic dependent (the fused tree kernel) may stage its schedule
   // tables while the last wave of this grid drains; it waits for this grid before reading any output
@@ -577,9 +581,9 @@ assemble_tiles_kernel(Net g, Coef c, const int32_t* __restrict__ rowptr, double*
     if (N1) flux_tile_n1<ACC>(g, c, rowptr, vals, b, lhs, rhs, t, sm);
     else flux_tile_gen<ACC>(g, c, rowptr, vals, b, lhs, rhs, t, sm);
   } else if (t < n_flux_tiles + n_pres_tiles) {
-    pressure_tile<ACC, N1>(g, c, rowptr, vals, b, lhs, rhs, t - n_flux_tiles);
+    pressure_tile<ACC, N1>(g, c, rowptr, vals, b, lhs && write_static, rhs, t - n_flux_tiles);
   } else {
-    lambda_tile<ACC>(g, rowptr, vals, b, lhs, rhs, t - n_flux_tiles - n_pres_tiles);
+    lambda_tile<ACC>(g, rowptr, vals, b, lhs && write_static, rhs, t - n_flux_tiles - n_pres_tiles);
   }
 }
 

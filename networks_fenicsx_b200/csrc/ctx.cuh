@@ -66,6 +66,11 @@ struct MatState {
   DevBuf<double> cell_rh;  // [nc] sum over the accumulated assemblies of R*h (N == 1: in flux-slot order)
   bool assembled = false;
   int acc_count = 0;  // number of lhs assemblies accumulated since the last zero (ADD_VALUES)
+  // vals holds, bit for bit, the pressure-row {-1, +1} and multiplier-row (0, +1) / (-1, 0) entries that a
+  // non-accumulating P1/DG0 lhs assembly writes: they depend on the pattern alone, so the next such
+  // assembly leaves them in place.  Set by that assembly; cleared by nxfx_matrix_zero, nxfx_matrix_touch
+  // and every accumulating or table-driven lhs assembly.
+  bool static_valid = false;
 };
 
 // Exact condensation of the table-driven (higher-order) path (condense.cuh): per-edge-type entry lists from
@@ -114,6 +119,7 @@ struct nxfx_ctx {
   nxfx::DevBuf<double> pos_stage;  // [n_nodes*gdim] upload staging
   nxfx::DevBuf<int4> slot_uvl;     // [E] {u, v, lm(u), lm(v)} in slot order
   nxfx::DevBuf<int2> slot_uv;      // [E] {u, v} in slot order (N == 1 assembly)
+  nxfx::DevBuf<int2> slot_lm;      // [E] {lm(u), lm(v)} in slot order (N == 1 back-substitution)
   nxfx::DevBuf<uint32_t> bif_in_bits;  // [ceil(n_inc / 32)] in-edge flag of every incidence
   nxfx::DevBuf<int32_t> slot_edge, edge_slot, edge_u, edge_v, bif_ptr, bif_inc;
   // pattern + values

@@ -36,6 +36,7 @@ Net make_net(const nxfx_ctx* c) {
   g.div_np1 = make_fastdiv((uint32_t)c->N + 1);
   g.div_n = make_fastdiv((uint32_t)std::max(c->N, 2));
   g.slot_uvl = c->slot_uvl.p;
+  g.slot_lm = c->slot_lm.p;
   g.slot_edge = c->slot_edge.p;
   g.edge_slot = c->edge_slot.p;
   g.bif_ptr = c->bif_ptr.p;
@@ -204,6 +205,7 @@ void note_lhs_assembled(nxfx_ctx* ctx, int accumulate) {
   MatState* m = ctx->cur;
   m->acc_count = (accumulate && m->assembled) ? m->acc_count + 1 : 1;
   m->assembled = true;
+  m->static_valid = false;  // nxfx_assemble sets it again after a non-accumulating P1/DG0 assembly
   ctx->pc_ready = false;
   ctx->bottom_factored = false;
 }
@@ -1185,6 +1187,9 @@ int nxfx_set_network(nxfx_ctx* ctx, int32_t n_nodes, int32_t n_edges, int32_t gd
   std::vector<int2> uv((size_t)E);
   for (int64_t s = 0; s < E; ++s) uv[s] = make_int2(uvl[s].x, uvl[s].y);
   if ((rc = upload(ctx, ctx->slot_uv, uv.data(), (size_t)E))) return rc;
+  std::vector<int2> lm((size_t)E);
+  for (int64_t s = 0; s < E; ++s) lm[s] = make_int2(uvl[s].z, uvl[s].w);
+  if ((rc = upload(ctx, ctx->slot_lm, lm.data(), (size_t)E))) return rc;
   std::vector<uint32_t> in_bits((size_t)(n_inc + 31) / 32 + 1, 0u);
   for (int32_t k = 0; k < n_inc; ++k)
     if (bif_inc[k] & 1) in_bits[k >> 5] |= 1u << (k & 31);
@@ -1311,7 +1316,24 @@ int nxfx_matrix_zero(nxfx_ctx* ctx) {
   NXFX_CUDA(ctx, cudaMemsetAsync(m->cell_rh.p, 0, m->cell_rh.n * sizeof(double), ctx->stream));
   m->assembled = false;
   m->acc_count = 0;
+  m->static_valid = false;
   if (ctx->pc_mat == m->id) ctx->pc_ready = false;
+  return NXFX_OK;
+}
+
+int nxfx_matrix_touch(nxfx_ctx* ctx) {
+  if (!ctx) return NXFX_ERR_INVALID;
+  NXFX_REQUIRE(ctx, ctx->has_pattern, "symbolic phase has not been run");
+  { int rc = ensure_matrix(ctx); if (rc) return rc; }
+  ctx->cur->static_valid = false;
+  return NXFX_OK;
+}
+
+int nxfx_matrix_static_valid(nxfx_ctx* ctx, int32_t* valid) {
+  if (!ctx || !valid) return NXFX_ERR_INVALID;
+  NXFX_REQUIRE(ctx, ctx->has_pattern, "symbolic phase has not been run");
+  { int rc = ensure_matrix(ctx); if (rc) return rc; }
+  *valid = ctx->cur->static_valid;
   return NXFX_OK;
 }
 
@@ -1362,14 +1384,19 @@ int nxfx_assemble(nxfx_ctx* ctx, const double* R_cell, double R_const, const dou
   const int npt = (int)cdiv(ctx->nc, kPresRows);
   const int nlt = (int)cdiv(ctx->n_bif, kLamRows);
   const int grid = nft + npt + nlt;
+  // a re-assembly that overwrites leaves the pressure / multiplier rows (pattern-only values) in place
+  const int ws = !(lhs && !accumulate && ctx->cur->static_valid);
   if (accumulate) {
-    if (n1) NXFX_LAUNCH(ctx, (assemble_tiles_kernel<true, true>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, nft, npt);
-    else NXFX_LAUNCH(ctx, (assemble_tiles_kernel<true, false>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, nft, npt);
+    if (n1) NXFX_LAUNCH(ctx, (assemble_tiles_kernel<true, true>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, ws, nft, npt);
+    else NXFX_LAUNCH(ctx, (assemble_tiles_kernel<true, false>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, ws, nft, npt);
   } else {
-    if (n1) NXFX_LAUNCH(ctx, (assemble_tiles_kernel<false, true>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, nft, npt);
-    else NXFX_LAUNCH(ctx, (assemble_tiles_kernel<false, false>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, nft, npt);
+    if (n1) NXFX_LAUNCH(ctx, (assemble_tiles_kernel<false, true>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, ws, nft, npt);
+    else NXFX_LAUNCH(ctx, (assemble_tiles_kernel<false, false>), grid, kTileRows, 0, g, c, ctx->rowptr.p, ctx->cur->vals.p, b, lhs, rhs, ws, nft, npt);
   }
-  if (lhs) note_lhs_assembled(ctx, accumulate);
+  if (lhs) {
+    note_lhs_assembled(ctx, accumulate);
+    ctx->cur->static_valid = !accumulate;  // ADD_VALUES turns them into k * {-1, +1}, k * (0, +-1)
+  }
   return NXFX_OK;
 }
 

@@ -1301,16 +1301,16 @@ edge_backsub_n1_kernel(Net g, TreeDev t, const double* __restrict__ cell_rh, con
   }
   // as a programmatic dependent of the tree kernel: r and cell_rh are older than that kernel
   // (it releases its dependents only after its own wait), the multipliers are its output.
-  // Thread <-> flux SLOT: the slot record, the flux pair of r / z and cell_rh are contiguous accesses;
+  // Thread <-> flux SLOT: the multiplier pair, the flux pair of r / z and cell_rh are contiguous accesses;
   // only the pressure entry (cell order) is indexed through slot_edge.
   const int slot = idx;
-  const int4 uv = g.slot_uvl[slot];
+  const int2 lm = g.slot_lm[slot];
   const int e = g.slot_edge[slot];
   const double2 rq = *reinterpret_cast<const double2*>(r + 2 * (size_t)slot);
   const double rp = r[g.poff + e], rh = cell_rh[slot];
   asm volatile("griddepcontrol.wait;" ::: "memory");
-  const double lu = uv.z >= 0 ? t.lam_nat[uv.z] : 0.0;
-  const double lv = uv.w >= 0 ? t.lam_nat[uv.w] : 0.0;
+  const double lu = lm.x >= 0 ? t.lam_nat[lm.x] : 0.0;
+  const double lv = lm.y >= 0 ? t.lam_nat[lm.y] : 0.0;
   const double c = (rq.x + rq.y) - 0.5 * rh * rp;
   const double q0 = (c + lu - lv) / rh;
   const double q1 = q0 + rp;

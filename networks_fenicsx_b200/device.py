@@ -82,13 +82,16 @@ def default_device(index: int = 0) -> Device:
 
 
 class DeviceArray:
-    """Flat device buffer of ``n`` elements."""
+    """Flat device buffer of ``n`` elements.  ``on_write`` (optional) is called after every write this
+    object or a view of it makes (``upload``, ``zero``): the owner of a borrowed buffer learns that its
+    contents changed (``Mat.values``: ``Mat.touch``)."""
 
-    def __init__(self, dev: Device, n: int, dtype=np.float64, ptr: int | None = None):
+    def __init__(self, dev: Device, n: int, dtype=np.float64, ptr: int | None = None, on_write=None):
         self.dev = dev
         self.n = int(n)
         self.dtype = np.dtype(dtype)
         self.owned = ptr is None
+        self.on_write = on_write
         if ptr is None:
             p = C.c_void_p()
             dev.call("nxfx_malloc", C.c_size_t(self.nbytes), C.byref(p))
@@ -112,6 +115,8 @@ class DeviceArray:
             self.dev.call("nxfx_memcpy_h2d", self.c_ptr, C.c_void_p(host.ctypes.data), C.c_size_t(self.nbytes))
         if sync:
             self.dev.sync()
+        if self.on_write is not None:
+            self.on_write()
 
     def download(self, out: np.ndarray | None = None, sync: bool = True) -> np.ndarray:
         if out is None:
@@ -126,9 +131,11 @@ class DeviceArray:
     def zero(self) -> None:
         if self.n:
             self.dev.call("nxfx_memset", self.c_ptr, 0, C.c_size_t(self.nbytes))
+        if self.on_write is not None:
+            self.on_write()
 
     def view(self, offset: int, n: int) -> "DeviceArray":
         assert 0 <= offset and offset + n <= self.n
-        v = DeviceArray(self.dev, n, self.dtype, ptr=self.ptr + offset * self.dtype.itemsize)
+        v = DeviceArray(self.dev, n, self.dtype, ptr=self.ptr + offset * self.dtype.itemsize, on_write=self.on_write)
         v._keepalive = self
         return v

@@ -153,6 +153,17 @@ class Vec:
         return PETSc.Vec().createWithArray(self.array_r.copy())
 
 
+class _Touch:
+    """``nxfx_matrix_touch`` of one matrix: the values were written other than by the assembly."""
+
+    def __init__(self, dev: Device, mat_id: int):
+        self.dev, self.mat_id = dev, mat_id
+
+    def __call__(self) -> None:
+        self.dev.call("nxfx_matrix_bind", C.c_int64(self.mat_id))
+        self.dev.call("nxfx_matrix_touch")
+
+
 class Mat:
     """Monolithic CSR matrix on the pattern of the device context (``nxfx_symbolic``).  Every ``Mat``
     owns its value array (``nxfx_matrix_create``) -- the reference hands out independent PETSc
@@ -177,7 +188,9 @@ class Mat:
         dev.call("nxfx_csr_device", C.byref(rp), C.byref(ci), C.byref(va))
         self.rowptr = DeviceArray(dev, self.n + 1, np.int32, ptr=rp.value)
         self.colidx = DeviceArray(dev, self.nnz, np.int32, ptr=ci.value)
-        self.values = DeviceArray(dev, self.nnz, np.float64, ptr=va.value)
+        # a write through Mat.values (upload, zero, or a view's) tells the library (nxfx_matrix_touch); the
+        # callback holds the device and the id, not the Mat, so that the Mat is still freed by refcount
+        self.values = DeviceArray(dev, self.nnz, np.float64, ptr=va.value, on_write=_Touch(dev, self.mat_id))
         self._zero_pending = True  # a new matrix is zero
         self._pattern_host = None
         self._prefix = ""
@@ -186,6 +199,21 @@ class Mat:
     def bind(self) -> None:
         """Make this matrix the target / operator of the following device calls."""
         self.dev.call("nxfx_matrix_bind", C.c_int64(self.mat_id))
+
+    def touch(self) -> None:
+        """Declare that the values were written other than by the assembly (a kernel of the caller's own
+        through ``values.ptr``, say): the next assembly then writes every entry again.  Writes made through
+        ``values.upload`` / ``values.zero`` call this themselves."""
+        _Touch(self.dev, self.mat_id)()
+
+    @property
+    def static_valid(self) -> bool:
+        """True if the values hold the pattern-only entries of an assembly (pressure and multiplier rows),
+        which the next overwriting assembly then leaves in place (``nxfx_matrix_static_valid``)."""
+        self.bind()
+        v = C.c_int32()
+        self.dev.call("nxfx_matrix_static_valid", C.byref(v))
+        return bool(v.value)
 
     @property
     def accumulated(self) -> int:
