@@ -472,7 +472,7 @@ btree_sweep_kernel(TreeDev t, CondDev c, int chunk0) {
   }
 }
 
-// Top chunk of a partitioned network, split around the caller's all-reduce (block version of tree_top_kernel's
+// Top chunk of a partitioned network, split around the caller's all-reduce (block version of tree_top_split_kernel's
 // kPartial / kFinish, precond.cuh).  sh_idx[i]: position k of top-chunk node b0 + i in the exchanged order of the
 // shared nodes (identical on every rank), -1 for a node private to this rank (sh_idx == nullptr: no shared node).
 // Payload, nt = max(n_shared, 1):

@@ -8,6 +8,7 @@
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
+#include <type_traits>
 
 #include "assemble.cuh"
 #include "ctx.cuh"
@@ -764,12 +765,14 @@ int forward_bottom(nxfx_ctx* ctx, const double* r) {
 }
 
 // the top chunk's half of a split phase: kPartial packs this rank's partial sums of the shared nodes into buf,
-// kFinish completes from the all-reduced buf (precond.cuh tree_top_kernel, condense.cuh btree_top_split_kernel)
+// kFinish completes from the all-reduced buf (precond.cuh tree_top_split_kernel, condense.cuh btree_top_split_kernel)
 template <bool FACTOR, int PHASE>
 int top_split(nxfx_ctx* ctx, double* buf) {
   const int top = ctx->tree.n_chunks - 1;
   if (!ctx->generic) {
-    NXFX_LAUNCH(ctx, (tree_top_kernel<FACTOR, PHASE>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), top, buf);
+    using Op = std::conditional_t<FACTOR, FactorOp, SolveOp>;
+    NXFX_LAUNCH(ctx, (tree_top_split_kernel<Op, PHASE>), 1, kTreeThreads, tree_smem_bytes(ctx->tree.cap), make_tree(ctx), top, buf,
+                (FusedN1{make_net(ctx), nullptr, nullptr}));
     return NXFX_OK;
   }
   if (ctx->n_bif == 0) return NXFX_OK;
@@ -1495,8 +1498,8 @@ int nxfx_set_tree_schedule(nxfx_ctx* ctx, const int32_t* t_of_bif, const int32_t
       s.coop_ok = n_chunks <= per_sm * ctx->sm_count;  // bottom blocks + one block for the top chunk
     cudaGetLastError();
     NXFX_CUDA(ctx, cudaFuncSetAttribute(tree_factor_solve_bottom_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes_fs(kChunkCapMax)));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute(tree_top_fs_kernel<kPartial>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes_fs(kChunkCapMax)));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute(tree_top_fs_kernel<kFinish>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes_fs(kChunkCapMax)));
+    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_split_kernel<FactorSolveOp, kPartial>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes_fs(kChunkCapMax)));
+    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_split_kernel<FactorSolveOp, kFinish>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes_fs(kChunkCapMax)));
     s.coop_fs_ok = false;
     per_sm = 0;
     const int fs_max = (int)tree_smem_bytes_fs(kChunkCapMax);
@@ -1513,10 +1516,10 @@ int nxfx_set_tree_schedule(nxfx_ctx* ctx, const int32_t* t_of_bif, const int32_t
     }
     cudaGetLastError();
     NXFX_CUDA(ctx, cudaFuncSetAttribute(tree_factor_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_kernel<true, kPartial>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_kernel<true, kFinish>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_kernel<false, kPartial>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
-    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_kernel<false, kFinish>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
+    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_split_kernel<FactorOp, kPartial>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
+    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_split_kernel<FactorOp, kFinish>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
+    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_split_kernel<SolveOp, kPartial>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
+    NXFX_CUDA(ctx, cudaFuncSetAttribute((tree_top_split_kernel<SolveOp, kFinish>), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
     NXFX_CUDA(ctx, cudaFuncSetAttribute(tree_solve_kernel<kTreeUp>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
     NXFX_CUDA(ctx, cudaFuncSetAttribute(tree_solve_kernel<kTreeDown>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tree_smem_bytes(kChunkCapMax)));
   }
@@ -1913,7 +1916,7 @@ int nxfx_pc_setup_apply_begin(nxfx_ctx* ctx, const double* r, double* buf) {
   FusedN1 fin{make_net(ctx), r, ctx->cur->cell_rh.p, ctx->lam_weight.p};
   const size_t smem = tree_smem_bytes_fs(s.cap);
   if (nb > 0) NXFX_LAUNCH(ctx, tree_factor_solve_bottom_kernel, nb, kTreeThreads, smem, t, fin);
-  NXFX_LAUNCH(ctx, tree_top_fs_kernel<kPartial>, 1, kTreeThreads, smem, t, nb, buf, fin);
+  NXFX_LAUNCH(ctx, (tree_top_split_kernel<FactorSolveOp, kPartial>), 1, kTreeThreads, smem, t, nb, buf, fin);
   ctx->bottom_factored = true;
   return NXFX_OK;
 }
@@ -1930,7 +1933,7 @@ int nxfx_pc_setup_apply_end(nxfx_ctx* ctx, const double* r, double* z, double* b
   }
   NXFX_REQUIRE(ctx, ctx->bottom_factored, "nxfx_pc_setup_apply_begin has not been run");
   FusedN1 fin{make_net(ctx), r, ctx->cur->cell_rh.p, ctx->lam_weight.p};
-  NXFX_LAUNCH(ctx, tree_top_fs_kernel<kFinish>, 1, kTreeThreads, tree_smem_bytes_fs(ctx->tree.cap), make_tree(ctx),
+  NXFX_LAUNCH(ctx, (tree_top_split_kernel<FactorSolveOp, kFinish>), 1, kTreeThreads, tree_smem_bytes_fs(ctx->tree.cap), make_tree(ctx),
               ctx->tree.n_chunks - 1, buf, fin);
   mark_factored(ctx);
   return backward_bottom(ctx, r, z, false);

@@ -16,6 +16,8 @@
 // as A; P^{-1} A = I up to rounding on forests.
 #pragma once
 
+#include <type_traits>
+
 #include "assemble.cuh"
 #include "peer.cuh"
 #include "spmv.cuh"
@@ -422,199 +424,298 @@ __device__ __forceinline__ void load_children(const TreeDev& t, const ChunkInfo&
   for (int i = threadIdx.x; i < ci.ce - ci.cb; i += blockDim.x) S.cidx[i] = t.t_cidx[ci.cb + i];
 }
 
-// Phases of the top chunk (multi-GPU, host-driven all-reduce): kPartial stops after folding in this
-// rank's bottom-chunk children, parks the partial sums of ALL top-chunk nodes in global scratch and packs
-// those of the SHARED nodes (t.top_sh_pos) into `buf` (all-reduced by the caller); kFinish reloads the
-// scratch and takes the shared nodes from the all-reduced buffer.  kFull = single GPU.
-enum { kFull = 0, kPartial = 1, kFinish = 2 };
-
-// numeric factorisation of one chunk: d_n = diag0_n - sum_c tg_c * gd_c, gd_n = tg_n / d_n;
-// t.d receives 1/d.  `top`: children below b0 live in bottom chunks (already written to HBM).
-// Partitioned network (t.n_sh > 0, top chunk): kPartial eliminates the nodes PRIVATE to this rank, folds them
-// into their shared parents and packs [partial d | tg] of the shared nodes into buf (2 * n_sh doubles);
-// kFinish takes the all-reduced buf and eliminates the shared nodes (identically on every rank).
-__device__ __forceinline__ void factor_chunk(const TreeDev& t, const TreeSmem& S, int chunk, bool top,
-                                             int phase = kFull, double* buf = nullptr,
-                                             const FusedN1* f = nullptr) {
-  const ChunkInfo ci = load_chunk_info(t, chunk, S);
-  const int b0 = ci.b0, nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
-  const int ns = top ? t.n_sh : 0;
-  load_children(t, ci, S);
-  for (int i = tid; i < nn; i += nth) S.par[i] = t.t_parent[b0 + i];
-  if (top && phase != kFull) load_shared_flags(t, ci, S);
-  auto eliminate = [&](bool shared_children_only) {
-    return [&, shared_children_only](int n) {
-      const int i = n - b0;
-      double acc = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0 && (!shared_children_only || tree_shared(S, c))) acc -= S.b[c] * S.c[c];
-      }
-      const double inv = 1.0 / acc;
-      S.a[i] = inv;
-      S.c[i] = S.b[i] * inv;
-    };
-  };
-  if (phase == kFinish) {
-    // private nodes: final (1/d, gd) from kPartial; shared nodes: the all-reduced partial sums
-    for (int i = tid; i < nn; i += nth) { S.a[i] = t.d[b0 + i]; S.c[i] = t.gd[b0 + i]; S.b[i] = 0.0; }
-    __syncthreads();
-    for (int k = tid; k < ns; k += nth) {
-      const int j = t.top_sh_pos[k];
-      S.a[j] = buf[k];
-      S.b[j] = buf[ns + k];
-    }
-    __syncthreads();
-    sweep_up_sel(S, ci, eliminate(true), kSharedNodes, 0, t.sh_lmax);
-    for (int k = tid; k < ns; k += nth) {
-      const int j = t.top_sh_pos[k];
-      t.d[b0 + j] = S.a[j];
-      t.gd[b0 + j] = S.c[j];
-    }
-    return;
-  }
-  if (f) {
-    for (int i = tid; i < nn; i += nth) {
-      S.a[i] = n1_node_diag(*f, t, b0 + i);
-      const int pe = t.t_pslot[b0 + i];
-      const double tg = pe >= 0 ? 1.0 / f->cell_rh[pe] : 0.0;
-      S.b[i] = tg;
-      // the top chunk reads the link conductances of its bottom-chunk children (the chunk roots)
-      const int p = t.t_parent[b0 + i];
-      if (p < b0 || p >= ci.b1) t.tg[b0 + i] = tg;
-    }
-  } else {
-    for (int i = tid; i < nn; i += nth) { S.a[i] = t.diag0[b0 + i]; S.b[i] = t.tg[b0 + i]; }
-  }
-  __syncthreads();
-  if (top) {
-    for (int i = tid; i < nn; i += nth) {
-      double acc = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k];
-        if (c < b0) acc -= t.tg[c] * __ldcg(t.gd + c);
-      }
-      S.a[i] = acc;
-    }
-    __syncthreads();
-  }
-  if (phase == kFull) {  // single GPU / bottom chunk: the plain sweep
-    sweep_up(S, ci, [&](int n) {
-      const int i = n - b0;
-      double acc = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0) acc -= S.b[c] * S.c[c];
-      }
-      const double inv = 1.0 / acc;
-      S.a[i] = inv;
-      S.c[i] = S.b[i] * inv;
-    });
-    for (int i = tid; i < nn; i += nth) { t.d[b0 + i] = S.a[i]; t.gd[b0 + i] = S.c[i]; }
-    return;
-  }
-  // kPartial
-  sweep_up_sel(S, ci, eliminate(false), kPrivateNodes, t.pr_lmin, 1 << 30);
-  for (int k = tid; k < ns; k += nth) {  // private children of the shared nodes
-    const int j = t.top_sh_pos[k];
-    double acc = S.a[j];
-    for (int q = S.cptr[j]; q < S.cptr[j + 1]; ++q) {
-      const int c = S.cidx[q] - b0;
-      if (c >= 0 && !tree_shared(S, c)) acc -= S.b[c] * S.c[c];
-    }
-    S.a[j] = acc;
-  }
-  __syncthreads();
-  for (int i = tid; i < nn; i += nth) {
-    t.d[b0 + i] = S.a[i];                       // private: 1/d (final); shared: partial d
-    t.gd[b0 + i] = tree_shared(S, i) ? S.b[i] : S.c[i];  // private: gd (final); shared: link conductance
-  }
-  for (int k = tid; k < ns; k += nth) {
-    const int j = t.top_sh_pos[k];
-    buf[k] = S.a[j];
-    buf[ns + k] = S.b[j];
-  }
-}
+// Phases of the top chunk of a partitioned network around a host-driven all-reduce (tree_top_split_kernel).
+enum { kPartial = 1, kFinish = 2 };
 
 // stage a chunk for the solve: a = r, b = 1/d, c = gd, par
-__device__ __forceinline__ void load_solve_chunk(const TreeDev& t, const ChunkInfo& ci, const TreeSmem& S,
+__device__ __forceinline__ void load_solve_chunk(const TreeDev& t, const TreeSmem& S, int b0, int b1,
                                                  const FusedN1* f = nullptr) {
-  const int nn = ci.b1 - ci.b0;
+  const int nn = b1 - b0;
   for (int i = threadIdx.x; i < nn; i += blockDim.x) {
-    S.a[i] = f ? n1_node_rhs(*f, t, ci.b0 + i) : t.r[ci.b0 + i];
-    S.b[i] = t.d[ci.b0 + i];
-    S.c[i] = t.gd[ci.b0 + i];
-    S.par[i] = t.t_parent[ci.b0 + i];
+    S.a[i] = f ? n1_node_rhs(*f, t, b0 + i) : t.r[b0 + i];
+    S.b[i] = t.d[b0 + i];
+    S.c[i] = t.gd[b0 + i];
+    S.par[i] = t.t_parent[b0 + i];
   }
 }
 
-// forward elimination of a staged chunk (S.a = r, S.b = 1/d, S.c = gd): r_n += sum_c gd_c r_c.
-// Partitioned network (top chunk): kPartial eliminates the private nodes, folds them into their shared
-// parents, parks everything in scratch (t.lam) and packs the partial right-hand sides of the shared nodes
-// into buf (n_sh doubles); kFinish continues from the all-reduced buf with the shared nodes.
-__device__ __forceinline__ void solve_up(const TreeDev& t, const TreeSmem& S, const ChunkInfo& ci, bool top,
-                                         int phase = kFull, double* buf = nullptr) {
-  const int b0 = ci.b0, nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
-  const int ns = top ? t.n_sh : 0;
-  if (top && phase != kFull) load_shared_flags(t, ci, S);
-  auto eliminate = [&](bool shared_children_only) {
-    return [&, shared_children_only](int n) {
-      const int i = n - b0;
-      double acc = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0 && (!shared_children_only || tree_shared(S, c))) acc += S.c[c] * S.a[c];
+// ---- node operations ------------------------------------------------------------------------------
+// What a leaf -> root sweep computes at a node, over the TreeSmem view of a staged chunk:
+//   FactorOp       d_n = diag0_n - sum_c tg_c gd_c; 1/d_n, gd_n = tg_n / d_n    a: d -> 1/d   b: tg        c: gd
+//   SolveOp        r_n += sum_c gd_c r_c                                     a: r          b: 1/d       c: gd
+//   FactorSolveOp  both in one pass                                         a: r          b: d -> 1/d  c: gd   e: tg
+// Each one provides
+//   stage(f)                 the chunk's own values (all threads of the block; f: from (r, R h), N == 1)
+//   fold_bottom(i)           children below b0 -- roots of bottom chunks, in global memory (top chunk)
+//   eliminate<CH, PIVOT>(n)  node n from its children that pass the filter CH, then (PIVOT) the pivot;
+//                            without the pivot it only folds the children in (partitioned top chunk)
+//   field(q, j)              exchanged partial sum q of shared node j, in the order of the exchange buffer
+//   park / restore           the global scratch that carries the top chunk from kPartial to kFinish
+//   store(i)                 the results of node i to global memory
+// The filter is spelled out in every child loop: behind a helper function the compiler schedules the
+// single-GPU sweeps differently.
+enum { kAllChildren = 0, kSharedChildren = 1, kPrivateChildren = 2 };
+
+struct FactorOp {
+  const TreeDev& t;
+  const TreeSmem& S;
+  int b0, b1;
+  static constexpr int kFields = 2;  // [partial d | tg]
+  static constexpr bool kSolves = false;
+
+  __device__ __forceinline__ void stage(const FusedN1* f) const {
+    const int nn = b1 - b0, tid = threadIdx.x, nth = blockDim.x;
+    for (int i = tid; i < nn; i += nth) S.par[i] = t.t_parent[b0 + i];
+    if (f) {
+      for (int i = tid; i < nn; i += nth) {
+        S.a[i] = n1_node_diag(*f, t, b0 + i);
+        const int pe = t.t_pslot[b0 + i];
+        const double tg = pe >= 0 ? 1.0 / f->cell_rh[pe] : 0.0;
+        S.b[i] = tg;
+        // the top chunk reads the link conductances of its bottom-chunk children (the chunk roots)
+        const int p = t.t_parent[b0 + i];
+        if (p < b0 || p >= b1) t.tg[b0 + i] = tg;
       }
-      S.a[i] = acc;
-    };
-  };
-  if (phase == kFinish) {
-    for (int i = tid; i < nn; i += nth) S.a[i] = t.lam[b0 + i];  // scratch of kPartial
-    __syncthreads();
-    for (int k = tid; k < ns; k += nth) S.a[t.top_sh_pos[k]] = buf[k];
-    __syncthreads();
-    sweep_up_sel(S, ci, eliminate(true), kSharedNodes, 0, t.sh_lmax);
-    for (int i = tid; i < nn; i += nth) t.r[b0 + i] = S.a[i];
-    return;
-  }
-  if (top) {
-    for (int i = tid; i < nn; i += nth) {
-      double acc = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k];
-        if (c < b0) acc += t.gd[c] * __ldcg(t.r + c);
-      }
-      S.a[i] = acc;
+    } else {
+      for (int i = tid; i < nn; i += nth) { S.a[i] = t.diag0[b0 + i]; S.b[i] = t.tg[b0 + i]; }
     }
-    __syncthreads();
   }
-  if (phase == kFull) {  // single GPU / bottom chunk: the plain sweep
-    sweep_up(S, ci, [&](int n) {
-      const int i = n - b0;
-      double acc = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0) acc += S.c[c] * S.a[c];
-      }
-      S.a[i] = acc;
-    });
-    for (int i = tid; i < nn; i += nth) t.r[b0 + i] = S.a[i];
-    return;
-  }
-  // kPartial
-  sweep_up_sel(S, ci, eliminate(false), kPrivateNodes, t.pr_lmin, 1 << 30);
-  for (int k = tid; k < ns; k += nth) {
-    const int j = t.top_sh_pos[k];
-    double acc = S.a[j];
-    for (int q = S.cptr[j]; q < S.cptr[j + 1]; ++q) {
-      const int c = S.cidx[q] - b0;
-      if (c >= 0 && !tree_shared(S, c)) acc += S.c[c] * S.a[c];
+  __device__ __forceinline__ void fold_bottom(int i) const {
+    double acc = S.a[i];
+    for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
+      const int c = S.cidx[k];
+      if (c < b0) acc -= t.tg[c] * __ldcg(t.gd + c);
     }
-    S.a[j] = acc;
+    S.a[i] = acc;
   }
+  template <int CH, bool PIVOT = true>
+  __device__ __forceinline__ void eliminate(int n) const {
+    const int i = n - b0;
+    double acc = S.a[i];
+    for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
+      const int c = S.cidx[k] - b0;
+      if (c >= 0 && (CH == kAllChildren || tree_shared(S, c) == (CH == kSharedChildren))) acc -= S.b[c] * S.c[c];
+    }
+    if (!PIVOT) {
+      S.a[i] = acc;
+      return;
+    }
+    const double inv = 1.0 / acc;
+    S.a[i] = inv;
+    S.c[i] = S.b[i] * inv;
+  }
+  __device__ __forceinline__ double& field(int q, int j) const { return q == 0 ? S.a[j] : S.b[j]; }
+  // private nodes: final (1/d, gd); shared nodes: (partial d, tg)
+  __device__ __forceinline__ void park(int i) const {
+    t.d[b0 + i] = S.a[i];
+    t.gd[b0 + i] = tree_shared(S, i) ? S.b[i] : S.c[i];
+  }
+  __device__ __forceinline__ void restore(int i) const { S.a[i] = t.d[b0 + i]; S.c[i] = t.gd[b0 + i]; S.b[i] = 0.0; }
+  __device__ __forceinline__ void store(int i) const { t.d[b0 + i] = S.a[i]; t.gd[b0 + i] = S.c[i]; }
+};
+
+struct SolveOp {
+  const TreeDev& t;
+  const TreeSmem& S;
+  int b0, b1;
+  static constexpr int kFields = 1;  // [partial rhs]
+  static constexpr bool kSolves = true;
+
+  __device__ __forceinline__ void stage(const FusedN1* f) const { load_solve_chunk(t, S, b0, b1, f); }
+  __device__ __forceinline__ void fold_bottom(int i) const {
+    double acc = S.a[i];
+    for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
+      const int c = S.cidx[k];
+      if (c < b0) acc += t.gd[c] * __ldcg(t.r + c);
+    }
+    S.a[i] = acc;
+  }
+  template <int CH, bool PIVOT = true>  // (a solve has no pivot)
+  __device__ __forceinline__ void eliminate(int n) const {
+    const int i = n - b0;
+    double acc = S.a[i];
+    for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
+      const int c = S.cidx[k] - b0;
+      if (c >= 0 && (CH == kAllChildren || tree_shared(S, c) == (CH == kSharedChildren))) acc += S.c[c] * S.a[c];
+    }
+    S.a[i] = acc;
+  }
+  __device__ __forceinline__ double& field(int, int j) const { return S.a[j]; }
+  __device__ __forceinline__ void park(int i) const { t.lam[b0 + i] = S.a[i]; }
+  __device__ __forceinline__ void restore(int i) const {
+    S.a[i] = t.lam[b0 + i];
+    S.b[i] = t.d[b0 + i];
+    S.c[i] = t.gd[b0 + i];
+    S.par[i] = t.t_parent[b0 + i];
+  }
+  __device__ __forceinline__ void store(int i) const { t.r[b0 + i] = S.a[i]; }
+};
+
+// Factorisation fused with the first solve (N == 1): the leaf -> root sweep of the factorisation and the forward
+// elimination of the first right-hand side visit the same nodes in the same order, so they share one staging pass
+// and one set of level barriers.  A fourth shared array e = tg sits behind the TreeSmem view (the parent needs
+// tg_c and gd_c of its children).
+__host__ __device__ constexpr size_t tree_smem_bytes_fs(int cap) {
+  return ((tree_smem_bytes(cap) + 15) & ~(size_t)15) + (size_t)cap * sizeof(double);
+}
+__device__ __forceinline__ double* tree_smem_e(unsigned char* raw, int cap) {
+  return reinterpret_cast<double*>(raw + ((tree_smem_bytes(cap) + 15) & ~(size_t)15));
+}
+
+struct FactorSolveOp {
+  const TreeDev& t;
+  const TreeSmem& S;
+  int b0, b1;
+  // behind the view; factor_solve_up passes its own __restrict__ copy (without it the compiler schedules the
+  // single-GPU sweeps differently)
+  double* Se = tree_smem_e(reinterpret_cast<unsigned char*>(S.a), t.cap);
+  static constexpr int kFields = 3;  // [partial d | tg | partial rhs]
+  static constexpr bool kSolves = true;
+
+  __device__ __forceinline__ void stage(const FusedN1& f) const {
+    const int nn = b1 - b0, tid = threadIdx.x, nth = blockDim.x;
+    if (f.cell_rh) {  // one cell per edge: diagonals / right-hand sides straight from (r, R h)
+      for (int i = tid; i < nn; i += nth) {
+        double dg;
+        S.a[i] = n1_node_rhs_diag(f, t, b0 + i, dg);
+        S.b[i] = dg;
+        const int pe = t.t_pslot[b0 + i];
+        const double tg = pe >= 0 ? 1.0 / f.cell_rh[pe] : 0.0;
+        Se[i] = tg;
+        const int p = t.t_parent[b0 + i];
+        S.par[i] = p;
+        if (p < b0 || p >= b1) t.tg[b0 + i] = tg;  // chunk roots: read by the top chunk
+      }
+    } else {  // several cells per edge: the node arrays were filled by bif_diag_kernel / bif_rhs_kernel
+      for (int i = tid; i < nn; i += nth) {
+        S.a[i] = t.r[b0 + i];
+        S.b[i] = t.diag0[b0 + i];
+        Se[i] = t.tg[b0 + i];
+        S.par[i] = t.t_parent[b0 + i];
+      }
+    }
+  }
+  __device__ __forceinline__ void fold_bottom(int i) const {
+    double ad = S.b[i], ar = S.a[i];
+    for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
+      const int c = S.cidx[k];
+      if (c < b0) {
+        const double gdc = __ldcg(t.gd + c);
+        ad -= __ldcg(t.tg + c) * gdc;
+        ar += gdc * __ldcg(t.r + c);
+      }
+    }
+    S.b[i] = ad;
+    S.a[i] = ar;
+  }
+  template <int CH, bool PIVOT = true>
+  __device__ __forceinline__ void eliminate(int n) const {
+    const int i = n - b0;
+    double ad = S.b[i], ar = S.a[i];
+    int k = S.cptr[i];
+    const int k1 = S.cptr[i + 1];
+#if NXFX_TREE_PAIR
+    // binary nodes: the loads of both children are issued together (the level's cost is its dependent chain);
+    // the sums run in the same order as the loop below
+    for (; k + 2 <= k1; k += 2) {
+      const int c0 = S.cidx[k] - b0, c1 = S.cidx[k + 1] - b0;
+      const int j0 = max(c0, 0), j1 = max(c1, 0);
+      const double e0 = Se[j0], g0 = S.c[j0], a0 = S.a[j0];
+      const double e1 = Se[j1], g1 = S.c[j1], a1 = S.a[j1];
+      if (c0 >= 0 && (CH == kAllChildren || tree_shared(S, c0) == (CH == kSharedChildren))) { ad -= e0 * g0; ar += g0 * a0; }
+      if (c1 >= 0 && (CH == kAllChildren || tree_shared(S, c1) == (CH == kSharedChildren))) { ad -= e1 * g1; ar += g1 * a1; }
+    }
+#endif
+    for (; k < k1; ++k) {
+      const int c = S.cidx[k] - b0;
+      if (c >= 0 && (CH == kAllChildren || tree_shared(S, c) == (CH == kSharedChildren))) {
+        ad -= Se[c] * S.c[c];
+        ar += S.c[c] * S.a[c];
+      }
+    }
+    if (!PIVOT) {
+      S.b[i] = ad;
+      S.a[i] = ar;
+      return;
+    }
+    const double inv = 1.0 / ad;
+    S.b[i] = inv;
+    S.c[i] = Se[i] * inv;
+    S.a[i] = ar;
+  }
+  __device__ __forceinline__ double& field(int q, int j) const { return q == 0 ? S.b[j] : (q == 1 ? Se[j] : S.a[j]); }
+  // private nodes: final (1/d, gd) and eliminated rhs; shared nodes: (partial d, tg) and partial rhs
+  __device__ __forceinline__ void park(int i) const {
+    t.d[b0 + i] = S.b[i];
+    t.gd[b0 + i] = tree_shared(S, i) ? Se[i] : S.c[i];
+    t.lam[b0 + i] = S.a[i];
+  }
+  __device__ __forceinline__ void restore(int i) const {
+    S.b[i] = t.d[b0 + i];
+    S.c[i] = t.gd[b0 + i];
+    S.a[i] = t.lam[b0 + i];
+    Se[i] = 0.0;
+    S.par[i] = t.t_parent[b0 + i];
+  }
+  __device__ __forceinline__ void store(int i) const { t.d[b0 + i] = S.b[i]; t.gd[b0 + i] = S.c[i]; }
+};
+
+// ---- top chunk of a partitioned network ----------------------------------------------------------
+// The top chunk holds nodes PRIVATE to this rank, which complete locally, and SHARED ones, which every rank
+// holds (t.top_sh_pos).  (1) eliminate the private nodes; (2) fold them into their shared parents; (3) the caller
+// sums the partial sums of the shared nodes (Op::field) over the ranks, in rank order; (4) eliminate the shared
+// nodes from their shared children -- identically on every rank.  A private node has no shared child.
+template <typename Op>
+__device__ __forceinline__ void top_partial(const Op& op, const ChunkInfo& ci) {
+  const TreeDev& t = op.t;
+  sweep_up_sel(op.S, ci, [&](int n) { op.template eliminate<kAllChildren>(n); }, kPrivateNodes, t.pr_lmin, 1 << 30);
+  for (int k = threadIdx.x, nth = blockDim.x; k < t.n_sh; k += nth)
+    op.template eliminate<kPrivateChildren, false>(ci.b0 + t.top_sh_pos[k]);
   __syncthreads();
-  for (int i = tid; i < nn; i += nth) t.lam[b0 + i] = S.a[i];
-  for (int k = tid; k < ns; k += nth) buf[k] = S.a[t.top_sh_pos[k]];
+}
+
+template <typename Op>
+__device__ __forceinline__ void top_finish(const Op& op, const ChunkInfo& ci) {
+  sweep_up_sel(op.S, ci, [&](int n) { op.template eliminate<kSharedChildren>(n); }, kSharedNodes, 0, op.t.sh_lmax);
+}
+
+// numeric factorisation of one chunk; t.d receives 1/d.  `top`: children below b0 live in bottom chunks (already
+// written to HBM).
+__device__ __forceinline__ void factor_chunk(const TreeDev& t, const TreeSmem& S, int chunk, bool top, const FusedN1* f) {
+  const ChunkInfo ci = load_chunk_info(t, chunk, S);
+  const FactorOp op{t, S, ci.b0, ci.b1};
+  const int nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
+  load_children(t, ci, S);
+  op.stage(f);
+  __syncthreads();
+  if (top) {
+    for (int i = tid; i < nn; i += nth) op.fold_bottom(i);
+    __syncthreads();
+  }
+  sweep_up(S, ci, [&](int n) { op.eliminate<kAllChildren>(n); });
+  for (int i = tid; i < nn; i += nth) op.store(i);
+}
+
+// load a chunk for the solve: child lists and load_solve_chunk
+__device__ __forceinline__ ChunkInfo stage_solve_chunk(const TreeDev& t, const TreeSmem& S, int chunk,
+                                                       const FusedN1* f = nullptr) {
+  const ChunkInfo ci = load_chunk_info(t, chunk, S);
+  load_children(t, ci, S);
+  load_solve_chunk(t, S, ci.b0, ci.b1, f);
+  __syncthreads();
+  return ci;
+}
+
+// forward elimination of a staged chunk: r_n += sum_c gd_c r_c
+__device__ __forceinline__ void solve_up(const TreeDev& t, const TreeSmem& S, const ChunkInfo& ci, bool top) {
+  const SolveOp op{t, S, ci.b0, ci.b1};
+  const int nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
+  if (top) {
+    for (int i = tid; i < nn; i += nth) op.fold_bottom(i);
+    __syncthreads();
+  }
+  sweep_up(S, ci, [&](int n) { op.eliminate<kAllChildren>(n); });
+  for (int i = tid; i < nn; i += nth) op.store(i);
 }
 
 // lam = r/d + gd * lam(parent); parents outside the chunk (top chunk) are read through L2
@@ -653,65 +754,36 @@ tree_factor_kernel(TreeDev t, int n_bottom, unsigned int* ticket, int do_top, Fu
   TreeSmem S = tree_view(tree_smem_raw, t.cap);
   const FusedN1* f = fin.cell_rh ? &fin : nullptr;
   if (n_bottom > 0) {
-    factor_chunk(t, S, blockIdx.x, false, kFull, nullptr, f);
+    factor_chunk(t, S, blockIdx.x, false, f);
     if (!do_top) return;
     if (!last_block_done(S, ticket, n_bottom)) return;
   }
   if (!do_top) return;
-  factor_chunk(t, S, n_bottom, true, kFull, nullptr, f);
+  factor_chunk(t, S, n_bottom, true, f);
   if (threadIdx.x == 0) *ticket = 0u;
 }
 
 // MODE kTreeUp: forward sweep of the bottom chunks, top chunk (forward + backward) in the last
 // block.  MODE kTreeDown: backward sweep of the bottom chunks.  (two-launch path)
-// Top chunk alone, in the phases of the multi-GPU path (one block).
-// FACTOR: kPartial writes [partial d | tg] to buf, kFinish factorises from the all-reduced buf.
-// SOLVE:  kPartial writes the partial right-hand side, kFinish solves (forward + backward).
-template <bool FACTOR, int PHASE>
-__global__ void __launch_bounds__(kTreeThreads)
-tree_top_kernel(TreeDev t, int top_chunk, double* buf) {
-  extern __shared__ __align__(16) unsigned char tree_smem_raw[];
-  TreeSmem S = tree_view(tree_smem_raw, t.cap);
-  if (FACTOR) {
-    factor_chunk(t, S, top_chunk, true, PHASE, buf);
-  } else {
-    const ChunkInfo ti = load_chunk_info(t, top_chunk, S);
-    load_children(t, ti, S);
-    load_solve_chunk(t, ti, S);
-    __syncthreads();
-    solve_up(t, S, ti, true, PHASE, buf);
-    if (PHASE == kFinish) solve_down(t, S, ti, true);
-  }
-}
-
 template <int MODE>
 __global__ void __launch_bounds__(kTreeThreads)
 tree_solve_kernel(TreeDev t, int n_bottom, unsigned int* ticket, int do_top) {
   extern __shared__ __align__(16) unsigned char tree_smem_raw[];
   TreeSmem S = tree_view(tree_smem_raw, t.cap);
   if (MODE == kTreeDown) {
-    const ChunkInfo ci = load_chunk_info(t, blockIdx.x, S);
-    load_children(t, ci, S);
-    load_solve_chunk(t, ci, S);
-    __syncthreads();
+    const ChunkInfo ci = stage_solve_chunk(t, S, blockIdx.x);
     solve_down(t, S, ci, false);
     return;
   }
   if (n_bottom > 0) {
-    const ChunkInfo ci = load_chunk_info(t, blockIdx.x, S);
-    load_children(t, ci, S);
-    load_solve_chunk(t, ci, S);
-    __syncthreads();
+    const ChunkInfo ci = stage_solve_chunk(t, S, blockIdx.x);
     solve_up(t, S, ci, false);
     for (int i = threadIdx.x; i < ci.b1 - ci.b0; i += blockDim.x) t.r[ci.b0 + i] = S.a[i];
     if (!do_top) return;
     if (!last_block_done(S, ticket, n_bottom)) return;
   }
   if (!do_top) return;
-  const ChunkInfo ti = load_chunk_info(t, n_bottom, S);
-  load_children(t, ti, S);
-  load_solve_chunk(t, ti, S);
-  __syncthreads();
+  const ChunkInfo ti = stage_solve_chunk(t, S, n_bottom);
   solve_up(t, S, ti, true);
   solve_down(t, S, ti, true);
   if (threadIdx.x == 0) *ticket = 0u;
@@ -727,10 +799,7 @@ tree_solve_coop_kernel(TreeDev t, int n_bottom, unsigned int* ticket, unsigned i
   extern __shared__ __align__(16) unsigned char tree_smem_raw[];
   TreeSmem S = tree_view(tree_smem_raw, t.cap);
   const FusedN1* f = fin.r ? &fin : nullptr;
-  const ChunkInfo ci = load_chunk_info(t, blockIdx.x, S);
-  load_children(t, ci, S);
-  load_solve_chunk(t, ci, S, f);
-  __syncthreads();
+  const ChunkInfo ci = stage_solve_chunk(t, S, blockIdx.x, f);
   if ((int)blockIdx.x == n_bottom) {
     if (threadIdx.x == 0) {
       while (atomicAdd(ticket, 0u) != (unsigned int)n_bottom) __nanosleep(32);
@@ -762,45 +831,19 @@ tree_solve_coop_kernel(TreeDev t, int n_bottom, unsigned int* ticket, unsigned i
   solve_down(t, S, ci, false);
 }
 
-// ---- factorisation fused with the first solve (N == 1, single GPU) --------------------------------
-// The leaf -> root sweep of the factorisation and the forward elimination of the first right-hand
-// side visit the same nodes in the same order: one staging pass, one set of level barriers.  A fourth
-// shared array e = tg sits behind the TreeSmem view (the parent needs tg_c and gd_c of its children).
-// Arithmetic per node is exactly that of factor_chunk + solve_up.
-__host__ __device__ constexpr size_t tree_smem_bytes_fs(int cap) {
-  return ((tree_smem_bytes(cap) + 15) & ~(size_t)15) + (size_t)cap * sizeof(double);
-}
-
+// Factorisation + first forward elimination of one chunk (FactorSolveOp).
 // wait_ticket (top chunk in its own block): the chunk's own values are staged first, then the block
 // waits until all wait_count bottom blocks have published their roots.
-// pc (top chunk, multi-GPU): the partial sums of the SHARED nodes are exchanged with the other ranks inside
-// the kernel, see the body.
+// pc (top chunk, multi-GPU): the partial sums of the shared nodes are exchanged with the other ranks over NVLink
+// inside the kernel, between top_partial and top_finish.
 template <bool DIST = false>
 __device__ __forceinline__ void factor_solve_up(const TreeDev& t, const TreeSmem& S, double* __restrict__ Se,
                                                 const ChunkInfo& ci, bool top, const FusedN1& f,
                                                 unsigned int* wait_ticket = nullptr, int wait_count = 0,
                                                 const PeerDev* pc = nullptr) {
-  const int b0 = ci.b0, nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
-  if (f.cell_rh) {  // one cell per edge: diagonals / right-hand sides straight from (r, R h)
-    for (int i = tid; i < nn; i += nth) {
-      double dg;
-      S.a[i] = n1_node_rhs_diag(f, t, b0 + i, dg);
-      S.b[i] = dg;
-      const int pe = t.t_pslot[b0 + i];
-      const double tg = pe >= 0 ? 1.0 / f.cell_rh[pe] : 0.0;
-      Se[i] = tg;
-      const int p = t.t_parent[b0 + i];
-      S.par[i] = p;
-      if (p < b0 || p >= ci.b1) t.tg[b0 + i] = tg;  // chunk roots: read by the top chunk
-    }
-  } else {  // several cells per edge: the node arrays were filled by bif_diag_kernel / bif_rhs_kernel
-    for (int i = tid; i < nn; i += nth) {
-      S.a[i] = t.r[b0 + i];
-      S.b[i] = t.diag0[b0 + i];
-      Se[i] = t.tg[b0 + i];
-      S.par[i] = t.t_parent[b0 + i];
-    }
-  }
+  const FactorSolveOp op{t, S, ci.b0, ci.b1, Se};
+  const int nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
+  op.stage(f);
   __syncthreads();
   NXFX_STAMP(top, 3);
   if (top) {  // fold in the bottom-chunk children (written by the other blocks of this launch)
@@ -812,131 +855,35 @@ __device__ __forceinline__ void factor_solve_up(const TreeDev& t, const TreeSmem
       __syncthreads();
     }
     NXFX_STAMP(top, 4);
-    for (int i = tid; i < nn; i += nth) {
-      double ad = S.b[i], ar = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k];
-        if (c < b0) {
-          const double gdc = __ldcg(t.gd + c);
-          ad -= __ldcg(t.tg + c) * gdc;
-          ar += gdc * __ldcg(t.r + c);
-        }
-      }
-      S.b[i] = ad;
-      S.a[i] = ar;
-    }
+    for (int i = tid; i < nn; i += nth) op.fold_bottom(i);
     __syncthreads();
     NXFX_STAMP(top, 5);
   }
-  // per-node elimination (factor + forward solve); the shared nodes of a partitioned network take only their
-  // SHARED children here -- their private children were folded into the exchanged partial sums
-  auto eliminate = [&](bool shared_children_only) {
-    return [&, shared_children_only](int n) {
-      const int i = n - b0;
-      double ad = S.b[i], ar = S.a[i];
-      int k = S.cptr[i];
-      const int k1 = S.cptr[i + 1];
-#if NXFX_TREE_PAIR
-      for (; k + 2 <= k1; k += 2) {  // both children in flight together (see the plain sweep below)
-        const int c0 = S.cidx[k] - b0, c1 = S.cidx[k + 1] - b0;
-        const int j0 = max(c0, 0), j1 = max(c1, 0);
-        const double e0 = Se[j0], g0 = S.c[j0], a0 = S.a[j0];
-        const double e1 = Se[j1], g1 = S.c[j1], a1 = S.a[j1];
-        if (c0 >= 0 && (!shared_children_only || tree_shared(S, c0))) { ad -= e0 * g0; ar += g0 * a0; }
-        if (c1 >= 0 && (!shared_children_only || tree_shared(S, c1))) { ad -= e1 * g1; ar += g1 * a1; }
-      }
-#endif
-      for (; k < k1; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0 && (!shared_children_only || tree_shared(S, c))) {
-          ad -= Se[c] * S.c[c];
-          ar += S.c[c] * S.a[c];
-        }
-      }
-      const double inv = 1.0 / ad;
-      S.b[i] = inv;
-      S.c[i] = Se[i] * inv;
-      S.a[i] = ar;
-    };
-  };
-  const bool multi = DIST && top && pc && pc->nranks > 1 && t.n_sh > 0;
-  if (!multi) {
-    // single GPU / bottom chunks: the plain level sweep (the latency-critical loop carries nothing else)
-    sweep_up(S, ci, [&](int n) {
-      const int i = n - b0;
-      double ad = S.b[i], ar = S.a[i];
-      int k = S.cptr[i];
-      const int k1 = S.cptr[i + 1];
-#if NXFX_TREE_PAIR
-      // binary nodes: the loads of both children are issued together (the level's cost is its dependent chain);
-      // the sums run in the same order as the loop below
-      for (; k + 2 <= k1; k += 2) {
-        const int c0 = S.cidx[k] - b0, c1 = S.cidx[k + 1] - b0;
-        const int j0 = max(c0, 0), j1 = max(c1, 0);
-        const double e0 = Se[j0], g0 = S.c[j0], a0 = S.a[j0];
-        const double e1 = Se[j1], g1 = S.c[j1], a1 = S.a[j1];
-        if (c0 >= 0) { ad -= e0 * g0; ar += g0 * a0; }
-        if (c1 >= 0) { ad -= e1 * g1; ar += g1 * a1; }
-      }
-#endif
-      for (; k < k1; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0) {
-          ad -= Se[c] * S.c[c];
-          ar += S.c[c] * S.a[c];
-        }
-      }
-      const double inv = 1.0 / ad;
-      S.b[i] = inv;
-      S.c[i] = Se[i] * inv;
-      S.a[i] = ar;
-    });
-  } else {
-    // Partitioned network.  The top chunk holds this rank's PRIVATE heavy nodes (complete locally) and the
-    // SHARED ones (replicated).  (1) eliminate the private nodes; (2) fold them into their shared parents;
-    // (3) exchange [partial pivot | link conductance | partial rhs] of the shared nodes with the other ranks
-    // over NVLink and add them up in rank order; (4) eliminate the shared nodes -- identically on every rank.
+  if (DIST && top && pc && pc->nranks > 1 && t.n_sh > 0) {
     const int ns = t.n_sh;
     const int32_t* __restrict__ pos = t.top_sh_pos;
     load_shared_flags(t, ci, S);
-    sweep_up_sel(S, ci, eliminate(false), kPrivateNodes, t.pr_lmin, 1 << 30);
-    for (int k = tid; k < ns; k += nth) {
-      const int j = pos[k];
-      double ad = S.b[j], ar = S.a[j];
-      for (int q = S.cptr[j]; q < S.cptr[j + 1]; ++q) {
-        const int c = S.cidx[q] - b0;
-        if (c >= 0 && !tree_shared(S, c)) {
-          ad -= Se[c] * S.c[c];
-          ar += S.c[c] * S.a[c];
-        }
-      }
-      S.b[j] = ad;
-      S.a[j] = ar;
-    }
-    __syncthreads();
+    top_partial(op, ci);
     NXFX_STAMP(top, 12);
-    peer_ll_send(*pc, 0, 3 * ns, [&](int i) {
-      return i < ns ? S.b[pos[i]] : (i < 2 * ns ? Se[pos[i - ns]] : S.a[pos[i - 2 * ns]]);
-    });
+    peer_ll_send(*pc, 0, FactorSolveOp::kFields * ns, [&](int i) { return op.field(i / ns, pos[i % ns]); });
     __syncthreads();  // the partial sums have been read out of shared memory: they may be overwritten
     for (int k = tid; k < ns; k += nth) {
-      double ad = 0.0, tg = 0.0, ar = 0.0;
-      for (int src = 0; src < pc->nranks; ++src) {  // rank order: the same sums on every rank
-        ad += peer_ll_recv(*pc, 0, src, k);
-        tg += peer_ll_recv(*pc, 0, src, ns + k);
-        ar += peer_ll_recv(*pc, 0, src, 2 * ns + k);
-      }
-      const int j = pos[k];
-      S.b[j] = ad;
-      Se[j] = tg;
-      S.a[j] = ar;
+      double v[FactorSolveOp::kFields] = {};
+      for (int src = 0; src < pc->nranks; ++src)  // rank order: the same sums on every rank
+#pragma unroll
+        for (int q = 0; q < FactorSolveOp::kFields; ++q) v[q] += peer_ll_recv(*pc, 0, src, q * ns + k);
+#pragma unroll
+      for (int q = 0; q < FactorSolveOp::kFields; ++q) op.field(q, pos[k]) = v[q];
     }
     __syncthreads();
     NXFX_STAMP(top, 13);
-    sweep_up_sel(S, ci, eliminate(true), kSharedNodes, 0, t.sh_lmax);
+    top_finish(op, ci);
+  } else {
+    // single GPU / bottom chunks: the plain level sweep (the latency-critical loop carries nothing else)
+    sweep_up(S, ci, [&](int n) { op.eliminate<kAllChildren>(n); });
   }
   NXFX_STAMP(top, 6);
-  for (int i = tid; i < nn; i += nth) { t.d[b0 + i] = S.b[i]; t.gd[b0 + i] = S.c[i]; }
+  for (int i = tid; i < nn; i += nth) op.store(i);
   NXFX_STAMP(top, 7);
 }
 
@@ -953,7 +900,7 @@ tree_factor_solve_coop_kernel(TreeDev t, int n_bottom, unsigned int* ticket, uns
                               FusedN1 fin, PeerDev pc) {
   extern __shared__ __align__(16) unsigned char tree_smem_raw[];
   TreeSmem S = tree_view(tree_smem_raw, t.cap);
-  double* Se = reinterpret_cast<double*>(tree_smem_raw + ((tree_smem_bytes(t.cap) + 15) & ~(size_t)15));
+  double* Se = tree_smem_e(tree_smem_raw, t.cap);
   const int G = (int)gridDim.x - 1;  // bottom blocks; the last block of the grid owns the top chunk
   const bool is_top = (int)blockIdx.x == G;
   NXFX_STAMP(is_top, 0);
@@ -1026,127 +973,67 @@ tree_factor_solve_coop_kernel(TreeDev t, int n_bottom, unsigned int* ticket, uns
   for (int c = (int)blockIdx.x; c < chunk; c += G) {  // the chunks that were written back
     __syncthreads();
     const ChunkInfo cj = load_chunk_info(t, c, S);
-    load_solve_chunk(t, cj, S);
+    load_solve_chunk(t, S, cj.b0, cj.b1);
     __syncthreads();
     solve_down(t, S, cj, false);
   }
 }
 
 // Multi-GPU form of the fused factor + first solve: bottom chunks only (no top chunk, no backward
-// sweep) ...
+// sweep); the top chunk follows in tree_top_split_kernel<FactorSolveOp, *>.
 __global__ void __launch_bounds__(kTreeThreads, 2)
 tree_factor_solve_bottom_kernel(TreeDev t, FusedN1 fin) {
   extern __shared__ __align__(16) unsigned char tree_smem_raw[];
   TreeSmem S = tree_view(tree_smem_raw, t.cap);
-  double* Se = reinterpret_cast<double*>(tree_smem_raw + ((tree_smem_bytes(t.cap) + 15) & ~(size_t)15));
+  double* Se = tree_smem_e(tree_smem_raw, t.cap);
   const ChunkInfo ci = load_chunk_info(t, blockIdx.x, S);
   load_children(t, ci, S);
   factor_solve_up(t, S, Se, ci, false, fin);
   for (int i = threadIdx.x; i < ci.b1 - ci.b0; i += blockDim.x) t.r[ci.b0 + i] = S.a[i];
 }
 
-// ... and the replicated top chunk in two phases around the caller's SUM all-reduce of
-// buf = [partial d | tg | partial rhs] of the SHARED nodes (3 n_sh doubles): kPartial folds in this rank's
-// bottom-chunk children, kFinish factorises, eliminates and back-substitutes from the reduced values.
-template <int PHASE>
+// Top chunk of a partitioned network alone (one block), in two phases around the caller's SUM all-reduce of
+// buf = Op::kFields x n_sh doubles, the exchanged partial sums of the shared nodes.  kPartial folds in this rank's
+// bottom-chunk children, runs steps 1 and 2, parks every node in global scratch and packs buf; kFinish restores
+// the scratch, takes the shared nodes from the reduced buf, runs step 4 and, for a solve, the backward sweep.
+// fin: the fused input of FactorSolveOp, which stages the chunk as the single-GPU top chunk does (it also fills
+// par and the link conductances t.tg of the roots).  The host-driven FactorOp / SolveOp split stages from the
+// node arrays and does not read fin.  FactorSolveOp::stage takes fin by reference while the other two take a
+// pointer: taking the address of a kernel parameter copies it to local memory, and the single-GPU kernels keep
+// the form they had.
+template <typename Op, int PHASE>
 __global__ void __launch_bounds__(kTreeThreads)
-tree_top_fs_kernel(TreeDev t, int top_chunk, double* buf, FusedN1 fin) {
+tree_top_split_kernel(TreeDev t, int top_chunk, double* buf, FusedN1 fin) {
   extern __shared__ __align__(16) unsigned char tree_smem_raw[];
   TreeSmem S = tree_view(tree_smem_raw, t.cap);
-  double* Se = reinterpret_cast<double*>(tree_smem_raw + ((tree_smem_bytes(t.cap) + 15) & ~(size_t)15));
   const ChunkInfo ci = load_chunk_info(t, top_chunk, S);
-  const int b0 = ci.b0, nn = ci.b1 - ci.b0, tid = threadIdx.x, nth = blockDim.x;
-  const int ns = t.n_sh;
+  const Op op{t, S, ci.b0, ci.b1};
+  const int nn = ci.b1 - ci.b0, ns = t.n_sh, tid = threadIdx.x, nth = blockDim.x;
   const int32_t* __restrict__ pos = t.top_sh_pos;
   load_children(t, ci, S);
   load_shared_flags(t, ci, S);
-  auto eliminate = [&](bool shared_children_only) {
-    return [&, shared_children_only](int n) {
-      const int i = n - b0;
-      double ad = S.b[i], ar = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k] - b0;
-        if (c >= 0 && (!shared_children_only || tree_shared(S, c))) {
-          ad -= Se[c] * S.c[c];
-          ar += S.c[c] * S.a[c];
-        }
-      }
-      const double inv = 1.0 / ad;
-      S.b[i] = inv;
-      S.c[i] = Se[i] * inv;
-      S.a[i] = ar;
-    };
-  };
   if (PHASE == kPartial) {
-    for (int i = tid; i < nn; i += nth) {
-      const int pe = t.t_pslot[b0 + i];
-      S.a[i] = n1_node_rhs(fin, t, b0 + i);
-      S.b[i] = n1_node_diag(fin, t, b0 + i);
-      Se[i] = pe >= 0 ? 1.0 / fin.cell_rh[pe] : 0.0;
-    }
+    if constexpr (std::is_same<Op, FactorSolveOp>::value) op.stage(fin);  // from (r, R h)
+    else op.stage(nullptr);                                                 // from the node arrays
     __syncthreads();
-    for (int i = tid; i < nn; i += nth) {  // this rank's bottom-chunk children
-      double ad = S.b[i], ar = S.a[i];
-      for (int k = S.cptr[i]; k < S.cptr[i + 1]; ++k) {
-        const int c = S.cidx[k];
-        if (c < b0) {
-          ad -= t.tg[c] * t.gd[c];
-          ar += t.gd[c] * t.r[c];
-        }
-      }
-      S.b[i] = ad;
-      S.a[i] = ar;
-    }
+    for (int i = tid; i < nn; i += nth) op.fold_bottom(i);
     __syncthreads();
-    sweep_up_sel(S, ci, eliminate(false), kPrivateNodes, t.pr_lmin, 1 << 30);  // the nodes private to this rank are complete
-    for (int k = tid; k < ns; k += nth) {              // ... and fold into their shared parents
-      const int j = pos[k];
-      double ad = S.b[j], ar = S.a[j];
-      for (int q = S.cptr[j]; q < S.cptr[j + 1]; ++q) {
-        const int c = S.cidx[q] - b0;
-        if (c >= 0 && !tree_shared(S, c)) {
-          ad -= Se[c] * S.c[c];
-          ar += S.c[c] * S.a[c];
-        }
-      }
-      S.b[j] = ad;
-      S.a[j] = ar;
-    }
-    __syncthreads();
-    for (int i = tid; i < nn; i += nth) {  // scratch (arrays kFinish overwrites anyway)
-      t.d[b0 + i] = S.b[i];                       // private: 1/d (final); shared: partial pivot
-      t.gd[b0 + i] = tree_shared(S, i) ? Se[i] : S.c[i];   // private: gd (final); shared: link conductance
-      t.lam[b0 + i] = S.a[i];                     // eliminated / partial right-hand side
-    }
-    for (int k = tid; k < ns; k += nth) {  // the shared ones go to the all-reduce
-      const int j = pos[k];
-      buf[k] = S.b[j];
-      buf[ns + k] = Se[j];
-      buf[2 * ns + k] = S.a[j];
-    }
+    top_partial(op, ci);
+    for (int i = tid; i < nn; i += nth) op.park(i);
+    for (int k = tid; k < ns; k += nth)
+#pragma unroll
+      for (int q = 0; q < Op::kFields; ++q) buf[q * ns + k] = op.field(q, pos[k]);
   } else {
-    for (int i = tid; i < nn; i += nth) {
-      S.b[i] = t.d[b0 + i];
-      S.c[i] = t.gd[b0 + i];
-      S.a[i] = t.lam[b0 + i];
-      Se[i] = 0.0;
-      S.par[i] = t.t_parent[b0 + i];
-    }
+    for (int i = tid; i < nn; i += nth) op.restore(i);
     __syncthreads();
-    for (int k = tid; k < ns; k += nth) {
-      const int j = pos[k];
-      S.b[j] = buf[k];
-      Se[j] = buf[ns + k];
-      S.a[j] = buf[2 * ns + k];
-    }
+    for (int k = tid; k < ns; k += nth)
+#pragma unroll
+      for (int q = 0; q < Op::kFields; ++q) op.field(q, pos[k]) = buf[q * ns + k];
     __syncthreads();
-    sweep_up_sel(S, ci, eliminate(true), kSharedNodes, 0, t.sh_lmax);
-    for (int k = tid; k < ns; k += nth) {
-      const int j = pos[k];
-      t.d[b0 + j] = S.b[j];
-      t.gd[b0 + j] = S.c[j];
-    }
-    solve_down(t, S, ci, true);
+    top_finish(op, ci);
+    // every node, as after a whole-chunk sweep: a private node writes back the final values kPartial parked
+    for (int i = tid; i < nn; i += nth) op.store(i);
+    if (Op::kSolves) solve_down(t, S, ci, true);
   }
 }
 
