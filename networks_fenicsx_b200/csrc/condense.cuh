@@ -407,184 +407,134 @@ __device__ __forceinline__ M2 mul2(M2 x, M2 y) {
   return M2{x.a * y.a + x.b * y.c, x.a * y.b + x.b * y.d, x.c * y.a + x.d * y.c, x.c * y.b + x.d * y.d};
 }
 
-// Block version of tree_sweep_kernel: one thread block per chunk, level by level.
-// MODE 0: factor   D_n = d0_n - sum_children H_c U_c,  Dinv_n,  G_n = Dinv_n U_n,  H_n = L_n Dinv_n
-// MODE 1: forward  r_n -= sum_children H_c r_c
-// MODE 2: backward z_n = Dinv_n r_n - G_n z_parent
-// MODE 3: forward then backward (top chunk)
+// 2 x 2 block forms of ScalarFactor / ScalarSolve (precond.cuh) over the nodal blocks of cond_node_kernel, for
+// btree_sweep_kernel and btree_top_split_kernel.  pack / unpack: the payload of shared node k in the exchange buffer
+// of the split top chunk, nt = max(n_shared, 1), 2 x 2 blocks row-major.
+// BlockFactor: D_n = d0_n - sum_c H_c U_c,  Dinv_n,  G_n = Dinv_n U_n,  H_n = L_n Dinv_n
+struct BlockFactor {
+  const TreeDev& t;
+  const CondDev& c;
+  static constexpr bool kSolves = false;
+  __device__ __forceinline__ M2 own(int n) const { return ld2(c.bd0, n); }
+  __device__ __forceinline__ void fold(M2& D, int ch) const {
+    const M2 p = mul2(ld2(c.bH, ch), ld2(c.bU, ch));
+    D.a -= p.a; D.b -= p.b; D.c -= p.c; D.d -= p.d;
+  }
+  __device__ __forceinline__ void store(int n, M2 D) const {
+    const double idet = 1.0 / (D.a * D.d - D.b * D.c);
+    const M2 Di{D.d * idet, -D.b * idet, -D.c * idet, D.a * idet};
+    st2(c.bDinv, n, Di);
+    st2(c.bG, n, mul2(Di, ld2(c.bU, n)));
+    st2(c.bH, n, mul2(ld2(c.bL, n), Di));
+  }
+  // partial diagonal block D at buf[4k], coupling blocks U (to the parent) at buf[4nt + 4k] and L (from the parent)
+  // at buf[8nt + 4k] -- 12 nt doubles
+  __device__ __forceinline__ void pack(double* buf, int nt, int k, int n, M2 D) const {
+    st2(buf, k, D);
+    st2(buf + 4 * (size_t)nt, k, ld2(c.bU, n));
+    st2(buf + 8 * (size_t)nt, k, ld2(c.bL, n));
+  }
+  // A shared node's coupling blocks come from the edge to its shared parent, which lives on rank 0 (partition_tree):
+  // the other ranks contribute zeros and the sum broadcasts them.  The DG0 identity placeholder on the P slot
+  // (cond_node_kernel) arrives summed over the ranks and is set again; the children's blocks have a zero P row and
+  // column, so folding them in afterwards leaves it as it is, as in the single-GPU sweep.
+  __device__ __forceinline__ M2 unpack(const double* buf, int nt, int k, int n) const {
+    M2 D = ld2(buf, k);
+    if (!c.cont) { D.a = 1.0; D.b = 0.0; D.c = 0.0; }
+    st2(c.bU, n, ld2(buf + 4 * (size_t)nt, k));
+    st2(c.bL, n, ld2(buf + 8 * (size_t)nt, k));
+    return D;
+  }
+};
+
+// BlockSolve: forward r_n -= sum_c H_c r_c ;  backward z_n = Dinv_n r_n - G_n z_parent
+struct BlockSolve {
+  const TreeDev& t;
+  const CondDev& c;
+  static constexpr bool kSolves = true;
+  __device__ __forceinline__ double2 own(int n) const { return make_double2(c.br[2 * (size_t)n], c.br[2 * (size_t)n + 1]); }
+  __device__ __forceinline__ void fold(double2& r, int ch) const {
+    const M2 H = ld2(c.bH, ch);
+    const double s0 = c.br[2 * (size_t)ch], s1 = c.br[2 * (size_t)ch + 1];
+    r.x -= H.a * s0 + H.b * s1;
+    r.y -= H.c * s0 + H.d * s1;
+  }
+  __device__ __forceinline__ void store(int n, double2 r) const {
+    c.br[2 * (size_t)n] = r.x;
+    c.br[2 * (size_t)n + 1] = r.y;
+  }
+  // the partial nodal right-hand side at buf[2k] -- 2 nt doubles
+  __device__ __forceinline__ void pack(double* buf, int, int k, int, double2 r) const {
+    buf[2 * k] = r.x;
+    buf[2 * k + 1] = r.y;
+  }
+  __device__ __forceinline__ double2 unpack(const double* buf, int, int k, int) const {
+    return make_double2(buf[2 * k], buf[2 * k + 1]);
+  }
+  __device__ __forceinline__ void down(int n) const {
+    const int p = t.t_parent[n];
+    const M2 Di = ld2(c.bDinv, n);
+    const double r0 = c.br[2 * (size_t)n], r1 = c.br[2 * (size_t)n + 1];
+    double z0 = Di.a * r0 + Di.b * r1, z1 = Di.c * r0 + Di.d * r1;
+    if (p >= 0) {
+      const M2 G = ld2(c.bG, n);
+      const double p0 = c.bz[2 * (size_t)p], p1 = c.bz[2 * (size_t)p + 1];
+      z0 -= G.a * p0 + G.b * p1;
+      z1 -= G.c * p0 + G.d * p1;
+    }
+    c.bz[2 * (size_t)n] = z0;
+    c.bz[2 * (size_t)n + 1] = z1;
+  }
+};
+
+// block form of tree_sweep_kernel: one thread block per chunk, chunk = blockIdx.x + chunk0
 template <int MODE>
 __global__ void __launch_bounds__(1024)
 btree_sweep_kernel(TreeDev t, CondDev c, int chunk0) {
-  const int chunk = chunk0 + blockIdx.x;
-  const int L0 = t.chunk_lptr[chunk], L1 = t.chunk_lptr[chunk + 1];
-  if (MODE == 0 || MODE == 1 || MODE == 3) {
-    for (int L = L1 - 1; L >= L0; --L) {
-      const int b = t.lvl_ptr[L], e = t.lvl_ptr[L + 1];
-      for (int n = b + threadIdx.x; n < e; n += blockDim.x) {
-        const int c0 = t.t_cptr[n], c1 = t.t_cptr[n + 1];
-        if (MODE == 0) {
-          M2 D = ld2(c.bd0, n);
-          for (int k = c0; k < c1; ++k) {
-            const int ch = t.t_cidx[k];
-            const M2 p = mul2(ld2(c.bH, ch), ld2(c.bU, ch));
-            D.a -= p.a; D.b -= p.b; D.c -= p.c; D.d -= p.d;
-          }
-          const double idet = 1.0 / (D.a * D.d - D.b * D.c);
-          const M2 Di{D.d * idet, -D.b * idet, -D.c * idet, D.a * idet};
-          st2(c.bDinv, n, Di);
-          st2(c.bG, n, mul2(Di, ld2(c.bU, n)));
-          st2(c.bH, n, mul2(ld2(c.bL, n), Di));
-        } else {
-          double r0 = c.br[2 * (size_t)n], r1 = c.br[2 * (size_t)n + 1];
-          for (int k = c0; k < c1; ++k) {
-            const int ch = t.t_cidx[k];
-            const M2 H = ld2(c.bH, ch);
-            const double s0 = c.br[2 * (size_t)ch], s1 = c.br[2 * (size_t)ch + 1];
-            r0 -= H.a * s0 + H.b * s1;
-            r1 -= H.c * s0 + H.d * s1;
-          }
-          c.br[2 * (size_t)n] = r0;
-          c.br[2 * (size_t)n + 1] = r1;
-        }
-      }
-      __syncthreads();
-    }
-  }
-  if (MODE == 2 || MODE == 3) {
-    for (int L = L0; L < L1; ++L) {
-      const int b = t.lvl_ptr[L], e = t.lvl_ptr[L + 1];
-      for (int n = b + threadIdx.x; n < e; n += blockDim.x) {
-        const int p = t.t_parent[n];
-        const M2 Di = ld2(c.bDinv, n);
-        const double r0 = c.br[2 * (size_t)n], r1 = c.br[2 * (size_t)n + 1];
-        double z0 = Di.a * r0 + Di.b * r1, z1 = Di.c * r0 + Di.d * r1;
-        if (p >= 0) {
-          const M2 G = ld2(c.bG, n);
-          const double p0 = c.bz[2 * (size_t)p], p1 = c.bz[2 * (size_t)p + 1];
-          z0 -= G.a * p0 + G.b * p1;
-          z1 -= G.c * p0 + G.d * p1;
-        }
-        c.bz[2 * (size_t)n] = z0;
-        c.bz[2 * (size_t)n + 1] = z1;
-      }
-      __syncthreads();
-    }
-  }
+  sweep_chunk<MODE>(t, chunk0 + blockIdx.x, BlockFactor{t, c}, BlockSolve{t, c});
 }
 
-// Top chunk of a partitioned network, split around the caller's all-reduce (block version of tree_top_split_kernel's
-// kPartial / kFinish, precond.cuh).  sh_idx[i]: position k of top-chunk node b0 + i in the exchanged order of the
-// shared nodes (identical on every rank), -1 for a node private to this rank (sh_idx == nullptr: no shared node).
-// Payload, nt = max(n_shared, 1):
-//   FACTOR: partial diagonal block D_k at buf[4k], coupling blocks U_k (to the parent) at buf[4nt + 4k] and
-//           L_k (from the parent) at buf[8nt + 4k], 2 x 2 row-major -- 12 nt doubles;
-//   SOLVE:  partial nodal right-hand side at buf[2k] -- 2 nt doubles.
-// A shared node's coupling blocks come from the edge to its shared parent, which lives on rank 0 (partition_tree):
-// the other ranks contribute zeros and the sum broadcasts them.
+// Top chunk of a partitioned network, split around the caller's all-reduce of the payloads of Op (BlockFactor or
+// BlockSolve): the block version of tree_top_split_kernel's kPartial / kFinish (precond.cuh).  sh_idx[i]: position
+// k of top-chunk node b0 + i in the exchanged order of the shared nodes (identical on every rank), -1 for a node
+// private to this rank (sh_idx == nullptr: no shared node).
 // kPartial eliminates the private nodes (a private node has private children or bottom-chunk roots only), folds
 // them and this rank's bottom-chunk roots into their shared parents and packs the shared nodes.
 // kFinish reads nothing but the all-reduced payload and what it computes from it: the shared children of a shared
 // node are folded in their exchanged order, so every rank performs the same operations in the same order and
-// writes bit-identical factors and nodal unknowns.  The DG0 identity placeholder on the P slot (cond_node_kernel)
-// arrives summed over the ranks and is set again here.  SOLVE kFinish then runs the backward sweep of the top chunk.
-template <bool FACTOR, int PHASE>
+// writes bit-identical factors and nodal unknowns.  A solve's kFinish then runs the backward sweep of the top chunk.
+template <typename Op, int PHASE>
 __global__ void __launch_bounds__(1024)
 btree_top_split_kernel(TreeDev t, CondDev c, int chunk, const int32_t* __restrict__ sh_idx, int nt, double* __restrict__ buf) {
+  const Op op{t, c};
   const int L0 = t.chunk_lptr[chunk], L1 = t.chunk_lptr[chunk + 1];
   const int b0 = t.lvl_ptr[L0];
   auto kof = [&](int n) { return (sh_idx && n >= b0) ? sh_idx[n - b0] : -1; };  // n < b0: a bottom-chunk root
-  for (int L = L1 - 1; L >= L0; --L) {
-    const int lb = t.lvl_ptr[L], le = t.lvl_ptr[L + 1];
-    for (int n = lb + threadIdx.x; n < le; n += blockDim.x) {
-      const int k = kof(n);
-      if (PHASE == kFinish && k < 0) continue;  // private: complete after kPartial
-      const int c0 = t.t_cptr[n], c1 = t.t_cptr[n + 1];
-      if (FACTOR) {
-        M2 D = PHASE == kFinish ? ld2(buf, k) : ld2(c.bd0, n);
-        auto fold = [&](int ch) {
-          const M2 p = mul2(ld2(c.bH, ch), ld2(c.bU, ch));
-          D.a -= p.a; D.b -= p.b; D.c -= p.c; D.d -= p.d;
-        };
-        if (PHASE == kPartial) {
-          for (int q = c0; q < c1; ++q)
-            if (kof(t.t_cidx[q]) < 0) fold(t.t_cidx[q]);
-          if (k >= 0) {
-            st2(buf, k, D);
-            st2(buf + 4 * (size_t)nt, k, ld2(c.bU, n));
-            st2(buf + 8 * (size_t)nt, k, ld2(c.bL, n));
-            continue;
-          }
-        } else {
-          for (int last = -1;;) {  // shared children in exchanged order
-            int best = 0x7fffffff, bc = -1;
-            for (int q = c0; q < c1; ++q) {
-              const int kc = kof(t.t_cidx[q]);
-              if (kc > last && kc < best) { best = kc; bc = t.t_cidx[q]; }
-            }
-            if (bc < 0) break;
-            fold(bc);
-            last = best;
-          }
-          if (!c.cont) { D.a = 1.0; D.b = 0.0; D.c = 0.0; }
-          st2(c.bU, n, ld2(buf + 4 * (size_t)nt, k));
-          st2(c.bL, n, ld2(buf + 8 * (size_t)nt, k));
+  levels_up(t, L0, L1, [&](int n) {
+    const int k = kof(n), c0 = t.t_cptr[n], c1 = t.t_cptr[n + 1];
+    if (PHASE == kFinish && k < 0) return;  // private: complete after kPartial
+    if (PHASE == kPartial) {  // the private children, then a shared node is packed, a private one eliminated
+      auto v = op.own(n);
+      for (int q = c0; q < c1; ++q)
+        if (kof(t.t_cidx[q]) < 0) op.fold(v, t.t_cidx[q]);
+      if (k >= 0) op.pack(buf, nt, k, n, v);
+      else op.store(n, v);
+    } else {  // the summed payload, then the shared children in exchanged order
+      auto v = op.unpack(buf, nt, k, n);
+      for (int last = -1;;) {
+        int best = 0x7fffffff, bc = -1;
+        for (int q = c0; q < c1; ++q) {
+          const int kc = kof(t.t_cidx[q]);
+          if (kc > last && kc < best) { best = kc; bc = t.t_cidx[q]; }
         }
-        const double idet = 1.0 / (D.a * D.d - D.b * D.c);
-        const M2 Di{D.d * idet, -D.b * idet, -D.c * idet, D.a * idet};
-        st2(c.bDinv, n, Di);
-        st2(c.bG, n, mul2(Di, ld2(c.bU, n)));
-        st2(c.bH, n, mul2(ld2(c.bL, n), Di));
-      } else {
-        double r0, r1;
-        if (PHASE == kFinish) { r0 = buf[2 * (size_t)k]; r1 = buf[2 * (size_t)k + 1]; }
-        else { r0 = c.br[2 * (size_t)n]; r1 = c.br[2 * (size_t)n + 1]; }
-        auto fold = [&](int ch) {
-          const M2 H = ld2(c.bH, ch);
-          const double s0 = c.br[2 * (size_t)ch], s1 = c.br[2 * (size_t)ch + 1];
-          r0 -= H.a * s0 + H.b * s1;
-          r1 -= H.c * s0 + H.d * s1;
-        };
-        if (PHASE == kPartial) {
-          for (int q = c0; q < c1; ++q)
-            if (kof(t.t_cidx[q]) < 0) fold(t.t_cidx[q]);
-          if (k >= 0) { buf[2 * (size_t)k] = r0; buf[2 * (size_t)k + 1] = r1; continue; }
-        } else {
-          for (int last = -1;;) {
-            int best = 0x7fffffff, bc = -1;
-            for (int q = c0; q < c1; ++q) {
-              const int kc = kof(t.t_cidx[q]);
-              if (kc > last && kc < best) { best = kc; bc = t.t_cidx[q]; }
-            }
-            if (bc < 0) break;
-            fold(bc);
-            last = best;
-          }
-        }
-        c.br[2 * (size_t)n] = r0;
-        c.br[2 * (size_t)n + 1] = r1;
+        if (bc < 0) break;
+        op.fold(v, bc);
+        last = best;
       }
+      op.store(n, v);
     }
-    __syncthreads();
-  }
-  if (FACTOR || PHASE != kFinish) return;
-  for (int L = L0; L < L1; ++L) {  // backward sweep of the whole top chunk (as btree_sweep_kernel MODE 2)
-    const int lb = t.lvl_ptr[L], le = t.lvl_ptr[L + 1];
-    for (int n = lb + threadIdx.x; n < le; n += blockDim.x) {
-      const int p = t.t_parent[n];
-      const M2 Di = ld2(c.bDinv, n);
-      const double r0 = c.br[2 * (size_t)n], r1 = c.br[2 * (size_t)n + 1];
-      double z0 = Di.a * r0 + Di.b * r1, z1 = Di.c * r0 + Di.d * r1;
-      if (p >= 0) {
-        const M2 G = ld2(c.bG, n);
-        const double p0 = c.bz[2 * (size_t)p], p1 = c.bz[2 * (size_t)p + 1];
-        z0 -= G.a * p0 + G.b * p1;
-        z1 -= G.c * p0 + G.d * p1;
-      }
-      c.bz[2 * (size_t)n] = z0;
-      c.bz[2 * (size_t)n + 1] = z1;
-    }
-    __syncthreads();
-  }
+  });
+  if constexpr (Op::kSolves && PHASE == kFinish) levels_down(t, L0, L1, [&](int n) { op.down(n); });
 }
 
 // Partitioned network, continuous pressure: the nodal pressure rows nq + node of the shared bifurcations

@@ -424,12 +424,12 @@ int tree_pass(nxfx_ctx* ctx, bool factor, const double* fuse_r = nullptr, bool f
     return NXFX_OK;
   }
   if (factor) {
-    if (nb > 0) NXFX_LAUNCH(ctx, tree_sweep_kernel<0>, nb, 1024, 0, t, ctx->edge_g.p, 0);
-    NXFX_LAUNCH(ctx, tree_sweep_kernel<0>, 1, 1024, 0, t, ctx->edge_g.p, nb);
+    if (nb > 0) NXFX_LAUNCH(ctx, tree_sweep_kernel<kTreeFactor>, nb, 1024, 0, t, ctx->edge_g.p, 0);
+    NXFX_LAUNCH(ctx, tree_sweep_kernel<kTreeFactor>, 1, 1024, 0, t, ctx->edge_g.p, nb);
   } else {
-    if (nb > 0) NXFX_LAUNCH(ctx, tree_sweep_kernel<1>, nb, 1024, 0, t, ctx->edge_g.p, 0);
-    NXFX_LAUNCH(ctx, tree_sweep_kernel<3>, 1, 1024, 0, t, ctx->edge_g.p, nb);
-    if (nb > 0) NXFX_LAUNCH(ctx, tree_sweep_kernel<2>, nb, 1024, 0, t, ctx->edge_g.p, 0);
+    if (nb > 0) NXFX_LAUNCH(ctx, tree_sweep_kernel<kTreeUp>, nb, 1024, 0, t, ctx->edge_g.p, 0);
+    NXFX_LAUNCH(ctx, tree_sweep_kernel<kTreeUpDown>, 1, 1024, 0, t, ctx->edge_g.p, nb);
+    if (nb > 0) NXFX_LAUNCH(ctx, tree_sweep_kernel<kTreeDown>, nb, 1024, 0, t, ctx->edge_g.p, 0);
   }
   return NXFX_OK;
 }
@@ -479,7 +479,7 @@ int cond_factor_local(nxfx_ctx* ctx) {
     TreeDev t = make_tree(ctx);
     NXFX_LAUNCH(ctx, cond_node_kernel<true>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, c, nullptr);
     const int nb = ctx->tree.n_chunks - 1;
-    if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<0>, nb, 1024, 0, t, c, 0);
+    if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<kTreeFactor>, nb, 1024, 0, t, c, 0);
   }
   return NXFX_OK;
 }
@@ -487,7 +487,7 @@ int cond_factor_local(nxfx_ctx* ctx) {
 int do_cond_setup(nxfx_ctx* ctx) {
   int rc = cond_factor_local(ctx);
   if (rc) return rc;
-  if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<0>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
+  if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<kTreeFactor>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
   mark_factored(ctx);
   return NXFX_OK;
 }
@@ -506,7 +506,7 @@ int cond_forward_local(nxfx_ctx* ctx, const double* r, const double* lam_w) {
     TreeDev t = make_tree(ctx);
     NXFX_LAUNCH(ctx, cond_node_kernel<false>, (int)cdiv(ctx->n_bif, kThreads), kThreads, 0, g, t, c, r, lam_w);
     const int nb = ctx->tree.n_chunks - 1;
-    if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<1>, nb, 1024, 0, t, c, 0);
+    if (nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<kTreeUp>, nb, 1024, 0, t, c, 0);
   }
   return NXFX_OK;
 }
@@ -517,7 +517,7 @@ int cond_backward_local(nxfx_ctx* ctx, double* z, bool add) {
   CondDev c = make_cond(ctx);
   TreeDev t = make_tree(ctx);
   const int nb = ctx->tree.n_chunks - 1;
-  if (ctx->n_bif > 0 && nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<2>, nb, 1024, 0, t, c, 0);
+  if (ctx->n_bif > 0 && nb > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<kTreeDown>, nb, 1024, 0, t, c, 0);
   const int grid = (int)cdiv((int64_t)ctx->E + ctx->n_bif, kCondThreads);
   if (add) NXFX_LAUNCH(ctx, cond_backsub_kernel<true>, grid, kCondThreads, 0, g, t, c, z);
   else NXFX_LAUNCH(ctx, cond_backsub_kernel<false>, grid, kCondThreads, 0, g, t, c, z);
@@ -528,7 +528,7 @@ int do_cond_apply(nxfx_ctx* ctx, const double* r, double* z, bool add) {
   NXFX_REQUIRE(ctx, ctx->pc_ready, "pc_setup has not been run");
   int rc = cond_forward_local(ctx, r, nullptr);
   if (rc) return rc;
-  if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<3>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
+  if (ctx->n_bif > 0) NXFX_LAUNCH(ctx, btree_sweep_kernel<kTreeUpDown>, 1, 1024, 0, make_tree(ctx), make_cond(ctx), ctx->tree.n_chunks - 1);
   return cond_backward_local(ctx, z, add);
 }
 
@@ -777,7 +777,8 @@ int top_split(nxfx_ctx* ctx, double* buf) {
   }
   if (ctx->n_bif == 0) return NXFX_OK;
   const int32_t* idx = ctx->n_shared > 0 ? ctx->top_sh_idx.p : nullptr;
-  NXFX_LAUNCH(ctx, (btree_top_split_kernel<FACTOR, PHASE>), 1, 1024, 0, make_tree(ctx), make_cond(ctx), top, idx,
+  using BlockOp = std::conditional_t<FACTOR, BlockFactor, BlockSolve>;
+  NXFX_LAUNCH(ctx, (btree_top_split_kernel<BlockOp, PHASE>), 1, 1024, 0, make_tree(ctx), make_cond(ctx), top, idx,
               std::max(ctx->n_shared, 1), buf);
   return NXFX_OK;
 }

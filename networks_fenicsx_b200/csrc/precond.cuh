@@ -222,58 +222,6 @@ bif_diag_kernel(Net g, TreeDev t, const double* __restrict__ edge_g) {
   t.tg[n] = pe >= 0 ? edge_g[pe] : 0.0;
 }
 
-// Generic (global-memory) sweeps for schedules that do not fit the shared-memory kernels.
-// MODE 0: numeric factorisation  d_t = diag0_t - sum_c g_c^2/d_c ; gd_t = g_t/d_t ; t.d <- 1/d_t
-// MODE 1: forward (leaf -> root)  r_t += sum_c gd_c r_c
-// MODE 2: backward (root -> leaf) lam_t = r_t/d_t + gd_t lam_parent
-// MODE 3: forward then backward (top chunk)
-// One thread block per chunk; chunk = blockIdx.x + chunk0.
-template <int MODE>
-__global__ void __launch_bounds__(1024)
-tree_sweep_kernel(TreeDev t, const double* __restrict__ edge_g, int chunk0) {
-  const int chunk = chunk0 + blockIdx.x;
-  const int L0 = t.chunk_lptr[chunk], L1 = t.chunk_lptr[chunk + 1];
-  if (MODE == 0 || MODE == 1 || MODE == 3) {
-    for (int L = L1 - 1; L >= L0; --L) {
-      const int b = t.lvl_ptr[L], e = t.lvl_ptr[L + 1];
-      for (int n = b + threadIdx.x; n < e; n += blockDim.x) {
-        const int c0 = t.t_cptr[n], c1 = t.t_cptr[n + 1];
-        if (MODE == 0) {
-          double dd = t.diag0[n];
-          for (int k = c0; k < c1; ++k) {
-            const int c = t.t_cidx[k];
-            dd -= edge_g[t.t_pedge[c]] * t.gd[c];
-          }
-          t.d[n] = 1.0 / dd;  // the solve multiplies by 1/d
-          const int pe = t.t_pedge[n];
-          t.gd[n] = pe >= 0 ? edge_g[pe] / dd : 0.0;
-        } else {
-          double rr = t.r[n];
-          for (int k = c0; k < c1; ++k) {
-            const int c = t.t_cidx[k];
-            rr += t.gd[c] * t.r[c];
-          }
-          t.r[n] = rr;
-        }
-      }
-      __syncthreads();
-    }
-  }
-  if (MODE == 2 || MODE == 3) {
-    for (int L = L0; L < L1; ++L) {
-      const int b = t.lvl_ptr[L], e = t.lvl_ptr[L + 1];
-      for (int n = b + threadIdx.x; n < e; n += blockDim.x) {
-        const int p = t.t_parent[n];
-        double v = t.r[n] * t.d[n];
-        if (p >= 0) v += t.gd[n] * t.lam[p];
-        t.lam[n] = v;
-        t.lam_nat[t.bif_of_t[n]] = v;
-      }
-      __syncthreads();
-    }
-  }
-}
-
 // ---- shared-memory tree sweeps ------------------------------------------------------------------
 // One thread block per bottom chunk: the chunk's node data, child lists and level table are staged
 // in shared memory once, the level loop then runs on-chip.  Per-level latency is what bounds these
@@ -335,7 +283,7 @@ __device__ __forceinline__ TreeSmem tree_view(unsigned char* raw, int cap) {
   return S;
 }
 
-enum { kTreeFactor = 0, kTreeUp = 1, kTreeDown = 2 };
+enum { kTreeFactor = 0, kTreeUp = 1, kTreeDown = 2, kTreeUpDown = 3 };  // kTreeUpDown: a top chunk, forward then backward
 
 struct ChunkInfo {
   int b0, b1, cb, ce, nl, Lw;  // Lw: levels 0..Lw all have <= 32 nodes (warp phase), -1 if none
@@ -414,6 +362,27 @@ __device__ __forceinline__ void sweep_down(const TreeSmem& S, const ChunkInfo& c
   __syncthreads();
   for (int L = ci.Lw + 1; L < ci.nl; ++L) {
     for (int n = S.lvl[L] + tid; n < S.lvl[L + 1]; n += blockDim.x) op(n);
+    __syncthreads();
+  }
+}
+
+// The same two sweeps over a chunk whose data stay in global memory (tree_sweep_kernel, btree_top_split_kernel):
+// the chunk's levels [L0, L1) straight from the schedule, every level strided over the whole block and closed by a
+// block barrier.
+template <typename NodeOp>
+__device__ __forceinline__ void levels_up(const TreeDev& t, int L0, int L1, NodeOp op) {
+  for (int L = L1 - 1; L >= L0; --L) {
+    const int b = t.lvl_ptr[L], e = t.lvl_ptr[L + 1];
+    for (int n = b + threadIdx.x; n < e; n += blockDim.x) op(n);
+    __syncthreads();
+  }
+}
+
+template <typename NodeOp>
+__device__ __forceinline__ void levels_down(const TreeDev& t, int L0, int L1, NodeOp op) {
+  for (int L = L0; L < L1; ++L) {
+    const int b = t.lvl_ptr[L], e = t.lvl_ptr[L + 1];
+    for (int n = b + threadIdx.x; n < e; n += blockDim.x) op(n);
     __syncthreads();
   }
 }
@@ -1035,6 +1004,67 @@ tree_top_split_kernel(TreeDev t, int top_chunk, double* buf, FusedN1 fin) {
     for (int i = tid; i < nn; i += nth) op.store(i);
     if (Op::kSolves) solve_down(t, S, ci, true);
   }
+}
+
+// ---- global-memory sweeps -----------------------------------------------------------------------------
+// For schedules that do not fit the shared-memory kernels, and for the 2 x 2 blocks of the higher-order
+// condensation (condense.cuh BlockFactor / BlockSolve).  A node op reads and writes global memory and provides
+//   own(n)        the node's own value
+//   fold(v, c)    child c folded into v
+//   store(n, v)   the node's results from its folded value (a factorisation pivots here)
+// and a solve op also down(n), the node of the backward sweep.
+// ScalarFactor: d_n = diag0_n - sum_c g_c gd_c ;  t.d <- 1/d_n ;  gd_n = g_n / d_n
+struct ScalarFactor {
+  const TreeDev& t;
+  const double* __restrict__ edge_g;
+  __device__ __forceinline__ double own(int n) const { return t.diag0[n]; }
+  __device__ __forceinline__ void fold(double& d, int c) const { d -= edge_g[t.t_pedge[c]] * t.gd[c]; }
+  __device__ __forceinline__ void store(int n, double d) const {
+    t.d[n] = 1.0 / d;  // the solve multiplies by 1/d
+    const int pe = t.t_pedge[n];
+    t.gd[n] = pe >= 0 ? edge_g[pe] / d : 0.0;
+  }
+};
+
+// ScalarSolve: forward r_n += sum_c gd_c r_c ;  backward lam_n = r_n / d_n + gd_n lam_parent
+struct ScalarSolve {
+  const TreeDev& t;
+  __device__ __forceinline__ double own(int n) const { return t.r[n]; }
+  __device__ __forceinline__ void fold(double& r, int c) const { r += t.gd[c] * t.r[c]; }
+  __device__ __forceinline__ void store(int n, double r) const { t.r[n] = r; }
+  __device__ __forceinline__ void down(int n) const {
+    const int p = t.t_parent[n];
+    double v = t.r[n] * t.d[n];
+    if (p >= 0) v += t.gd[n] * t.lam[p];
+    t.lam[n] = v;
+    t.lam_nat[t.bif_of_t[n]] = v;
+  }
+};
+
+// node n of a whole-chunk sweep: its children in t_cidx order
+template <typename Op>
+__device__ __forceinline__ void eliminate_node(const TreeDev& t, const Op& op, int n) {
+  const int c0 = t.t_cptr[n], c1 = t.t_cptr[n + 1];
+  auto v = op.own(n);
+  for (int k = c0; k < c1; ++k) op.fold(v, t.t_cidx[k]);
+  op.store(n, v);
+}
+
+// MODE kTreeFactor / kTreeUp (leaf -> root), kTreeDown (root -> leaf), kTreeUpDown (top chunk) over one chunk.
+template <int MODE, typename Factor, typename Solve>
+__device__ __forceinline__ void sweep_chunk(const TreeDev& t, int chunk, const Factor& factor, const Solve& solve) {
+  const int L0 = t.chunk_lptr[chunk], L1 = t.chunk_lptr[chunk + 1];
+  if (MODE == kTreeFactor) levels_up(t, L0, L1, [&](int n) { eliminate_node(t, factor, n); });
+  if (MODE == kTreeUp || MODE == kTreeUpDown) levels_up(t, L0, L1, [&](int n) { eliminate_node(t, solve, n); });
+  if (MODE == kTreeDown || MODE == kTreeUpDown) levels_down(t, L0, L1, [&](int n) { solve.down(n); });
+}
+
+// One thread block per chunk; chunk = blockIdx.x + chunk0.  The block form, btree_sweep_kernel (condense.cuh), is a
+// kernel of its own: edge_g is read through the read-only cache only as a __restrict__ kernel parameter.
+template <int MODE>
+__global__ void __launch_bounds__(1024)
+tree_sweep_kernel(TreeDev t, const double* __restrict__ edge_g, int chunk0) {
+  sweep_chunk<MODE>(t, chunk0 + blockIdx.x, ScalarFactor{t, edge_g}, ScalarSolve{t});
 }
 
 // Edge condensation: c_e = sum r_q - w.F,  F_N = sum r_p

@@ -2,9 +2,10 @@
 
 1. the per-rank table-driven systems sum to the whole network's system (including the nodal pressure rows of
    the shared bifurcations, which are partial sums on every rank);
-2. a NumPy emulation of the split top-chunk elimination of condense.cuh (btree_top_split_kernel): per rank the
-   kPartial payload, the payloads summed in rank order, kFinish on every rank, back-substitution -- the gathered
-   solution is the whole network's direct solve and the replicated nodal unknowns agree bit for bit."""
+2. a NumPy emulation of the split top-chunk elimination of condense.cuh (btree_top_split_kernel<BlockFactor /
+   BlockSolve, kPartial / kFinish>): per rank the kPartial payload, the payloads summed in rank order, kFinish on
+   every rank, back-substitution -- the gathered solution is the whole network's direct solve and the replicated
+   nodal unknowns agree bit for bit."""
 
 import numpy as np
 import pytest

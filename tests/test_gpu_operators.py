@@ -198,7 +198,8 @@ CASES = [
     ("n2_coop_chunks", lambda: ng.make_tree(8, 3, 4), 2, (1, 0), 16, 0, (3, 4, 5)),
     ("n3_coop_chunks", lambda: ng.make_tree(8, 3, 4), 3, (1, 0), 16, 0, (3, 4, 5)),
     ("n7_coop_chunks", lambda: ng.make_tree(7, 3, 4), 7, (1, 0), 8, 0, (3, 4, 5)),
-    # no shared-memory schedule (chunks deeper than kLevelCap = 64 levels): tree_sweep_kernel<0> x 2, <1>, <3>, <2>
+    # no shared-memory schedule (chunks deeper than kLevelCap = 64 levels):
+    # tree_sweep_kernel<kTreeFactor> x 2, <kTreeUp>, <kTreeUpDown>, <kTreeDown>
     ("chain_global_sweeps_n1", lambda: helpers.linear_graph(400, dim=3), 1, (1, 0), 150, 0, (4, 6, 11)),
     ("chain_global_sweeps_n3", lambda: helpers.linear_graph(400, dim=3), 3, (1, 0), 150, 0, (4, 6, 11)),
     # no bifurcation: the edge kernels only
