@@ -366,6 +366,20 @@ int nxfx_residual_finish(nxfx_ctx* ctx, const double* buf_d, double* r_d, double
  * out_d [2*n_cells]: DG1 dofs (cell-wise [q(first vertex), q(second vertex)]).                       */
 int nxfx_global_flux(nxfx_ctx* ctx, const double* x_d, double* out_d);
 
+/* ---- gather of device-resident inputs and outputs ------------------------------------------ *
+ *   dst_d[r*N + j] = src_d[row(r)*S + (S == N ? j : 0)],  r < n_rows, j < N,
+ *   row(r) = map_d[r] (int32 device table) or r when map_d is NULL;  S in {1, N}.
+ * One kernel on the ctx's stream, asynchronous.  Its uses:
+ *   - a coefficient given as a CUDA tensor (HydraulicNetworkAssembler.compute_forms): per graph edge
+ *     (S = 1) or per cell (S = N) -> per cell, N = cells_per_edge, n_rows = local edges; on a partitioned
+ *     network map_d = the rank's global edge ids restricts a whole-network array to the local edges
+ *     (the device counterpart of np.repeat and arr[global_edges] of the NumPy path);
+ *   - the higher-order global flux of device Functions (post_processing.extract_global_flux):
+ *     N = S = 1, map_d = the flux dof of every DG entry.
+ * The caller orders the producer of src_d before the call (the ctx's stream or an event).            */
+int nxfx_gather(nxfx_ctx* ctx, const double* src_d, const int32_t* map_d, int32_t S, int64_t n_rows,
+                int32_t N, double* dst_d);
+
 #ifdef __cplusplus
 }
 #endif

@@ -143,6 +143,7 @@ SIGNATURES = {
     "nxfx_residual_partial": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "nxfx_residual_finish": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "nxfx_global_flux": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "nxfx_gather": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p]),
 }
 
 _lib = None

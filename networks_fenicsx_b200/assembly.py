@@ -14,6 +14,7 @@ from __future__ import annotations
 
 import ctypes as C
 import logging
+import sys
 import typing
 
 import numpy as np
@@ -62,6 +63,23 @@ def compute_integration_data(
         infl[c] = np.stack([ei * N + N - 1, np.ones_like(ei)], axis=1).astype(np.int32).ravel()
         outfl[c] = np.stack([eo * N, np.zeros_like(eo)], axis=1).astype(np.int32).ravel()
     return infl, outfl
+
+
+def _is_cuda_tensor(v) -> bool:
+    torch = sys.modules.get("torch")  # a tensor exists only once torch has been imported
+    return torch is not None and isinstance(v, torch.Tensor) and v.is_cuda
+
+
+def _check_cuda_tensor(t, dev, name: str) -> None:
+    """Device inputs are taken as they are: float64, contiguous, on the mesh's GPU."""
+    import torch  # noqa: PLC0415
+
+    if t.dtype != torch.float64:
+        raise TypeError(f"{name}: CUDA tensors must be float64, got {t.dtype} (no implicit conversion)")
+    if t.device.index != dev.index:
+        raise ValueError(f"{name} is on {t.device}, the mesh on cuda:{dev.index}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} must be a contiguous tensor")
 
 
 class BlockForm:
@@ -157,18 +175,39 @@ class HydraulicNetworkAssembler:
             p_bc_ex: boundary pressure: callable ``p(x)`` with ``x`` of shape (3, npoints)
                 (DOLFINx interpolation convention), a :class:`fem.CoordinateExpr`
                 (``SpatialCoordinate(mesh)[i]`` arithmetic), an object with ``eval(x)``, or an array
-                of vertex values.
+                of vertex values (NumPy, or a CUDA ``torch.Tensor``).
             f: source term: ``None`` (0), a float, or an array with one value per cell.
             R: resistance: ``None`` (1), a float, an array per cell or per graph edge.
             jit_options, form_compiler_options: accepted for signature compatibility; there is no
                 JIT (the element kernels are compiled ahead of time into libnxfx_b200).
+
+        Arrays may be CUDA tensors (``torch.Tensor``): float64, contiguous, one-dimensional, on the mesh's device
+        (anything else raises before any work is enqueued; nothing is converted).  They are read as the
+        NumPy arrays are, at this call: the assembler copies them into its own device buffers on the
+        library's stream, after the work the current torch stream has enqueued so far (an event, no host
+        wait), and the caller may free or overwrite them as soon as the call returns.  With device inputs
+        only, the call does not wait for the device.  On a partitioned network ``R`` / ``f`` tensors of the
+        whole network's size are restricted to this rank's edges on the device (``nxfx_gather``).
         """
         nm = self._network_mesh
         dev = nm.device
         nv = nm.mesh.topology.index_map(0).size_local
         nc = nm.mesh.topology.index_map(1).size_local
+        # CUDA tensors: every check before anything is enqueued
+        pbc_t = p_bc_ex if _is_cuda_tensor(p_bc_ex) else None
+        if pbc_t is not None:
+            _check_cuda_tensor(pbc_t, dev, "p_bc")
+            if tuple(pbc_t.shape) != (nv,):
+                raise ValueError(f"p_bc array must have one value per mesh vertex ({nv})")
+        R_plan = self._device_coef_plan(R, nc, "R")
+        f_plan = self._device_coef_plan(f, nc, "f")
+        tensors = [t for t in (pbc_t, R if R_plan else None, f if f_plan else None) if t is not None]
+        if tensors:
+            dev.wait_for_torch(*tensors)
         # p_bc interpolated into P1 on the parent mesh (assembly.py:225-234)
-        if isinstance(p_bc_ex, np.ndarray):
+        if pbc_t is not None:
+            self._set_pbc_device(pbc_t, nv)
+        elif isinstance(p_bc_ex, np.ndarray):
             pbc = np.ascontiguousarray(p_bc_ex, dtype=np.float64)
             if pbc.shape != (nv,):
                 raise ValueError(f"p_bc array must have one value per mesh vertex ({nv})")
@@ -181,29 +220,92 @@ class HydraulicNetworkAssembler:
                 )
             x = nm.mesh.geometry.x
             pbc = np.ascontiguousarray(np.asarray(fn(x.T), dtype=np.float64) * np.ones(nv))
-        self._pbc_host = pbc
-        if self._pbc_d is None or self._pbc_d.n != pbc.size:
-            self._pbc_d = dev.empty(pbc.size)
-            self._pbc_d.zero()
-        # the forms read p_bc at BOUNDARY vertices only (assembly.py:258-260): when those are a few contiguous
-        # runs of vertex ids (generated trees: the inlet and the last generation) only the runs travel over PCIe
-        runs = self._boundary_runs()
-        if runs is None:
-            self._pbc_d.upload(pbc, sync=False)
-            self.pbc_h2d_bytes = pbc.nbytes
-        else:
-            for a, b in runs:
-                dev.call("nxfx_memcpy_h2d", C.c_void_p(self._pbc_d.ptr + 8 * a), C.c_void_p(pbc.ctypes.data + 8 * a),
-                         C.c_size_t(8 * (b - a)))
-            self.pbc_h2d_bytes = int(sum(8 * (b - a) for a, b in runs))
-        dev.call("nxfx_set_boundary_pressure", self._pbc_d.c_ptr)  # into the vertex records
-        dev.sync()
+        if pbc_t is None:
+            self._pbc_host = pbc
+            self._ensure_pbc_buffer(nv)
+            # the forms read p_bc at BOUNDARY vertices only (assembly.py:258-260): when those are a few contiguous
+            # runs of vertex ids (generated trees: the inlet and the last generation) only the runs travel over PCIe
+            runs = self._boundary_runs()
+            if runs is None:
+                self._pbc_d.upload(pbc, sync=False)
+                self.pbc_h2d_bytes = pbc.nbytes
+            else:
+                for a, b in runs:
+                    dev.call("nxfx_memcpy_h2d", C.c_void_p(self._pbc_d.ptr + 8 * a), C.c_void_p(pbc.ctypes.data + 8 * a),
+                             C.c_size_t(8 * (b - a)))
+                self.pbc_h2d_bytes = int(sum(8 * (b - a) for a, b in runs))
+            dev.call("nxfx_set_boundary_pressure", self._pbc_d.c_ptr)  # into the vertex records
+            dev.sync()
         nm._pbc_owner = self  # the vertex records now hold THIS assembler's boundary data
-        self._R = self._coefficient(R, 1.0, nc, "R", self._R[0])
-        self._f = self._coefficient(f, 0.0, nc, "f", self._f[0])
+        if R_plan:
+            self._R = self._gather_coef(R, R_plan, nc, self._R[0])
+        else:
+            self._R = self._coefficient(R, 1.0, nc, "R", self._R[0])
+        if f_plan:
+            self._f = self._gather_coef(f, f_plan, nc, self._f[0])
+        else:
+            self._f = self._coefficient(f, 0.0, nc, "f", self._f[0])
         C_ = nm.num_edge_colors
         self._a = _BilinearBlocks(C_)
         self._L = _LinearBlocks(C_)
+
+    def _ensure_pbc_buffer(self, nv: int) -> None:
+        if self._pbc_d is None or self._pbc_d.n != nv:
+            self._pbc_d = self._network_mesh.device.empty(nv)
+            self._pbc_d.zero()
+
+    def _set_pbc_device(self, pbc_t, nv: int) -> None:
+        """p_bc from a checked CUDA tensor: device-to-device into the assembler's own copy (the boundary runs only
+        when :meth:`_boundary_runs` finds them), then into the vertex records; no host wait."""
+        dev = self._network_mesh.device
+        self._pbc_host = None
+        self._ensure_pbc_buffer(nv)
+        src = pbc_t.data_ptr()
+        runs = self._boundary_runs()
+        for a, b in [(0, nv)] if runs is None else runs:
+            if b > a:
+                dev.call("nxfx_memcpy_d2d", C.c_void_p(self._pbc_d.ptr + 8 * a), C.c_void_p(src + 8 * a),
+                         C.c_size_t(8 * (b - a)))
+        self.pbc_h2d_bytes = 0
+        dev.call("nxfx_set_boundary_pressure", self._pbc_d.c_ptr)
+
+    def _device_coef_plan(self, val, nc: int, name: str):
+        """``(rows, S)`` of the ``nxfx_gather`` that turns a CUDA tensor coefficient into one value per cell
+        (``rows``: ``"local"`` or ``"global"`` -- a whole-network array on a partitioned mesh), ``None`` for
+        anything that is not a CUDA tensor.  Checks the tensor; the sizes are tried in the order of
+        :meth:`_coefficient`."""
+        if not _is_cuda_tensor(val):
+            return None
+        nm = self._network_mesh
+        _check_cuda_tensor(val, nm.device, name)
+        N, E = nm.cells_per_edge, nm.graph_edges.shape[0]
+        n = val.numel() if val.dim() == 1 else -1
+        if getattr(nm, "_partition", None) is not None and n >= 0 and n != nc:
+            Eg = nm._global_graph.number_of_edges()
+            if n == Eg:
+                return ("global", 1)
+            if n == Eg * N:
+                return ("global", N)
+        if n == E:
+            return ("local", 1)
+        if n == nc:
+            return ("local", N)
+        raise ValueError(f"{name} must be a scalar, one value per cell ({nc}) or per graph edge")
+
+    def _gather_coef(self, t, plan, nc: int, previous=None):
+        """Per-cell device copy of a checked CUDA tensor coefficient (``previous`` reused when it has the size)."""
+        nm = self._network_mesh
+        dev = nm.device
+        rows, S = plan
+        out = previous if previous is not None and previous.n == nc else dev.empty(nc)
+        gmap = None
+        if rows == "global":
+            if getattr(nm, "_global_edges_d", None) is None:  # uploaded once per mesh
+                nm._global_edges_d = dev.from_host(np.ascontiguousarray(nm._partition.global_edges, dtype=np.int32))
+            gmap = nm._global_edges_d.c_ptr
+        dev.call("nxfx_gather", C.c_void_p(t.data_ptr()), gmap, S, nm.graph_edges.shape[0], nm.cells_per_edge,
+                 out.c_ptr)
+        return (out, 0.0)
 
     def _boundary_runs(self, max_runs: int = 8):
         """``[(first, last + 1), ...]`` of the boundary vertex ids if they form at most ``max_runs`` contiguous

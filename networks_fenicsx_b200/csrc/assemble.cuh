@@ -600,4 +600,16 @@ global_flux_kernel(Net g, const double* __restrict__ x, double* __restrict__ out
   }
 }
 
+// dst[r * N + j] = src[row(r) * S + (S == N ? j : 0)], row(r) = map ? map[r] : r, S in {1, N} (nxfx_gather)
+__global__ void gather_kernel(int64_t n_rows, int N, int S, const int32_t* __restrict__ map, const double* __restrict__ src,
+              double* __restrict__ dst) {
+  const int64_t total = n_rows * N;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / N;
+    const int j = (int)(i - r * N);
+    const int64_t row = map ? (int64_t)map[r] : r;
+    dst[i] = src[row * S + (S == N ? j : 0)];
+  }
+}
+
 }  // namespace nxfx

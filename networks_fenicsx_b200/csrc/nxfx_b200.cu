@@ -2160,6 +2160,16 @@ int nxfx_global_flux(nxfx_ctx* ctx, const double* x, double* out) {
   return NXFX_OK;
 }
 
+int nxfx_gather(nxfx_ctx* ctx, const double* src, const int32_t* map, int32_t S, int64_t n_rows, int32_t N,
+                double* dst) {
+  if (!ctx) return NXFX_ERR_INVALID;
+  NXFX_REQUIRE(ctx, N >= 1 && (S == 1 || S == N) && n_rows >= 0, "N >= 1, S in {1, N}, n_rows >= 0");
+  if (n_rows == 0) return NXFX_OK;
+  NXFX_REQUIRE(ctx, src && dst, "null src / dst");
+  NXFX_LAUNCH(ctx, gather_kernel, vec_grid(ctx, n_rows * N), kThreads, 0, n_rows, (int)N, (int)S, map, src, dst);
+  return NXFX_OK;
+}
+
 #ifdef NXFX_TREE_STAMPS
 // development builds only (not part of include/nxfx_b200.h)
 int nxfx_debug_tree_stamps(nxfx_ctx* ctx, unsigned long long* out32) {

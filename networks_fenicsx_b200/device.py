@@ -27,8 +27,16 @@ class Device:
         self.handle = handle
         self.index = int(index)
         self._finalizer = weakref.finalize(self, self.lib.nxfx_destroy, handle)
+        self.stream = None  # cudaStream_t of the ctx as an int; None: the legacy default stream
+        self._torch_stream = None
         if stream is not None:
-            self.call("nxfx_set_stream", C.c_void_p(stream))
+            self.set_stream(stream)
+
+    def set_stream(self, stream: int | None) -> None:
+        """Run the ctx on ``stream`` (a ``cudaStream_t`` as an int; None or 0: the legacy default stream)."""
+        self.call("nxfx_set_stream", C.c_void_p(stream or None))
+        self.stream = int(stream) if stream else None
+        self._torch_stream = None
 
     def call(self, name: str, *args) -> None:
         rc = getattr(self.lib, name)(self.handle, *args)
@@ -50,6 +58,39 @@ class Device:
         ms = C.c_double()
         self.call("nxfx_timer_stop", C.byref(ms))
         return ms.value
+
+    # ---- ordering against torch (CUDA tensors handed in or out) ----------------------------------
+    def torch_stream(self):
+        """The ctx's stream as a ``torch.cuda.Stream``."""
+        import torch  # noqa: PLC0415
+
+        if self._torch_stream is None:
+            cuda = torch.device("cuda", self.index)
+            self._torch_stream = (torch.cuda.ExternalStream(self.stream, device=cuda) if self.stream
+                                  else torch.cuda.default_stream(cuda))
+        return self._torch_stream
+
+    def wait_for_torch(self, *tensors) -> None:
+        """Order the work this ctx enqueues next after what the current torch stream has enqueued so far (an
+        event, no host wait), and keep torch's caching allocator from handing ``tensors`` to a new tensor before
+        the ctx's stream has passed that work (``record_stream``)."""
+        import torch  # noqa: PLC0415
+
+        lib = self.torch_stream()
+        cur = torch.cuda.current_stream(lib.device)
+        if cur.cuda_stream != lib.cuda_stream:
+            lib.wait_stream(cur)
+        for t in tensors:
+            t.record_stream(lib)
+
+    def torch_wait(self) -> None:
+        """Order the work the current torch stream enqueues next after what this ctx has enqueued so far."""
+        import torch  # noqa: PLC0415
+
+        lib = self.torch_stream()
+        cur = torch.cuda.current_stream(lib.device)
+        if cur.cuda_stream != lib.cuda_stream:
+            cur.wait_stream(lib)
 
     def empty(self, n: int, dtype=np.float64) -> "DeviceArray":
         return DeviceArray(self, int(n), np.dtype(dtype))
@@ -84,14 +125,23 @@ def default_device(index: int = 0) -> Device:
 class DeviceArray:
     """Flat device buffer of ``n`` elements.  ``on_write`` (optional) is called after every write this
     object or a view of it makes (``upload``, ``zero``): the owner of a borrowed buffer learns that its
-    contents changed (``Mat.values``: ``Mat.touch``)."""
+    contents changed (``Mat.values``: ``Mat.touch``).
 
-    def __init__(self, dev: Device, n: int, dtype=np.float64, ptr: int | None = None, on_write=None):
+    ``__cuda_array_interface__`` (version 3) exposes the buffer without a copy, e.g. ``torch.as_tensor(a,
+    device="cuda")``; the tensor keeps this object, and so the memory, alive.  ``shape`` / ``strides`` (bytes)
+    describe a strided view of the buffer (default: the ``n`` elements, contiguous).  The interface names the
+    ctx's stream; the Python layer itself orders the ctx's stream against torch's current stream with events
+    (:meth:`Device.wait_for_torch`, :meth:`Device.torch_wait`), since torch does not read that field."""
+
+    def __init__(self, dev: Device, n: int, dtype=np.float64, ptr: int | None = None, on_write=None,
+                 shape: tuple | None = None, strides: tuple | None = None):
         self.dev = dev
         self.n = int(n)
         self.dtype = np.dtype(dtype)
         self.owned = ptr is None
         self.on_write = on_write
+        self.shape = (self.n,) if shape is None else tuple(int(s) for s in shape)
+        self.strides = None if strides is None else tuple(int(s) for s in strides)
         if ptr is None:
             p = C.c_void_p()
             dev.call("nxfx_malloc", C.c_size_t(self.nbytes), C.byref(p))
@@ -107,6 +157,18 @@ class DeviceArray:
     @property
     def c_ptr(self) -> C.c_void_p:
         return C.c_void_p(self.ptr)
+
+    @property
+    def __cuda_array_interface__(self) -> dict:
+        # stream: 1 = the legacy default stream (0 is not allowed by the protocol)
+        return {"shape": self.shape, "typestr": self.dtype.str, "data": (self.ptr, False), "version": 3,
+                "strides": self.strides, "stream": self.dev.stream or 1}
+
+    def as_tensor(self):
+        """Zero-copy ``torch.Tensor`` on the ctx's device over this buffer (through ``__cuda_array_interface__``)."""
+        import torch  # noqa: PLC0415
+
+        return torch.as_tensor(self, device=torch.device("cuda", self.dev.index))
 
     def upload(self, host: np.ndarray, sync: bool = True) -> None:
         host = np.ascontiguousarray(host, dtype=self.dtype)

@@ -300,7 +300,7 @@ class DistributedSolver:
         mesh = NetworkMesh(part.graph, N=N, color_strategy=color_strategy, device=device,
                            node_degree=part.node_degree, comm=SerialComm())
         if stream is not None:
-            mesh.device.call("nxfx_set_stream", C.c_void_p(stream))
+            mesh.device.set_stream(stream)
         assembler = HydraulicNetworkAssembler(mesh, flux_degree=flux_degree, pressure_degree=pressure_degree)
         assembler.compute_forms(p_bc_ex=p_bc_ex, f=self._restrict(f, N, graph), R=self._restrict(R, N, graph))
         solver = Solver(assembler, schedule=part.schedule)

@@ -715,6 +715,23 @@ class NetworkMesh:
         self.device.call("nxfx_mesh_geometry_device", C.byref(p))
         return DeviceArray(self.device, self._n_vertices * 4, np.float64, ptr=p.value)
 
+    def vertex_coordinates_device(self):
+        """The vertex coordinates on the GPU: a ``(n_vertices, 3)`` float64 CUDA ``torch.Tensor`` viewing the
+        32-byte vertex records of the device (row stride 4), without a copy -- for evaluating ``p_bc(x, t)`` on the
+        GPU and handing it to :meth:`HydraulicNetworkAssembler.compute_forms`.  The view is borrowed from the
+        context (valid while this mesh lives) and is READ-ONLY by contract: the assembly reads the cell lengths
+        from these records, and torch has no read-only tensors (it refuses the read-only flag of
+        ``__cuda_array_interface__``), so nothing stops a write.  Work enqueued on the current torch stream after
+        this call sees the coordinates the library has enqueued so far."""
+        p = C.c_void_p()
+        dev = self.device
+        dev.call("nxfx_mesh_geometry_device", C.byref(p))
+        nv = self._n_vertices
+        view = DeviceArray(dev, nv * 4, np.float64, ptr=p.value, shape=(nv, 3), strides=(32, 8))
+        view._owner = self  # the records belong to this mesh's context
+        dev.torch_wait()
+        return view.as_tensor()
+
     def _geometry_x(self) -> npt.NDArray[np.float64]:
         if self._x_host is None:
             self._x_host = np.ascontiguousarray(self.geometry_device().download().reshape(-1, 4)[:, :3])

@@ -8,6 +8,7 @@ from pathlib import Path
 
 import numpy as np
 
+from .assembly import _is_cuda_tensor
 from .fem import Function, FunctionSpace
 from .mesh import NetworkMesh
 
@@ -20,7 +21,9 @@ def extract_global_flux(graph_mesh: NetworkMesh, functions: list[Function]) -> F
 
     Args:
         graph_mesh: The network mesh
-        functions: The list of functions ``[flux_1, ..., flux_M, pressure, lm]``
+        functions: The list of functions ``[flux_1, ..., flux_M, pressure, lm]``; functions of
+            ``Solver.create_functions(device=True)`` (or any functions whose arrays are CUDA tensors) give a
+            function whose ``x.array`` is a CUDA tensor (no host copy; ready for the current torch stream)
     """
     flux_functions = functions[:-2]
     q_degree = flux_functions[0].function_space.element.basix_element.degree
@@ -30,6 +33,8 @@ def extract_global_flux(graph_mesh: NetworkMesh, functions: list[Function]) -> F
         lambda: np.arange((q_degree + 1) * nc, dtype=np.int32).reshape(nc, q_degree + 1), "global_flux",
     )
     dev = graph_mesh.device
+    if _is_cuda_tensor(flux_functions[0].x.array):
+        return _global_flux_device(graph_mesh, flux_functions, V, q_degree)
     if q_degree != 1:
         # higher order: host gather through the cell -> dof tables of the per-colour spaces
         global_q = Function(V, name="Global_Flux")
@@ -55,16 +60,71 @@ def extract_global_flux(graph_mesh: NetworkMesh, functions: list[Function]) -> F
     return global_q
 
 
+def _global_flux_device(graph_mesh: NetworkMesh, flux_functions: list[Function], V: FunctionSpace,
+                        q_degree: int) -> Function:
+    """``extract_global_flux`` of device functions: P1 through ``nxfx_global_flux``, higher degrees through
+    ``nxfx_gather`` over the DG entry -> flux dof table (the host gather below, built once per mesh and degree).
+    The output (and the scratch copy of flux blocks that are not contiguous) come from torch's caching allocator,
+    so that a time loop calling this allocates and frees nothing through the driver (no implicit host waits)."""
+    import torch  # noqa: PLC0415
+
+    dev = graph_mesh.device
+    arrays = [f.x.array for f in flux_functions]
+    for i, flux in enumerate(flux_functions):
+        flux.name = f"Flux_{i}"
+    cuda = torch.device("cuda", dev.index)
+    out = torch.empty(V.num_dofs, dtype=torch.float64, device=cuda)
+    # the flux blocks of create_functions(device=True) follow each other in one buffer: read them in place
+    src = arrays[0].data_ptr()
+    xq = None
+    if any(a.data_ptr() != src + 8 * sum(b.numel() for b in arrays[:i]) for i, a in enumerate(arrays)):
+        xq = torch.empty(sum(a.numel() for a in arrays), dtype=torch.float64, device=cuda)
+        src = xq.data_ptr()
+    dev.wait_for_torch(*[t for t in (out, xq) if t is not None])
+    if xq is not None:
+        off = 0
+        for a in arrays:
+            if a.numel():
+                dev.call("nxfx_memcpy_d2d", C.c_void_p(src + 8 * off), C.c_void_p(a.data_ptr()),
+                         C.c_size_t(8 * a.numel()))
+            off += a.numel()
+    out_ptr = C.c_void_p(out.data_ptr())
+    if q_degree == 1:
+        dev.call("nxfx_global_flux", C.c_void_p(src), out_ptr)
+    else:
+        if getattr(graph_mesh, "_global_flux_index", None) is None:
+            graph_mesh._global_flux_index = {}
+        cache = graph_mesh._global_flux_index
+        if q_degree not in cache:
+            nc = V.num_dofs // (q_degree + 1)
+            idx = np.zeros((nc, q_degree + 1), dtype=np.int32)
+            off = 0
+            for i, flux in enumerate(flux_functions):
+                dm = flux.function_space.dofmap.list
+                cells = graph_mesh.entity_maps[i].sub_topology_to_topology(np.arange(dm.shape[0], dtype=np.int32))
+                idx[cells] = off + dm
+                off += flux.function_space.num_dofs
+            cache[q_degree] = dev.from_host(idx.ravel())
+        dev.call("nxfx_gather", C.c_void_p(src), cache[q_degree].c_ptr, 1, V.num_dofs, 1, out_ptr)
+    global_q = Function(V, name="Global_Flux", array=out)
+    dev.torch_wait()
+    return global_q
+
+
 def export_functions(functions: list[Function], outpath: Path | str):
     """Write the solution functions as ``.npy`` arrays (``flux_i``, ``pressure``, ``lm``) --
     the reference writes ADIOS2 VTX files (post_processing.py:55-78); ADIOS2 is not part of this
-    build, see DESIGN.md "out of scope"."""
+    build, see DESIGN.md "out of scope".  Device functions are copied to the host."""
     export_path = Path(outpath)
     export_path.mkdir(parents=True, exist_ok=True)
     for i, q in enumerate(functions[:-2]):
-        np.save(export_path / f"flux_{i}.npy", q.x.array)
-    np.save(export_path / "pressure.npy", functions[-2].x.array)
-    np.save(export_path / "lm.npy", functions[-1].x.array)
+        np.save(export_path / f"flux_{i}.npy", _host(q.x.array))
+    np.save(export_path / "pressure.npy", _host(functions[-2].x.array))
+    np.save(export_path / "lm.npy", _host(functions[-1].x.array))
+
+
+def _host(a) -> np.ndarray:
+    return a.cpu().numpy() if _is_cuda_tensor(a) else a
 
 
 def export_submeshes(network_mesh: NetworkMesh, outpath: str | Path):

@@ -121,22 +121,36 @@ class Solver:
     def ksp(self) -> KSP:
         return self._ksp
 
-    def create_functions(self) -> list[Function]:
+    def create_functions(self, device: bool = False) -> list[Function]:
         """Functions ``[flux_color_i ..., pressure, global_flux]`` backed by pinned host memory; pass
-        them to :meth:`solve` to have the solution copied straight into them (no staging copy)."""
+        them to :meth:`solve` to have the solution copied straight into them (no staging copy).
+
+        ``device=True``: the ``x.array`` of every function is a float64 CUDA ``torch.Tensor``, a view into ONE
+        device buffer in block order; :meth:`solve` then writes the solution there and nothing crosses PCIe.
+        The buffer lives as long as any of the tensors."""
         asm = self.assembler
         dev = asm.network.device
         out = []
         spaces = [*asm.flux_spaces, asm.pressure_space, asm.lm_space]
         names = [f"flux_color_{i}" for i in range(len(spaces) - 2)] + ["pressure", "global_flux"]
-        # ONE pinned buffer in block order, the functions are views into it: solve() has the library mirror x into
-        # it while the residual check still runs (nxfx_set_solution_mirror)
-        mirror = dev.pinned(asm.num_dofs)
+        if device:
+            buf = dev.empty(asm.num_dofs)
+            buf.zero()
+            whole = buf.as_tensor()  # holds buf; the block views hold the whole
+            dev.torch_wait()  # the zeros are there for the current torch stream
+        else:
+            # ONE pinned buffer in block order, the functions are views into it: solve() has the library mirror x
+            # into it while the residual check still runs (nxfx_set_solution_mirror)
+            mirror = dev.pinned(asm.num_dofs)
         off = 0
         for V, name in zip(spaces, names):
-            fn = Function(V, name=name, array=mirror[off:off + V.num_dofs])
-            fn._pinned = True
-            fn._mirror = mirror
+            if device:
+                fn = Function(V, name=name, array=whole[off:off + V.num_dofs])
+                fn._device_buffer = buf
+            else:
+                fn = Function(V, name=name, array=mirror[off:off + V.num_dofs])
+                fn._pinned = True
+                fn._mirror = mirror
             off += V.num_dofs
             out.append(fn)
         return out
@@ -194,10 +208,19 @@ class Solver:
 
         Args:
             functions: functions to assign to (reused across solves to avoid host allocations);
-                created from the assembler's spaces if not given.
+                created from the assembler's spaces if not given.  Functions of
+                ``create_functions(device=True)`` receive the solution on the device: the solve writes into
+                their buffer after the work the current torch stream has enqueued so far, and the values are
+                ready for that stream when the call returns.  :attr:`x` holds the same values.
         """
         asm = self.assembler
         dev = asm.network.device
+        buf = getattr(functions[0], "_device_buffer", None) if functions else None
+        if functions and any(getattr(fn, "_device_buffer", None) is not buf for fn in functions):
+            raise ValueError("device functions must all come from one create_functions(device=True) call, and "
+                             "cannot be mixed with host functions")
+        if buf is not None:
+            return self._solve_device(functions, buf, dev)
         if functions is None:
             # fresh Functions per call (as the reference does); their arrays are filled from a
             # pinned staging buffer that the solver keeps, so repeated solves do not pay for
@@ -254,6 +277,28 @@ class Solver:
                     )
                 off += n
             dev.sync()
+        return functions
+
+    def _solve_device(self, functions: list[Function], buf, dev) -> list[Function]:
+        if buf.n != self._x.n:
+            raise ValueError("functions do not match the block layout [flux colours, pressure, multipliers]")
+        opts = self.solve_options()
+        self.info = _lib.SolveInfo()
+        self._A._materialise_zero()
+        self._A.bind()
+        dev.wait_for_torch()  # torch work still reading the previous solution comes before the overwrite
+        nbytes = C.c_size_t(buf.nbytes)
+        if self._dist is None:
+            try:
+                dev.call("nxfx_solve", self._b.device_ptr(), buf.c_ptr, C.byref(opts), C.byref(self.info))
+            finally:
+                self._record_info()
+            dev.call("nxfx_memcpy_d2d", self._x.device_ptr_overwrite(), buf.c_ptr, nbytes)
+        else:  # the distributed layer owns solver.x: copy its local dofs
+            self._run_solve(opts, dev)
+            dev.call("nxfx_memcpy_d2d", buf.c_ptr, self._x.device_ptr(), nbytes)
+        self._x.mark_device_modified()
+        dev.torch_wait()
         return functions
 
     def _run_solve(self, opts, dev) -> None:
